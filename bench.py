@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the TexPose render hot path on B200 (contract: see the task's bench.py section).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], "C2"): LineMOD-duck-shaped synthetic full-frame render, 480x640 rays x 128
 samples, static + transient + light heads, random-init (seed 0) weights, bf16 tensor-core MLP.  One step = ONE frame.
@@ -47,7 +47,13 @@ def parse():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-parity-frame", action="store_true", help="skip the fp32-parity-mode frame (split-fp16 kernel vs SIMT)")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the one-view-per-GPU block")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def peaks():
@@ -319,6 +325,40 @@ def kernel_ms_of_timed_steps(call_ms, steps, warmup):
     return sum(call_ms[-per * steps:]) / steps
 
 
+DUMP_LIMIT_BYTES = 64 << 20     # all arrays of one --dump-outputs directory
+DUMP_WHOLE_BYTES = 8 << 20      # larger arrays are stored at DUMP_RAYS rays
+DUMP_RAYS = 8192
+
+
+def dump_outputs(out_dir, outputs, n_rays):
+    """Writes every tensor of `outputs` as out_dir/<name>.npy: floating point as float32 (float64 stays), integers as float64.
+    An array over DUMP_WHOLE_BYTES (the per-sample outputs [1, rays, samples, ...], 0.65 GB a frame) is stored at DUMP_RAYS rays drawn
+    with a fixed seed, listed in sample_ray_idx.npy.  The bench's inputs are seeded, so the same arguments write the same files
+    and two builds can be compared array by array.  Returns the bytes written."""
+    import numpy as np
+    import torch
+    pick = torch.randperm(n_rays, generator=torch.Generator().manual_seed(0))[:DUMP_RAYS].sort().values
+    arrays = {}
+    for name, t in outputs.items():
+        if not isinstance(t, torch.Tensor):
+            continue
+        dtype = torch.float32 if t.is_floating_point() and t.dtype != torch.float64 else torch.float64
+        t = t.detach()
+        if t.numel() * dtype.itemsize > DUMP_WHOLE_BYTES:
+            if t.dim() < 2 or t.shape[1] != n_rays:
+                raise ValueError(f"--dump-outputs: {name} {tuple(t.shape)} is too large to store whole and has no ray dimension")
+            t = t.index_select(1, pick.to(t.device))
+            arrays["sample_ray_idx"] = pick.to(torch.float64)
+        arrays[name] = t.to("cpu", dtype)
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+    return total
+
+
 # ---------------------------------------------------------------------------------------------- our arm
 
 def run_ours(args, rank, world, local_rank):
@@ -447,11 +487,21 @@ def run_ours(args, rank, world, local_rank):
         h2d = int(t.item())
         d2h = sum(t.numel() * t.element_size() for t in out_h.values())      # rank 0 reads the gathered frame back
 
+    last = {}
+
+    def step_timed():
+        last["ret"] = step_resident()
+
     _C.launch_counts.clear()
     # CUDA events around the fused launch INSIDE the timed region (two event records per step on the launching stream): the kernel
     # time of the roofline and the step time of the headline come from the same iterations, so kernel <= step by construction
     with CallTimer({"tp_render_fused_forward"}) as ct:
-        ms, clocks = timed(step_resident, args.steps, args.warmup, sampler=True)
+        ms, clocks = timed(step_timed, args.steps, args.warmup, sampler=True)
+    if args.dump_outputs and rank == 0:
+        # written before any later block renders again: N > 1 returns views of the frame buffers the next gathers overwrite
+        frame = last["ret"] if world == 1 else last["ret"][0]
+        nbytes = dump_outputs(args.dump_outputs, frame, H * W)
+        print(f"bench.py: wrote {nbytes / 2 ** 20:.1f} MiB of step {args.steps} outputs to {args.dump_outputs}", file=sys.stderr)
     per_step = {k: v // (args.steps + args.warmup) for k, v in _C.launch_counts.items() if v >= args.steps + args.warmup}
     launches = sum(per_step.values()) * args.steps
     k_ms = kernel_ms_of_timed_steps(ct.per_call_ms().get("tp_render_fused_forward", []), args.steps, args.warmup)

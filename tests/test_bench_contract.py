@@ -76,3 +76,30 @@ def test_kernel_time_comes_from_the_timed_iterations():
     assert f([9.0, 9.0, 9.0, 1.0, 2.0, 3.0], steps=3, warmup=3) == 2.0          # warm-up calls dropped
     assert f([5.0, 5.0, 1.0, 1.0, 2.0, 2.0], steps=2, warmup=1) == 3.0          # several launches per step are summed per step
     assert f([1.0, 2.0, 3.0], steps=2, warmup=2) is None and f([], 3, 1) is None and f([1.0, 2.0], 0, 2) is None
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_large_ones(tmp_path, monkeypatch):
+    import numpy as np
+    import pytest
+    import torch
+    import bench
+    monkeypatch.setattr(bench, "DUMP_WHOLE_BYTES", 4096)
+    monkeypatch.setattr(bench, "DUMP_RAYS", 16)
+    g = torch.Generator().manual_seed(0)
+    out = dict(rgb=torch.rand(1, 100, 3, generator=g), alpha=torch.rand(1, 100, 32, generator=g).bfloat16(),
+               density=torch.rand(1, 100, 32, 2, generator=g, dtype=torch.float64), idx=torch.tensor([3]), note="not an array")
+    nbytes = bench.dump_outputs(str(tmp_path / "a"), out, 100)
+    got = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    assert sorted(got) == ["alpha", "density", "idx", "rgb", "sample_ray_idx"]
+    assert nbytes == sum(a.nbytes for a in got.values())
+    pick = got["sample_ray_idx"].astype(np.int64)
+    assert len(pick) == 16 and len(set(pick)) == 16 and list(pick) == sorted(pick)
+    assert got["rgb"].dtype == np.float32 and np.array_equal(got["rgb"], out["rgb"].numpy())              # small: whole
+    assert got["alpha"].dtype == np.float32 and np.array_equal(got["alpha"], out["alpha"].float()[:, pick].numpy())
+    assert got["density"].dtype == np.float64 and np.array_equal(got["density"], out["density"][:, pick].numpy())
+    assert got["idx"].dtype == np.float64 and got["idx"].tolist() == [3.0]
+    bench.dump_outputs(str(tmp_path / "b"), out, 100)                                                  # same arguments, same files
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / (k + ".npy"))) for k, a in got.items())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 1024)
+    with pytest.raises(ValueError, match="limit"):
+        bench.dump_outputs(str(tmp_path / "c"), out, 100)
