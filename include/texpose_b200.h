@@ -429,6 +429,24 @@ int tp_peer_allreduce_mean(void* const* windows, int world, int rank, int64_t n_
                            int grid_ctas, int64_t timeout_ms, void* stream);
 int tp_peer_status(const void* window, uint32_t* status_host);
 
+/* The same exchange with a device-held epoch, so that it can be captured in a CUDA graph (a capture freezes the host epoch
+ * argument of tp_peer_allreduce_mean and the host-chosen buffer of the pack).  Together the two calls replace "write buffer
+ * (epoch & 1), then tp_peer_allreduce_mean(epoch)":
+ *   tp_peer_stage copies src[0:n] into data buffer (e+1)&1 of the LOCAL window, e = the window's device epoch (header byte
+ *   768, 0 after create), and advances the device epoch to e+1 (16-byte vectors, local HBM only, never waits);
+ *   tp_peer_allreduce_mean_dev is tp_peer_allreduce_mean with `epoch` read from the local window's device epoch: publish,
+ *   bounded wait, rank-order sum / world -> out, NaN in `out` + the failed epoch in the status word on a timeout.
+ * Caller: one tp_peer_stage, then one tp_peer_allreduce_mean_dev, per exchange, on one stream, and the same number of
+ * exchanges on every rank (eager calls and graph replays count alike: they advance one counter); a window is driven either
+ * by this pair or by tp_peer_allreduce_mean with host epochs, never both.  src: local, 16-byte aligned, >= n floats.
+ * n_floats must be the n the window was sized for (tp_peer_window_bytes(n)): it places data buffer 1, and the stage writes
+ * there without a bounds check.
+ * Arguments as above; TP_ERR_BAD_ARG for null pointers, n < 0 or a rank outside the world, TP_ERR_ALIGN for a window that is
+ * not 256-byte aligned or an `src` / `out` that is not 16-byte aligned. */
+int tp_peer_stage(void* window, int64_t n_floats, const float* src, void* stream);
+int tp_peer_allreduce_mean_dev(void* const* windows, int world, int rank, int64_t n_floats, float* out, int grid_ctas,
+                               int64_t timeout_ms, void* stream);
+
 /* Completion barrier over the same windows (no data): rank publishes `epoch` (1, 2, ...) to every peer's header and waits
  * for every peer's.  Stream-ordered after a tp_render_fused_forward launch whose output pointers address the root rank's
  * window, it makes that rank's row block of the frame visible to the root (one-frame multi-GPU render, SURVEY 8e: "row

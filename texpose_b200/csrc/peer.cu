@@ -18,6 +18,18 @@
 //   parity: a peer can only start overwriting buffer e&1 at step e+2, and it cannot pass step e+1's wait before this
 //   rank has published e+1, which it does after finishing the reads of step e (stream order) -- no trailing barrier.
 //
+// Device-held epoch (CUDA-graph capturable exchange): the epoch above is a host argument, which a graph capture freezes.
+// The header also holds epoch u32 at byte 768 (the window's device epoch, 0 after create) and stage_done u32 at byte 772
+// (CTA completion counter of tp_peer_stage, 0 between launches).  The pair tp_peer_stage + tp_peer_allreduce_mean_dev
+// replaces step 1 and the epoch argument:
+//   1'. tp_peer_stage copies the caller's gradients into buffer (e+1)&1 of the OWN window, e = the device epoch, then the
+//       last CTA to finish stores e+1 (every CTA reads e before it counts itself done; no CTA waits for another);
+//   2-4. tp_peer_allreduce_mean_dev runs the same kernel body with epoch = the local window's device epoch.
+//   Invariants: epochs still count 1, 2, 3, ... identically on every rank (one stage per exchange, on every rank); eager
+//   calls and graph replays of the pair advance the same counter, so they interleave freely; the parity argument above is
+//   unchanged, since the stage of step e+2 is stream-ordered after this rank's reduce of step e+1; no kernel waits for its
+//   own grid.  A window is driven either by host epochs or by its device epoch, never both (they share the arrive slots).
+//
 // The window is the one driver object the library creates (like a communicator): tp_peer_window_create / _destroy,
 // _export / _import / _release are host calls made once at set-up; the per-step call allocates nothing.
 #include "common.cuh"
@@ -29,6 +41,8 @@ constexpr int kMaxWorld = 16;
 constexpr int64_t kHeaderBytes = 1024;
 constexpr int kStatusWord = 128;   // u32 index of the status word inside the header (byte 512)
 constexpr int kBarrierSlot0 = 32;  // u32 index of the barrier slots [16] (tp_peer_barrier; separate from the exchange's arrive[16])
+constexpr int kEpochWord = 192;    // u32 index of the device epoch (byte 768): tp_peer_stage advances it, _allreduce_mean_dev reads it
+constexpr int kStageDone = 193;    // u32 index of tp_peer_stage's CTA completion counter (byte 772)
 
 struct Windows {
   uint8_t* base[kMaxWorld];
@@ -76,8 +90,9 @@ __device__ __forceinline__ void reduce_slices(const Windows& w, int64_t data_off
   }
 }
 
-__global__ void __launch_bounds__(256) peer_allreduce_mean_kernel(const Windows w, int world, int rank, int64_t n4, int64_t cap_bytes,
-                                                                  uint32_t epoch, float* out, unsigned long long timeout_ns) {
+// Steps 2-4 of one exchange; the two kernels below differ only in where `epoch` comes from.
+__device__ __forceinline__ void allreduce_mean_body(const Windows& w, int world, int rank, int64_t n4, int64_t cap_bytes,
+                                                    uint32_t epoch, float* out, unsigned long long timeout_ns) {
   uint32_t* my_hdr = reinterpret_cast<uint32_t*>(w.base[rank]);
   // 2. publish (one CTA): this rank's buffer of `epoch` was written by earlier work on this stream
   if (blockIdx.x == 0 && threadIdx.x < world) {
@@ -143,6 +158,43 @@ __global__ void __launch_bounds__(256) peer_allreduce_mean_kernel(const Windows 
   }
 }
 
+__global__ void __launch_bounds__(256) peer_allreduce_mean_kernel(const Windows w, int world, int rank, int64_t n4, int64_t cap_bytes,
+                                                                  uint32_t epoch, float* out, unsigned long long timeout_ns) {
+  allreduce_mean_body(w, world, rank, n4, cap_bytes, epoch, out, timeout_ns);
+}
+
+// The epoch is the local window's device epoch, stored by the tp_peer_stage launch that precedes this one on the stream
+// (kernel boundary: every CTA reads the same value, and nothing writes it while this grid runs).
+__global__ void __launch_bounds__(256) peer_allreduce_mean_dev_kernel(const Windows w, int world, int rank, int64_t n4,
+                                                                      int64_t cap_bytes, float* out, unsigned long long timeout_ns) {
+  const uint32_t epoch = *(reinterpret_cast<const volatile uint32_t*>(w.base[rank]) + kEpochWord);
+  allreduce_mean_body(w, world, rank, n4, cap_bytes, epoch, out, timeout_ns);
+}
+
+// Step 1': src[0:n] -> data buffer (e+1)&1 of the local window, then the device epoch becomes e+1.  Every CTA reads e once,
+// before it counts itself done; the last CTA to count itself done stores e+1 and re-arms the counter.  No CTA waits.
+__global__ void __launch_bounds__(256) peer_stage_kernel(uint8_t* win, int64_t n_floats, int64_t cap_bytes, const float* src) {
+  uint32_t* hdr = reinterpret_cast<uint32_t*>(win);
+  __shared__ uint32_t e_s;
+  if (threadIdx.x == 0) e_s = *reinterpret_cast<volatile uint32_t*>(hdr + kEpochWord);
+  __syncthreads();
+  const uint32_t e = e_s;
+  float* dst = reinterpret_cast<float*>(win + kHeaderBytes + (int64_t)((e + 1u) & 1u) * cap_bytes);
+  const int64_t n4 = n_floats / 4;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  for (int64_t i = tid; i < n4; i += stride) reinterpret_cast<float4*>(dst)[i] = reinterpret_cast<const float4*>(src)[i];
+  if (tid < n_floats - n4 * 4) dst[n4 * 4 + tid] = src[n4 * 4 + tid];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(hdr + kStageDone, 1u) == gridDim.x - 1) {
+      *reinterpret_cast<volatile uint32_t*>(hdr + kEpochWord) = e + 1u;
+      *reinterpret_cast<volatile uint32_t*>(hdr + kStageDone) = 0u;
+    }
+  }
+}
+
 // Completion barrier over the windows' headers (no data): publish `epoch` into slot `rank` of every peer's header, then wait
 // until every peer's slot in the LOCAL header has reached it.  Used after the fused render launch whose compositing epilogue
 // stored this rank's row block of the frame straight into the root rank's window: when the root passes the barrier, every
@@ -170,6 +222,15 @@ __global__ void peer_barrier_kernel(const Windows w, int world, int rank, uint32
 }
 
 inline int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
+
+// host array of `world` window pointers -> kernel argument; every window must be non-null and 256-byte aligned
+inline int load_windows(void* const* windows, int world, Windows* w) {
+  for (int p = 0; p < kMaxWorld; ++p) {
+    w->base[p] = p < world ? static_cast<uint8_t*>(windows[p]) : nullptr;
+    if (p < world && (w->base[p] == nullptr || (reinterpret_cast<uintptr_t>(w->base[p]) & 255u) != 0)) return TP_ERR_ALIGN;
+  }
+  return TP_OK;
+}
 
 }  // namespace
 
@@ -236,10 +297,7 @@ TP_API int tp_peer_allreduce_mean(void* const* windows, int world, int rank, int
     return TP_ERR_BAD_ARG;
   if ((reinterpret_cast<uintptr_t>(out) & 15u) != 0) return TP_ERR_ALIGN;
   Windows w;
-  for (int p = 0; p < kMaxWorld; ++p) {
-    w.base[p] = p < world ? static_cast<uint8_t*>(windows[p]) : nullptr;
-    if (p < world && (w.base[p] == nullptr || (reinterpret_cast<uintptr_t>(w.base[p]) & 255u) != 0)) return TP_ERR_ALIGN;
-  }
+  if (int rc = load_windows(windows, world, &w)) return rc;
   if (n_floats == 0) return TP_OK;
   const int64_t n4 = (n_floats + 3) / 4;   // buffers are padded to 256 B, `out` must hold round_up(n,4) floats
   int grid = grid_ctas > 0 ? grid_ctas : tp_grid_for(n4, 256, 2);
@@ -249,13 +307,35 @@ TP_API int tp_peer_allreduce_mean(void* const* windows, int world, int rank, int
   return tp_launch_status();
 }
 
+TP_API int tp_peer_stage(void* window, int64_t n_floats, const float* src, void* stream) {
+  if (window == nullptr || src == nullptr || n_floats < 0) return TP_ERR_BAD_ARG;
+  if ((reinterpret_cast<uintptr_t>(window) & 255u) != 0 || (reinterpret_cast<uintptr_t>(src) & 15u) != 0) return TP_ERR_ALIGN;
+  if (n_floats == 0) return TP_OK;
+  peer_stage_kernel<<<tp_grid_for((n_floats + 3) / 4, 256, 2), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<uint8_t*>(window), n_floats, tp_peer_capacity_bytes(n_floats), src);
+  return tp_launch_status();
+}
+
+TP_API int tp_peer_allreduce_mean_dev(void* const* windows, int world, int rank, int64_t n_floats, float* out, int grid_ctas,
+                                      int64_t timeout_ms, void* stream) {
+  if (windows == nullptr || out == nullptr || world < 1 || world > kMaxWorld || rank < 0 || rank >= world || n_floats < 0)
+    return TP_ERR_BAD_ARG;
+  if ((reinterpret_cast<uintptr_t>(out) & 15u) != 0) return TP_ERR_ALIGN;
+  Windows w;
+  if (int rc = load_windows(windows, world, &w)) return rc;
+  if (n_floats == 0) return TP_OK;
+  const int64_t n4 = (n_floats + 3) / 4;
+  int grid = grid_ctas > 0 ? grid_ctas : tp_grid_for(n4, 256, 2);
+  if (timeout_ms <= 0) timeout_ms = 10000;
+  peer_allreduce_mean_dev_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      w, world, rank, n4, tp_peer_capacity_bytes(n_floats), out, (unsigned long long)timeout_ms * 1000000ull);
+  return tp_launch_status();
+}
+
 TP_API int tp_peer_barrier(void* const* windows, int world, int rank, uint32_t epoch, int64_t timeout_ms, void* stream) {
   if (windows == nullptr || world < 1 || world > kMaxWorld || rank < 0 || rank >= world || epoch == 0) return TP_ERR_BAD_ARG;
   Windows w;
-  for (int p = 0; p < kMaxWorld; ++p) {
-    w.base[p] = p < world ? static_cast<uint8_t*>(windows[p]) : nullptr;
-    if (p < world && (w.base[p] == nullptr || (reinterpret_cast<uintptr_t>(w.base[p]) & 255u) != 0)) return TP_ERR_ALIGN;
-  }
+  if (int rc = load_windows(windows, world, &w)) return rc;
   if (timeout_ms <= 0) timeout_ms = 10000;
   peer_barrier_kernel<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(w, world, rank, epoch, (unsigned long long)timeout_ms * 1000000ull);
   return tp_launch_status();

@@ -160,15 +160,44 @@ def peer_allreduce_mean(window_ptrs: Sequence[int], rank: int, n_floats: int, ep
                 timeout_ms, st.cuda_stream)
 
 
+def peer_stage(window_ptr: int, n_floats: int, src: torch.Tensor, stream=None):
+    """Data buffer (e+1)&1 of the local window <- src[:n], then the window's device epoch e becomes e+1 (tp_peer_stage)."""
+    if not src.is_cuda or src.dtype != torch.float32 or not src.is_contiguous() or src.numel() < n_floats:
+        raise RuntimeError("peer_stage: `src` must be a contiguous CUDA fp32 tensor of at least n floats")
+    st = stream if stream is not None else torch.cuda.current_stream(src.device)
+    with torch.cuda.device(src.device):
+        _C.call("tp_peer_stage", window_ptr, n_floats, src.data_ptr(), st.cuda_stream)
+
+
+def peer_allreduce_mean_dev(window_ptrs: Sequence[int], rank: int, n_floats: int, out: torch.Tensor,
+                            grid_ctas: int = 0, timeout_ms: int = 0, stream=None):
+    """peer_allreduce_mean with the epoch read from the local window's device epoch (tp_peer_allreduce_mean_dev)."""
+    if not out.is_cuda or out.dtype != torch.float32 or out.numel() < (n_floats + 3) // 4 * 4:
+        raise RuntimeError("peer_allreduce_mean_dev: `out` must be a CUDA fp32 tensor of at least n rounded up to 4 floats")
+    arr = (ctypes.c_void_p * len(window_ptrs))(*window_ptrs)
+    st = stream if stream is not None else torch.cuda.current_stream(out.device)
+    with torch.cuda.device(out.device):
+        _C.call("tp_peer_allreduce_mean_dev", arr, len(window_ptrs), rank, n_floats, out.data_ptr(), grid_ctas,
+                timeout_ms, st.cuda_stream)
+
+
 class PeerGradExchange(GradBucket):
     """GradBucket whose exchange is ONE kernel over NVLink peer memory instead of a library allreduce.
 
     Set-up (once): every rank creates a window, the 64-byte IPC handles travel through `all_gather_object`, every rank opens
     its peers' windows.  Per step: one `cat` packs the gradients into the local window's buffer of the step's parity, one
     launch publishes / waits / reduces, `.grad`s become views of the reduced buffer.  All ranks must sit on one node with
-    peer access (NVLink / NVSwitch); anything else raises at set-up -- there is no silent fallback to the allreduce."""
+    peer access (NVLink / NVSwitch); anything else raises at set-up -- there is no silent fallback to the allreduce.
 
-    def __init__(self, params: Iterable[torch.nn.Parameter], group=None, timeout_ms: int = 10000):
+    capturable=True makes `allreduce_mean()` capturable in a CUDA graph (e.g. inside `train_graph.GraphedStep`, like
+    `torch.optim.Adam(capturable=True)`): the epoch and the parity buffer are then chosen on the device, not on the host.
+    Each call, eager or replayed, is one `cat` into a fixed local staging buffer, `tp_peer_stage` (copy into the window's
+    buffer of the next device epoch and advance it), `tp_peer_allreduce_mean_dev` into `flat`, and the views of `unpack()`.
+    Eager calls and replays advance the same device counter, so every rank must make the same sequence of exchanges --
+    counting GraphedStep's eager warm-up steps -- as it must make the same sequence of calls without a graph.  Without
+    capturable, a call made while the current stream is capturing raises: the host epoch would be frozen into the graph."""
+
+    def __init__(self, params: Iterable[torch.nn.Parameter], group=None, timeout_ms: int = 10000, capturable: bool = False):
         super().__init__(params)
         if not (dist.is_available() and dist.is_initialized()):
             raise RuntimeError("PeerGradExchange needs an initialised process group (use GradBucket for a single process)")
@@ -182,10 +211,21 @@ class PeerGradExchange(GradBucket):
         self.ptrs = [self.window.ptr if r == self.rank else self.window.open_peer(h) for r, h in enumerate(handles)]
         self.flat = torch.zeros((self.n + 3) // 4 * 4, dtype=torch.float32, device=dev)    # the reduced gradients land here
         self.epoch = 0
+        self.capturable = bool(capturable)
+        self.staging = torch.zeros_like(self.flat) if self.capturable else None
         torch.cuda.synchronize(dev)
         dist.barrier(group)          # every window exists, is zeroed and is open everywhere before the first publish
 
     def allreduce_mean(self, group=None):
+        if self.capturable:
+            self.pack(into=self.staging[:self.n])
+            peer_stage(self.window.ptr, self.n, self.staging)
+            peer_allreduce_mean_dev(self.ptrs, self.rank, self.n, self.flat, timeout_ms=self.timeout_ms)
+            self.unpack()
+            return
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError("PeerGradExchange.allreduce_mean() is being captured in a CUDA graph, which would freeze its "
+                               "host-chosen epoch: construct the exchange with capturable=True")
         self.epoch += 1
         self.pack(into=self.window.buffers[self.epoch & 1])
         peer_allreduce_mean(self.ptrs, self.rank, self.n, self.epoch, self.flat, timeout_ms=self.timeout_ms)

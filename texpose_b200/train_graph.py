@@ -16,6 +16,12 @@ Requirements (checked where they can be): the optimizer is capturable (`torch.op
 inputs from the static tensors, takes no data-dependent Python branch and makes no host read-back -- in `opt.b200` terms:
 `rng = 'torch'` (the in-kernel Philox mode draws its seed on the host) and no `nan_guard`; shapes are fixed.  The warm-up
 iterations are real training steps on the inputs present in the static buffers.
+
+Data-parallel: call the gradient exchange inside `fn` after `backward()`.  `parallel.PeerGradExchange(params, capturable=True)`
+keeps its epoch on the device, so every replay runs a new exchange and nothing NCCL-side is captured; its warm-up calls here are
+eager exchanges on the same counter, so every rank must build its GraphedStep (same `warmup`) and replay in the same sequence.
+A `PeerGradExchange` without `capturable` refuses to be captured.  `parallel.GradBucket` captures the NCCL allreduce instead; a
+process group whose communicator lives in a graph does not tear down cleanly.
 """
 from __future__ import annotations
 
