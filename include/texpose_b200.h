@@ -266,36 +266,26 @@ int tp_tc32_forward(const float* center, const float* ray, const float* depth, i
                     const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,
                     int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot, void* stream);
 
-/* One slot of the saved tile images -> row-major fp32 [S,256]. */
-int tp_tc_unpack_images(const void* images, int slot, int n_slots, int64_t S, float* out, void* stream);
-
 /* ---- tensor-core backward of the two heads on the saved tile images (K2b, bf16 mode) ------------------------- */
 
 /* out[i] (=/+=) sum_z partial[z*count + i], fixed order (second stage of every split reduction). */
 int tp_reduce_partials(const float* partial, int splits, int64_t count, float* out, int accumulate, void* stream);
 
-int tp_tc_bwd_num_chunks(void);              /* chunks of the transposed weight image the chain kernel streams (34) */
-int64_t tp_tc_dz_bytes(int64_t S);           /* bytes of the dz tile images: ceil(S/128) x 6 x 64 KB */
+int tp_tc_bwd_num_chunks(void);              /* chunks of the transposed weight image tp_tc_heads_backward streams (34) */
+int64_t tp_tc_dz_bytes(int64_t S);           /* bytes of the dz tile images tp_tc_heads_backward writes: ceil(S/128) x 6 x 64 KB */
 int tp_tc_dw_splits(int64_t S, int n_jobs);  /* split partials per job that tp_tc_dw_gemm writes */
 
-/* autograd of mlp_rgb[1..3] / mlp_trans[1..3] w.r.t. their inputs (layers/nerf_static_transient_light.py:118-134):
- * dz_rgb [S,3], dz_trans [S,5] = grads of the output layers' pre-activations; packed_bwd = tp_tc_pack_weights image of
- * {W3^T, W2^T, W1^T} of both heads (34 chunks, transpose flag); saved = activations of tp_tc_nerf_stl_forward.
- * Writes the dz tile images [tiles][6] = {rgb dz2, dz1, dz0, trans dz2, dz1, dz0}. */
-int tp_tc_backward_chain(const float* dz_rgb, const float* dz_trans, int64_t S, const void* packed_bwd,
-                         const void* saved, void* dz_images, void* stream);
-
 /* n_jobs (<= 8) weight-gradient GEMMs in one launch: job j computes dz[a_slots[j]]^T x[b_slots[j]] (256x256 fp32) over all
- * samples; partial is [splits][n_jobs][256][256] with splits = tp_tc_dw_splits(S, n_jobs).  a_slots/b_slots: HOST arrays.
+ * samples (staged backward: dz = images of tp_tc_chain_backward, x = images tp_tc32_forward saved); partial is
+ * [splits][n_jobs][256][256] with splits = tp_tc_dw_splits(S, n_jobs).  a_slots/b_slots: HOST arrays.
  * Reduce with tp_reduce_partials(partial, splits, n_jobs*65536, ...). */
 int tp_tc_dw_gemm(const void* a_images, int a_nslots, const void* b_images, int b_nslots, const int32_t* a_slots,
                   const int32_t* b_slots, int n_jobs, int64_t S, float* partial, int64_t partial_floats, int flags,
                   void* stream);
 
-/* Fused backward of both heads in five launches (replaces tp_tc_backward_chain + tp_tc_dw_gemm + the thin helpers): the dX chain
- * kernel also accumulates, on the tensor pipe, every thin gradient -- bias gradients, output-layer weight gradients, the xyz /
- * view-direction columns of mlp_rgb[0], per-image sums for the latent terms -- then two finish kernels and the six 256x256
- * weight-gradient GEMMs write the reference's parameter gradients (autograd of layers/nerf_static_transient_light.py:104-137
+/* Backward of both heads on the images tp_tc_nerf_stl_forward saved, in five launches: the dX chain kernel also accumulates,
+ * on the tensor pipe, every thin gradient -- bias gradients, output-layer weight gradients, the xyz / view-direction columns
+ * of mlp_rgb[0], per-image sums for the latent terms -- then two finish kernels and the six 256x256 weight-gradient GEMMs write the reference's parameter gradients (autograd of layers/nerf_static_transient_light.py:104-137
  * under the losses of model/nerf_adapt_st_gan.py:747-763) straight into caller tensors.
  * grads: HOST array of 16 DEVICE pointers {rgb dW0 [256,ld_r0], db0, dW1 [256,256], db1, dW2, db2, dW3 [3,256], db3 [3],
  * transient dW0 [256,ld_t0], db0, dW1, db1, dW2, db2, dW3 [5,256], db3 [5]}.  d_lat_* [B,n] or NULL.  B = images,
@@ -319,9 +309,6 @@ int tp_thin_colsum(const float* x, int64_t S, int C, float* out, float* workspac
 /* partial[blk][m][k] = sum_s thin[s][m] * x[s][k] for a thin fp32 operand [S,M], M in {1,3,5}; x = image slot. */
 int tp_tc_thin_dw(const float* thin, int M, const void* images, int slot, int n_slots, int64_t S, float* partial,
                   int64_t partial_floats, int* n_blocks_out, void* stream);
-
-/* row-major fp32 [S,256] -> bf16 tile image slot (interop / tests). */
-int tp_tc_pack_images(const float* in, int64_t S, void* images, int slot, int n_slots, void* stream);
 
 /* ---- fused patch gather + ray-wise losses + backward seeds (SURVEY 8 f2) ---------------------------------------- */
 

@@ -29,7 +29,7 @@ def test_c3_fused_backward_vs_oracle():
     opt, g = C3.graph(DEV)
     _C.launch_counts.clear()
     got, rand, loss, (zn, zf) = C3.cuda_step(opt, g, inp, slice(0, C3.B), DEV, seed=21)
-    assert _C.launch_counts.get("tp_tc_heads_backward", 0) == 1          # the fused tcgen05 backward, not the multi-kernel fallback
+    assert _C.launch_counts.get("tp_tc_heads_backward", 0) == 1          # the fused tcgen05 backward, not the staged kernels
     assert _C.launch_counts.get("tp_linear_backward_weight", 0) == 0     # ... and nothing on the fp32 SIMT path
     want, ref_loss, (ozn, ozf) = C3.oracle_step(g, inp, slice(0, C3.B), rand)
     assert torch.equal(zn, ozn) and torch.equal(zf, ozf)

@@ -898,30 +898,6 @@ __global__ void __launch_bounds__(256) ray_bias_kernel(const float* __restrict__
   }
 }
 
-
-// tile image [tiles][n_slots][k8=32][128 rows][8] bf16 -> row-major fp32 [S,256] (consumers: the fp32 SIMT kernels)
-__global__ void unpack_images_kernel(const uint8_t* __restrict__ images, int slot, int n_slots, long long S,
-                                     float* __restrict__ out) {
-  const long long total = ((S + 127) / 128) * 4096;     // 16-byte vectors
-  for (long long v = blockIdx.x * (long long)blockDim.x + threadIdx.x; v < total; v += (long long)gridDim.x * blockDim.x) {
-    const long long tile = v >> 12;
-    const int k8 = (int)((v >> 7) & 31), r = (int)(v & 127);
-    const long long s = tile * 128 + r;
-    if (s >= S) continue;
-    const uint4 q = *reinterpret_cast<const uint4*>(images + ((size_t)tile * n_slots + slot) * kABytes + k8 * 2048 + r * 16);
-    const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-    float f[8];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      f[2 * e] = __uint_as_float(w[e] << 16);
-      f[2 * e + 1] = __uint_as_float(w[e] & 0xffff0000u);
-    }
-    float4* o = reinterpret_cast<float4*>(out + s * 256 + k8 * 8);
-    o[0] = make_float4(f[0], f[1], f[2], f[3]);
-    o[1] = make_float4(f[4], f[5], f[6], f[7]);
-  }
-}
-
 }  // namespace tc
 
 TP_API int tp_tc_num_chunks(void) { return tc::kNumChunks; }
@@ -934,15 +910,6 @@ TP_API int64_t tp_tc_prof_offset(void) { return (int64_t)tp_num_sms() * (2 * tc:
 // save buffer: [tiles][7][64 KB] tile images, then [tiles][4][4 KB] ReLU bitmasks (tiles rounded up to whole super-tiles)
 TP_API int64_t tp_tc_save_bytes(int64_t S) {
   return ((S + 255) / 256) * 2 * (tc::kSaveSlots * (int64_t)tc::kABytes + tc::kMaskBitSlots * (int64_t)tc::kMaskBitBytes);
-}
-
-TP_API int tp_tc_unpack_images(const void* images, int slot, int n_slots, int64_t S, float* out, void* stream) {
-  if (!images || !out) return TP_ERR_BAD_ARG;
-  if (slot < 0 || slot >= n_slots || S < 0) return TP_ERR_BAD_SHAPE;
-  if (S == 0) return TP_OK;
-  tc::unpack_images_kernel<<<tp_grid_for(((S + 127) / 128) * 4096, 256, 8), 256, 0, (cudaStream_t)stream>>>(
-      reinterpret_cast<const uint8_t*>(images), slot, n_slots, S, out);
-  return tp_launch_status();
 }
 
 TP_API int tp_tc_pack_weights(const int64_t* chunk_desc, int n_chunks, void* packed, void* stream) {

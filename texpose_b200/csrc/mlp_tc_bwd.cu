@@ -1,16 +1,21 @@
 // K2b (bf16 mode): tensor-core backward of the two NeRF heads (trunk frozen, layers/nerf_static_transient_light.py:34,87).
 //
-// autograd of the reference replays ~20 aten kernels per head layer; here the backward is three kinds of kernels working on
-// the bf16 *tile images* ([32 k8][128 rows][8], 64 KB per 128 samples) that the fused forward saved:
+// autograd of the reference replays ~20 aten kernels per head layer; here the backward works on the bf16 *tile images*
+// ([32 k8][128 rows][8], 64 KB per 128 samples) and ReLU bitmasks that the forward saved.  tp_tc_heads_backward (five launches,
+// the yaml's 3 x 256 heads after the lock-step forward):
 //
-//   backward_chain_kernel   dz3 -> dh3 = dz3 W3 -> dz2 = dh3*[h3>0] -> dh2 = dz2 W2 -> dz1 -> dh1 = dz1 W1 -> dz0   (per head)
-//                           tcgen05 M=128 x N=256 MMAs, weights (transposed images) streamed like the forward, the ReLU mask
-//                           comes from the saved activation tile (bulk-loaded to SMEM), every dz tile is bulk-stored as an
-//                           image for the weight-gradient GEMMs.  HBM-bound: 64 KB in + 64 KB out per stage and tile.
-//   dw_gemm_kernel          dW[n,k] = sum_s dz[s,n] x[s,k]: both operands are read straight from the tile images as MN-major
-//                           UMMA operands (the image of a [s x n] K-major tile IS the image of an [n x s] MN-major tile), full
-//                           256x256 fp32 accumulator in TMEM (2 x M=128), split over tiles across CTAs, fixed-order reduce.
-//   image_colsum / thin_dw  bias gradients and the 3/5-row output-layer and xyz-column weight gradients (HBM-bound helpers).
+//   backward_chain_fused_kernel  dz3 -> dh3 = dz3 W3 -> dz2 = dh3*[h3>0] -> dh2 = dz2 W2 -> dz1 -> dh1 = dz1 W1 -> dz0 (per head)
+//                                tcgen05 M=128 x N=256 MMAs, weights (transposed images) streamed like the forward, every dz
+//                                tile stored as an image for the weight-gradient GEMMs; every thin gradient (biases, output
+//                                layers, xyz / view columns, per-image sums) accumulated on the tensor pipe in the same kernel.
+//   bwd_finish1/2_kernel         fixed-order reduction of the per-CTA thin partials, latent and layer-0 closed forms.
+//   dw_gemm_kernel               dW[n,k] = sum_s dz[s,n] x[s,k]: both operands are read straight from the tile images as
+//                                MN-major UMMA operands (the image of a [s x n] K-major tile IS the image of an [n x s] MN-major
+//                                tile), full 256x256 fp32 accumulator in TMEM (2 x M=128), split over tiles across CTAs;
+//                                dw_reduce_kernel reduces the splits in fixed order.
+//
+// dw_gemm_kernel and the HBM-bound helpers thin_dw / image_ray_sums / thin_colsum also serve the staged backward
+// (csrc/mlp_tc_chain.cu, any 256-wide head depth, and batches whose images are too small for the fused chain kernel).
 #include "tc_common.cuh"
 #include "../../include/texpose_b200.h"
 
@@ -29,9 +34,6 @@ constexpr int kStages = 4;
 constexpr uint32_t kOffA = 0;                        // dz operand tile (64 KB)
 constexpr uint32_t kOffM = kABytes;                  // saved activation of the current stage (ReLU mask source, 64 KB)
 constexpr uint32_t kOffZ = 2 * kABytes;              // dz3 tiles of the two heads: 2 x [2 k8][128][8] (4 KB each)
-constexpr uint32_t kOffRing = kOffZ + 8192;
-constexpr uint32_t kOffBar = kOffRing + kStages * kChunkBytes;
-constexpr uint32_t kSmemBytes = kOffBar + 128;
 constexpr int kNumStagesPerTile = 6;                 // per head: output layer (K=16), hidden 2, hidden 1
 constexpr int kBwdChunks = 34;                       // (1 + 8 + 8) x 2
 constexpr int kFwdSlots = 7, kDzSlots = 6;
@@ -49,194 +51,12 @@ struct BwdParams {
   uint8_t* dz_out;            // [tiles][6][64 KB]: rgb dz2,dz1,dz0, trans dz2,dz1,dz0
 };
 
-__global__ void __launch_bounds__(kThreads, 1) backward_chain_kernel(const BwdParams p) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  const uint32_t sbase = smem_u32(smem);
-  const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
-  const int lane = threadIdx.x & 31;
-  const uint32_t bar0 = sbase + kOffBar;
-  auto bar_full = [&](int s) { return bar0 + 8 * s; };
-  auto bar_empty = [&](int s) { return bar0 + 8 * (kStages + s); };
-  const uint32_t bar_acc = bar0 + 8 * (2 * kStages), bar_ready = bar_acc + 8, bar_mask = bar_acc + 16;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + kOffBar + 8 * (2 * kStages + 3));
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; ++s) {
-      mbar_init(bar_full(s), 1);
-      mbar_init(bar_empty(s), 1);
-    }
-    mbar_init(bar_acc, 1);
-    mbar_init(bar_ready, 256);
-    mbar_init(bar_mask, 1);
-    fence_barrier_init();
-  }
-  if (warp == 9) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(256)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const long long n_tiles = (p.S + 127) / 128;
-
-  if (warp == 8) {
-    // ================================================================ weight producer
-    uint32_t stage = 0, phase = 0;
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      int c = 0;
-      for (int s = 0; s < kNumStagesPerTile; ++s) {
-        const int nch = (s % 3 == 0) ? 1 : 8;
-        for (int j = 0; j < nch; ++j, ++c) {
-          const uint32_t bytes = (s % 3 == 0) ? kChunkBytes / 2 : kChunkBytes;
-          mbar_wait(bar_empty(stage), phase ^ 1);
-          if (elect_one_sync()) {
-            mbar_expect_tx(bar_full(stage), bytes);
-            bulk_g2s(sbase + kOffRing + stage * kChunkBytes, p.packed + (size_t)c * kChunkBytes, bytes, bar_full(stage));
-          }
-          __syncwarp();
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 9) {
-    // ================================================================ MMA issuer
-    uint32_t stage = 0, phase = 0, ready_ph = 0;
-    const uint32_t idesc = umma_idesc(128, 256);
-    constexpr uint32_t kHi = (128u >> 4) | (1u << 14);
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      for (int s = 0; s < kNumStagesPerTile; ++s) {
-        const int nch = (s % 3 == 0) ? 1 : 8;
-        for (int c = 0; c < nch; ++c) {
-          mbar_wait(bar_full(stage), phase);
-          if (c == 0) {
-            mbar_wait(bar_ready, ready_ph);
-            ready_ph ^= 1;
-          }
-          tc_fence_after();
-          const uint32_t wsm = sbase + kOffRing + stage * kChunkBytes;
-          if (elect_one_sync()) {
-            const uint32_t b_lo = (wsm >> 4) | ((4096u >> 4) << 16);
-            if (s % 3 == 0) {   // K=16 step on the dz3 tile of this head
-              const uint32_t a_lo = ((sbase + kOffZ + (s / 3) * 4096) >> 4) | ((2048u >> 4) << 16);
-              umma_bf16_lohi(tmem_base, a_lo, kHi, b_lo, kHi, idesc, 0u);
-            } else {
-              const uint32_t a_lo = ((sbase + kOffA + c * 4 * 2048) >> 4) | ((2048u >> 4) << 16);
-              umma_bf16_lohi(tmem_base, a_lo, kHi, b_lo, kHi, idesc, c > 0 ? 1u : 0u);
-              umma_bf16_lohi(tmem_base, a_lo + (4096u >> 4), kHi, b_lo + (8192u >> 4), kHi, idesc, 1u);
-            }
-            if (c == nch - 1) umma_commit(bar_acc);
-            umma_commit(bar_empty(stage));
-          }
-          __syncwarp();
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else {
-    // ================================================================ epilogue warps: mask, convert, store dz images
-    const int q = warp & 3, half = warp >> 2, row = q * 32 + lane;
-    const uint32_t a_smem = sbase + kOffA, m_smem = sbase + kOffM;
-    const uint32_t tmem_d = tmem_base + ((uint32_t)(q * 32) << 16) + half * 128;
-    uint32_t acc_ph = 0, mask_ph = 0;
-    bool store_pending = false;
-    // first mask tile of this CTA
-    if (threadIdx.x == 32 && (long long)blockIdx.x < n_tiles) {
-      mbar_expect_tx(bar_mask, kABytes);
-      bulk_g2s(m_smem, p.saved + ((size_t)blockIdx.x * kFwdSlots + kMaskSlot[0]) * kABytes, kABytes, bar_mask);
-    }
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      // dz3 tiles of both heads: [2 k8][128 rows][8] bf16, columns >= 3 / 5 zero
-      if (half == 0) {
-        const long long s = tile * 128 + row;
-        float zr[3] = {0.f, 0.f, 0.f}, zt[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
-        if (s < p.S) {
-#pragma unroll
-          for (int c = 0; c < 3; ++c) zr[c] = p.dz_rgb[s * 3 + c];
-#pragma unroll
-          for (int c = 0; c < 5; ++c) zt[c] = p.dz_trans[s * 5 + c];
-        }
-        const uint32_t z0 = sbase + kOffZ + row * 16;
-        st_shared_v4(z0, pack_bf16(zr[0], zr[1]), pack_bf16(zr[2], 0.f), 0u, 0u);
-        st_shared_v4(z0 + 2048, 0u, 0u, 0u, 0u);
-        st_shared_v4(z0 + 4096, pack_bf16(zt[0], zt[1]), pack_bf16(zt[2], zt[3]), pack_bf16(zt[4], 0.f), 0u);
-        st_shared_v4(z0 + 4096 + 2048, 0u, 0u, 0u, 0u);
-      }
-      fence_proxy_async_smem();
-      tc_fence_before();
-      mbar_arrive(bar_ready);
-
-      for (int s = 0; s < kNumStagesPerTile; ++s) {
-        mbar_wait(bar_acc, acc_ph);
-        acc_ph ^= 1;
-        mbar_wait(bar_mask, mask_ph);
-        mask_ph ^= 1;
-        tc_fence_after();
-        if (store_pending) {          // the previous dz image store must have finished reading A
-          if (threadIdx.x == 0) bulk_wait_read();
-          named_bar_sync(1, 256);
-          store_pending = false;
-        }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          uint32_t v[32];
-          TP_TMEM_LD32(tmem_d + j * 32, v);
-          TP_TMEM_WAIT32(v);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const uint32_t off = (uint32_t)(half * 16 + j * 4 + i) * 2048 + row * 16;
-            uint32_t m0, m1, m2, m3;
-            asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(m0), "=r"(m1), "=r"(m2), "=r"(m3) : "r"(m_smem + off));
-            const uint32_t mw[4] = {m0, m1, m2, m3};
-            uint32_t o[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const float lo = (mw[e] & 0xffffu) ? __uint_as_float(v[i * 8 + 2 * e]) : 0.f;
-              const float hi = (mw[e] >> 16) ? __uint_as_float(v[i * 8 + 2 * e + 1]) : 0.f;
-              o[e] = pack_bf16(lo, hi);
-            }
-            st_shared_v4(a_smem + off, o[0], o[1], o[2], o[3]);
-          }
-        }
-        fence_proxy_async_smem();
-        named_bar_sync(1, 256);           // every thread finished reading M and writing A
-        if (threadIdx.x == 0) {
-          bulk_s2g(p.dz_out + ((size_t)tile * kDzSlots + s) * kABytes, a_smem, kABytes);
-          bulk_commit();
-        }
-        store_pending = true;
-        if (threadIdx.x == 32) {          // prefetch the next stage's mask tile (possibly of this CTA's next tile)
-          const bool last = s == kNumStagesPerTile - 1;
-          const long long nt = last ? tile + gridDim.x : tile;
-          if (nt < n_tiles) {
-            mbar_expect_tx(bar_mask, kABytes);
-            bulk_g2s(m_smem, p.saved + ((size_t)nt * kFwdSlots + kMaskSlot[last ? 0 : s + 1]) * kABytes, kABytes, bar_mask);
-          }
-        }
-        if (s != kNumStagesPerTile - 1) {
-          tc_fence_before();
-          mbar_arrive(bar_ready);
-        }
-      }
-    }
-    if (threadIdx.x == 0) bulk_wait_all();
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 9) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256) : "memory");
-  }
-}
-
 // UMMA instruction descriptor with both operands MN-major (bits 15, 16)
 __host__ __device__ constexpr uint32_t umma_idesc_mn(int M, int N) { return umma_idesc(M, N) | (1u << 15) | (1u << 16); }
 
 // ------------------------------------------------------------------------------------------ fused chain + thin gradients
 //
-// Same dX chain, plus every "thin" gradient of the two heads, computed by the otherwise idle tensor pipe while the operands are
+// The dX chain, plus every "thin" gradient of the two heads, computed by the otherwise idle tensor pipe while the operands are
 // in SMEM anyway (the chain is HBM-bound).  All of them have the form  D[n, j] = sum_s X[s, n] * T[s, j]  with X a 128 x 256 tile
 // image already resident (a dz tile in A, or the saved h3 tile in M) used as an MN-major A operand (2 x M=128 feature halves),
 // and T a thin bf16 tile [128 samples x 16|48] built by the epilogue warps, used as an MN-major B operand:
@@ -1097,23 +917,6 @@ __global__ void __launch_bounds__(256) thin_colsum_kernel(const float* __restric
   }
 }
 
-// row-major fp32 [S,256] -> tile image slot (test / interop helper)
-__global__ void pack_images_kernel(const float* __restrict__ in, long long S, uint8_t* __restrict__ images, int slot,
-                                   int n_slots) {
-  const long long total = ((S + 127) / 128) * 4096;
-  for (long long v = blockIdx.x * (long long)blockDim.x + threadIdx.x; v < total; v += (long long)gridDim.x * blockDim.x) {
-    const long long tile = v >> 12;
-    const int k8 = (int)((v >> 7) & 31), r = (int)(v & 127);
-    const long long s = tile * 128 + r;
-    uint4 q = make_uint4(0u, 0u, 0u, 0u);
-    if (s < S) {
-      const float* x = in + s * 256 + k8 * 8;
-      q = make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
-    }
-    *reinterpret_cast<uint4*>(images + ((size_t)tile * n_slots + slot) * kABytes + k8 * 2048 + r * 16) = q;
-  }
-}
-
 }  // namespace tcb
 
 TP_API int tp_tc_bwd_num_chunks(void) { return tcb::kBwdChunks; }
@@ -1124,28 +927,6 @@ TP_API int tp_tc_dw_splits(int64_t S, int n_jobs) {
   if (splits < 1) splits = 1;
   if (splits > n_tiles) splits = n_tiles;
   return (int)splits;
-}
-
-TP_API int tp_tc_backward_chain(const float* dz_rgb, const float* dz_trans, int64_t S, const void* packed_bwd,
-                                const void* saved, void* dz_images, void* stream) {
-  if (!dz_rgb || !dz_trans || !packed_bwd || !saved || !dz_images) return TP_ERR_BAD_ARG;
-  if (S < 0) return TP_ERR_BAD_SHAPE;
-  if (((uintptr_t)packed_bwd & 15) || ((uintptr_t)saved & 15) || ((uintptr_t)dz_images & 15)) return TP_ERR_ALIGN;
-  if (!tp_device_is_sm100()) return TP_ERR_ARCH;
-  if (S == 0) return TP_OK;
-  tcb::BwdParams p;
-  p.dz_rgb = dz_rgb; p.dz_trans = dz_trans; p.S = S;
-  p.packed = reinterpret_cast<const uint8_t*>(packed_bwd);
-  p.saved = reinterpret_cast<const uint8_t*>(saved);
-  p.dz_out = reinterpret_cast<uint8_t*>(dz_images);
-  const long long n_tiles = (S + 127) / 128;
-  int grid = tp_num_sms();
-  if (n_tiles < grid) grid = (int)n_tiles;
-  cudaError_t e = cudaFuncSetAttribute(tcb::backward_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)tcb::kSmemBytes);
-  if (e != cudaSuccess) return (int)e;
-  tcb::backward_chain_kernel<<<grid, tcb::kThreads, tcb::kSmemBytes, (cudaStream_t)stream>>>(p);
-  return tp_launch_status();
 }
 
 TP_API int tp_tc_dw_gemm(const void* a_images, int a_nslots, const void* b_images, int b_nslots, const int32_t* a_slots,
@@ -1210,15 +991,6 @@ TP_API int tp_tc_thin_dw(const float* thin, int M, const void* images, int slot,
   if (M == 1) tcb::thin_dw_kernel<1><<<(unsigned)blocks, 256, 0, st>>>(thin, img, slot, n_slots, S, tpb, partial);
   else if (M == 3) tcb::thin_dw_kernel<3><<<(unsigned)blocks, 256, 0, st>>>(thin, img, slot, n_slots, S, tpb, partial);
   else tcb::thin_dw_kernel<5><<<(unsigned)blocks, 256, 0, st>>>(thin, img, slot, n_slots, S, tpb, partial);
-  return tp_launch_status();
-}
-
-TP_API int tp_tc_pack_images(const float* in, int64_t S, void* images, int slot, int n_slots, void* stream) {
-  if (!in || !images) return TP_ERR_BAD_ARG;
-  if (S < 0 || slot < 0 || slot >= n_slots) return TP_ERR_BAD_SHAPE;
-  if (S == 0) return TP_OK;
-  tcb::pack_images_kernel<<<tp_grid_for(((S + 127) / 128) * 4096, 256, 8), 256, 0, (cudaStream_t)stream>>>(
-      in, S, reinterpret_cast<uint8_t*>(images), slot, n_slots);
   return tp_launch_status();
 }
 

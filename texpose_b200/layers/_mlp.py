@@ -206,21 +206,6 @@ def mlp_backward(cfg: MLPConfig, sv: _Saved, S: int, per_image: int, feat_p, rgb
     return g_feat_layers, g_rgb_layers, g_trans_layers, d_lat_trans, d_lat_light
 
 
-def _inputs_from_images(cfg: MLPConfig, sv: _Saved, S: int, per_image: int):
-    """Layer inputs for the backward from the activations the fused bf16 forward saved (bf16 values, fp32 storage)."""
-    from .. import mlp_tc
-    geom = sv.geom
-    lt, ll = sv.lat
-    feat = mlp_tc.unpack_image(sv.images, mlp_tc.SLOT_FEAT, S)
-    xyz = ops.points_from_depth(geom["center"], geom["ray"], geom["depth"]).view(S, 3)
-    first = [(feat, 1, feat.shape[1]), geom["view_seg"](), (xyz, 1, 3), (ll, per_image, cfg.n_latent_light)]
-    sv.rgb_in = [first] + [[(mlp_tc.unpack_image(sv.images, mlp_tc.SLOT_RGB_H1 + i, S), 1, 256)] for i in range(3)]
-    first_t = [(feat, 1, feat.shape[1]), (lt, per_image, cfg.n_latent_trans)]
-    sv.trans_in = [first_t] + [[(mlp_tc.unpack_image(sv.images, mlp_tc.SLOT_TRANS_H1 + i, S), 1, 256)] for i in range(3)]
-    sv.feat, sv.trunk_in = feat, []
-    sv.images = None
-
-
 def run_mlp(cfg: MLPConfig, geom, lat_trans, lat_light, *params):
     """NerfMLP.apply, except that an empty sample set (an eval frame whose mask prior selects no pixel, an empty shard)
     returns empty outputs of the reference's shapes without a launch -- as the reference's torch ops do."""
@@ -264,9 +249,11 @@ class NerfMLP(torch.autograd.Function):
                 use_tc32, single, use_tc = True, 1, False
         staged_train = False
         if sv is not None and cfg.stl and not trunk_grad and cfg.precision in ("bf16", "auto") and geom.get("mode") == "rays":
-            from .. import mlp_tc, mlp_tc32
-            # training on an architecture the lock-step kernel / fused backward are not specialised for: staged kernels
-            staged_train = (not mlp_tc.supported(cfg, feat_p, rgb_p, trans_p)) and mlp_tc32.supported(cfg, feat_p, rgb_p, trans_p) \
+            from .. import mlp_tc, mlp_tc32, mlp_tc_bwd
+            # training on the staged kernels: an architecture the lock-step kernel / fused backward are not specialised for, or
+            # images so small that one CTA's tile range of the fused backward would touch more than four of them
+            lockstep = mlp_tc.supported(cfg, feat_p, rgb_p, trans_p) and mlp_tc_bwd.fused_supported(S, per_image)
+            staged_train = not lockstep and mlp_tc32.supported(cfg, feat_p, rgb_p, trans_p) \
                 and (len(rgb_p) - 1) + (len(trans_p) - 1) + 1 <= 16
         if staged_train:
             from .. import mlp_tc32
@@ -309,8 +296,8 @@ class NerfMLP(torch.autograd.Function):
         need = ctx.needs_input_grad[4:]
         g = lambda t: t.contiguous().float() if t is not None else None
         if getattr(sv, "images", None) is not None:
-            # bf16 mode: tensor-core backward on the tile images the fused forward saved (csrc/mlp_tc_bwd.cu), or -- architectures
-            # outside its fixed stage table -- the staged kernels (csrc/mlp_tc_chain.cu)
+            # bf16 mode: the backward of whichever kernels the forward chose -- the fused backward on the tile images the lock-step
+            # forward saved (csrc/mlp_tc_bwd.cu), or the staged kernels (csrc/mlp_tc_chain.cu)
             from .. import mlp_tc_bwd
             fn = mlp_tc_bwd.heads_backward_staged if getattr(sv, "staged", False) else mlp_tc_bwd.heads_backward
             gr, gt, d_lt, d_ll = fn(cfg, sv, S, ctx.per_image, rgb_p, trans_p, g(g_rgb), g(g_density),

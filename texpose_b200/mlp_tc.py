@@ -249,13 +249,3 @@ def render_fused(cfg, kinv, pinv, H, W, ray_idx, ray0, R, z_near, z_far, N, lat_
             cfg.L_view, ops._p(img_r), ops._p(img_t), float(min_uncert), *[dst(k) for k in RENDER_KEYS], ops._p(scratch),
             scratch.numel(), STATIC_ONLY if static_only else 0, ops._stream())
     return ret
-
-
-SLOT_FEAT, SLOT_RGB_H1, SLOT_TRANS_H1, N_SLOTS = 0, 1, 4, 7
-
-
-def unpack_image(images, slot: int, S: int) -> torch.Tensor:
-    """One saved activation (bf16 tile images) -> row-major fp32 [S,256]."""
-    out = torch.empty(S, _F, device=images.device)
-    _C.call("tp_tc_unpack_images", ops._p(images), slot, N_SLOTS, S, ops._p(out), ops._stream())
-    return out

@@ -1,4 +1,8 @@
-"""Host side of the tensor-core backward (csrc/mlp_tc_bwd.cu): transposed weight image, kernel sequencing.
+"""Host side of the tensor-core backward of the two heads (bf16 mode): transposed weight image, kernel sequencing.
+
+Two backwards, one per forward: `heads_backward` (csrc/mlp_tc_bwd.cu, tp_tc_heads_backward) after the lock-step forward, and
+`heads_backward_staged` (csrc/mlp_tc_chain.cu + the dW GEMM and thin helpers here) after the single-pass staged forward.
+NerfMLP.forward picks the forward, and with it the backward.
 
 Gradient sinks are the reference's: mlp_rgb.*, mlp_trans.*, the two latents (model/nerf_adapt_st_gan.py:56-69,108-127);
 the trunk is frozen (layers/nerf_static_transient_light.py:34).
@@ -12,10 +16,7 @@ import torch
 
 from . import _C, ops
 
-FWD_SLOTS, DZ_SLOTS = 7, 6
 last_profile_workspace = None       # (workspace tensor, float offset of the counters) of the last instrumented call
-# forward-save slots: 0 feat, 1-3 rgb h1..h3, 4-6 trans h1..h3; dz slots: rgb dz2,dz1,dz0, trans dz2,dz1,dz0
-_BIG_PAIRS = {"rgb": [(0, 2), (1, 1), (2, 0)], "trans": [(3, 5), (4, 4), (5, 0)]}      # (dz slot, x slot) for layers 2,1,0
 
 
 def _bwd_table(rgb_p, trans_p):
@@ -50,13 +51,6 @@ def pack_bwd(holder, rgb_p, trans_p):
     if holder is not None:
         holder._packed_bwd = (key, img, desc, where)
     return img
-
-
-def backward_chain(dz_rgb, dz_trans, S, packed_bwd, saved):
-    dz_images = torch.empty(_C.load().tp_tc_dz_bytes(S), dtype=torch.uint8, device=dz_rgb.device)
-    _C.call("tp_tc_backward_chain", ops._p(dz_rgb), ops._p(dz_trans), S, ops._p(packed_bwd), ops._p(saved),
-            ops._p(dz_images), ops._stream())
-    return dz_images
 
 
 def reduce_partials(partial, splits, count, out=None):
@@ -112,30 +106,15 @@ def thin_dw(thin, images, slot, n_slots, S):
     return reduce_partials(partial, nb.value, M * 256).view(M, 256)
 
 
-def unpack(images, slot, n_slots, S):
-    out = torch.empty(S, 256, device=images.device)
-    _C.call("tp_tc_unpack_images", ops._p(images), slot, n_slots, S, ops._p(out), ops._stream())
-    return out
-
-
 def fused_supported(S, per_image) -> bool:
+    """Whether tp_tc_heads_backward takes a batch: one CTA's contiguous tile range may touch at most four images."""
     return bool(_C.load().tp_tc_heads_backward_supported(S, per_image))
 
 
 def heads_backward(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans, need_lat_light):
-    """Returns (rgb layer grads [(dW,db)]*4, trans layer grads, d_lat_trans, d_lat_light).
-
-    Default: five launches (tp_tc_heads_backward).  The multi-kernel sequence below it is kept for batches whose images are
-    so small that one CTA's tile range would touch more than four of them, and as the cross-check in the tests
-    (TEXPOSE_BWD=unfused)."""
-    if os.environ.get("TEXPOSE_BWD", "fused") != "unfused" and fused_supported(S, per_image):
-        return heads_backward_fused(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans,
-                                    need_lat_light)
-    return heads_backward_unfused(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans,
-                                  need_lat_light)
-
-
-def heads_backward_fused(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans, need_lat_light):
+    """Backward of the yaml's 3 x 256 heads on the tile images the lock-step forward saved, in five launches
+    (tp_tc_heads_backward).  Returns (rgb layer grads [(dW,db)]*4, trans layer grads, d_lat_trans, d_lat_light).
+    The batch must satisfy fused_supported(S, per_image); NerfMLP.forward sends any other batch to the staged kernels."""
     dev = sv.rgb.device
     geom = sv.geom
     lt, ll = sv.lat
@@ -170,50 +149,13 @@ def heads_backward_fused(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density
     return pairs[:4], pairs[4:], d_lt, d_ll
 
 
-def heads_backward_unfused(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans, need_lat_light):
-    dev = sv.rgb.device
-    geom = sv.geom
-    lt, ll = sv.lat
-    B, R, N = geom["shape"]
-    dz_rgb = torch.empty(S, 3, device=dev)
-    dz_trans = torch.empty(S, 5, device=dev)
-    _C.call("tp_stl_output_grad", ops._p(sv.rgb), ops._p(sv.density), ops._p(sv.uncert), ops._p(g_rgb), ops._p(g_density),
-            ops._p(g_uncert), S, ops._p(dz_rgb), ops._p(dz_trans), None, ops._stream())
-    packed = pack_bwd(cfg.packed, rgb_p, trans_p)
-    dz = backward_chain(dz_rgb, dz_trans, S, packed, sv.images)
-    # ---- all six 256x256 weight gradients in one launch: layers 2,1,0 of the rgb head, then of the transient head
-    big = dw_gemm(dz, DZ_SLOTS, sv.images, FWD_SLOTS, _BIG_PAIRS["rgb"] + _BIG_PAIRS["trans"], S)
-    # per-ray column sums of every dz image: bias gradients (summed over rays) and the per-ray / per-image columns of layer 0
-    ray_sums = [image_ray_sums(dz, k, DZ_SLOTS, S, N) for k in range(DZ_SLOTS)]           # each [B*R,256]
-    img_sums = [ops.group_colsum(r, B * R, R) for r in ray_sums]                          # each [B,256]
-    tot = [g.sum(dim=0) if B > 1 else g.view(-1).clone() for g in img_sums]
-    grads_r, grads_t = [None] * 4, [None] * 4
-    grads_r[3] = (thin_dw(dz_rgb, sv.images, 3, FWD_SLOTS, S), thin_colsum(dz_rgb, S))
-    grads_t[3] = (thin_dw(dz_trans, sv.images, 6, FWD_SLOTS, S), thin_colsum(dz_trans, S))
-    grads_r[2], grads_r[1] = (big[0], tot[0]), (big[1], tot[1])
-    grads_t[2], grads_t[1] = (big[3], tot[3]), (big[4], tot[4])
-    # ---- layer 0 of each head: feature columns from the GEMM, per-sample xyz / per-ray view / per-image latent columns
-    W_r0, W_t0 = rgb_p[0][0], trans_p[0][0]
-    g_ray, g_img, g_timg = ray_sums[2], img_sums[2], img_sums[5]
-    view_t, _, vc = geom["view_seg"]()
-    dW_view, _ = ops.linear_backward_weight(g_ray, [(view_t, 1, vc)], B * R, want_bias=False)           # [256,27]
-    xyz = ops.points_from_depth(geom["center"], geom["ray"], geom["depth"]).view(S, 3)
-    dW_xyz = thin_dw(xyz, dz, 2, DZ_SLOTS, S).t().contiguous()                                          # [256,3]
-    dW_light, _ = ops.linear_backward_weight(g_img, [(ll, 1, cfg.n_latent_light)], B, want_bias=False)  # [256,48]
-    grads_r[0] = (torch.cat([big[2], dW_view, dW_xyz, dW_light], dim=1), tot[2])
-    d_ll = ops.linear_backward_input(g_img, W_r0, B, cfg.n_latent_light, None, w_col0=256 + vc + 3) if need_lat_light else None
-    dW_lt, _ = ops.linear_backward_weight(g_timg, [(lt, 1, cfg.n_latent_trans)], B, want_bias=False)    # [256,16]
-    grads_t[0] = (torch.cat([big[5], dW_lt], dim=1), tot[5])
-    d_lt = ops.linear_backward_input(g_timg, W_t0, B, cfg.n_latent_trans, None, w_col0=256) if need_lat_trans else None
-    return grads_r, grads_t, d_lt, d_ll
-
-
 def heads_backward_staged(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans, need_lat_light):
     """The two heads' backward for ANY head depth (256-wide layers), on the staged kernels: the activations are the tile images /
     ReLU bitmasks the single-pass staged forward saved (slots: feature, rgb hidden 1.., transient hidden 1.., encoding tile), the
     dX chains are two tp_tc_chain_backward launches (one per head: its output layer's dz enters as the thin operand), the
-    256 x 256 weight gradients one tp_tc_dw_gemm launch, the thin pieces the helpers of the multi-kernel path.  Used when
-    tp_tc_heads_backward's fixed stage table (the yaml's 3 x 256 heads) does not describe the architecture."""
+    256 x 256 weight gradients one tp_tc_dw_gemm launch, the thin pieces the helpers above.  Used when tp_tc_heads_backward's
+    fixed stage table (the yaml's 3 x 256 heads) does not describe the architecture, or when its images are too small for it
+    (fused_supported is false)."""
     from . import mlp_tc32  # noqa: F401  (save layout)
     dev = sv.rgb.device
     geom = sv.geom
