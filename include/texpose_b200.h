@@ -179,11 +179,9 @@ int64_t tp_tc_prof_offset(void);
  * adds the two accumulator columns, so the output layers see their weights to ~16 mantissa bits. */
 int tp_tc_pack_weights(const int64_t* chunk_desc, int n_chunks, void* packed, void* stream);
 
-/* out[b,:] = bias + W[:, col0:col0+ncols] latent[b]   (per-image constants folded into a bias; fp32) */
-int tp_tc_image_bias(const float* W, int64_t ldw, int col0, int ncols, const float* bias, const float* latent, int B,
-                     int nout, float* out, void* stream);
-/* Both heads' image biases in one launch: out_rgb[b,:] = b_rgb + W_rgb[:, col_rgb:col_rgb+n_light] light[b],
- * out_trans[b,:] = b_trans + W_trans[:, col_trans:col_trans+n_trans] trans[b]  (256 outputs each; same arithmetic as tp_tc_image_bias). */
+/* Both heads' image biases in one launch (per-image constants folded into a bias; fp32):
+ * out_rgb[b,:] = b_rgb + W_rgb[:, col_rgb:col_rgb+n_light] light[b],
+ * out_trans[b,:] = b_trans + W_trans[:, col_trans:col_trans+n_trans] trans[b]  (256 outputs each). */
 int tp_tc_image_biases(const float* W_rgb, int64_t ld_rgb, int col_rgb, int n_light, const float* b_rgb, const float* light,
                        const float* W_trans, int64_t ld_trans, int col_trans, int n_trans, const float* b_trans,
                        const float* trans, int B, float* out_rgb, float* out_trans, void* stream);
@@ -197,15 +195,14 @@ int tp_tc_ray_bias(const float* ray, int64_t R, int64_t rays_per_image, int L_vi
  * biasbuf: 16 floats {trunk7 b[0], rgb3 b[0:3], trans3 b[0:5], 0...} (the 256-wide stages' biases live in `packed`).
  * Outputs rgb [S,3,2], density [S,2], uncert [S].  save: NULL, or tp_tc_save_bytes(S) bytes receiving, per 128-sample
  * tile, the bf16 tile images [7][32 k8][128 rows][8] of {trunk feature, rgb hidden 1-3, transient hidden 1-3} that the
- * backward consumes (training).  dbg_layer/dbg_out: debugging aids (pass -1, NULL).  flags: 0 = default; bit 17 (0x20000) =
- * static-only rendering (inference launch only): the stage list stops after the rgb head, so the launch does 78 % of the work;
- * rgb[:, :, 1], density[:, 1] and uncert are written as zeros -- for callers that use only the static outputs (rgb_static /
- * depth / opacity_static of Model.evaluate_full, model/nerf_adapt_st_gan.py:341-362) and for the plain layers/nerf.py model;
- * bit 1 = 16 epilogue warps instead of 8, bits 5-6 = tile skew + 1 (A/B switches, DESIGN.md section 4). */
+ * backward consumes (training).  flags: 0 = default; bit 17 (0x20000) = static-only rendering (inference launch only): the
+ * stage list stops after the rgb head, so the launch does 78 % of the work; rgb[:, :, 1], density[:, 1] and uncert are written
+ * as zeros -- for callers that use only the static outputs (rgb_static / depth / opacity_static of Model.evaluate_full,
+ * model/nerf_adapt_st_gan.py:341-362) and for the plain layers/nerf.py model.  Any other flag bit is TP_ERR_BAD_ARG. */
 int tp_tc_nerf_stl_forward(const float* center, const float* ray, const float* depth, int64_t S, int N,
                            int64_t per_image, const void* packed, const float* biasbuf, const float* raybias,
                            const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,
-                           int64_t scratch_bytes, void* save, int dbg_layer, float* dbg_out, int flags, void* stream);
+                           int64_t scratch_bytes, void* save, int flags, void* stream);
 int64_t tp_tc_save_bytes(int64_t S);
 
 /* Graph.render after ray selection (model/nerf_adapt_st_gan.py:565-631: get_center_and_ray + ray_batch_sample, sample_depth,
@@ -219,7 +216,7 @@ int64_t tp_tc_save_bytes(int64_t S);
  *   1 = midpoints (sample_stratified false), 2 = in-kernel Philox keyed by seed (same stream as tp_sample_depth mode 2);
  *   packed / biasbuf as for tp_tc_nerf_stl_forward; wview [3+6*L_view,256] = columns 256.. of mlp_rgb[0].weight transposed
  *   (view-direction inputs, layers/nerf_static_transient_light.py:111-117); imgbias_rgb / imgbias_trans [B,256] from
- *   tp_tc_image_bias (per-image latents folded into the layer-0 biases).
+ *   tp_tc_image_biases (per-image latents folded into the layer-0 biases).
  * Outputs (any may be NULL = not materialised): rgb, rgb_static, rgb_transient [B*R,3]; depth, opacity, opacity_static,
  * opacity_transient, uncert [B*R] (uncert includes + min_uncert, layers/..light.py:207); alpha_static, alpha_transient [B*R*N];
  * density [B*R*N,2].  Output pointers may address a peer GPU's memory (NVLink stores: the one-frame multi-GPU gather).
@@ -251,7 +248,7 @@ int tp_render_fused_forward(const float* kinv, const float* pose_inv, int B, int
  *   [ceil(S/128)][n_save][64 KB] receives the output of every hidden stage that names a save slot as a bf16 tile image
  *   [32 k8][128 rows][8] -- the operands of the tensor-core backward (tp_tc_chain_backward, tp_tc_dw_gemm) -- and slot enc_slot
  *   (-1 = none) the encoding tile [xyz, enc(xyz), 1, 0...]: dz^T of it = the encoding columns of a layer's dW and its bias sum;
- *   bias: fp32 static biases; raybias [rays,256] from tp_tc_ray_bias, imgbias [images,256] from tp_tc_image_bias.
+ *   bias: fp32 static biases; raybias [rays,256] from tp_tc_ray_bias, imgbias [images,256] from tp_tc_image_biases.
  * Outputs rgb [S,3,2], density [S,2], uncert [S] as tp_tc_nerf_stl_forward.  scratch >= tp_tc32_scratch_bytes().  Range of the
  * split mode: |weights|, |hidden activations| < 65 504 (fp16 hi part); a violation is reported through the status word. */
 int64_t tp_tc32_slot_bytes(void);
@@ -280,8 +277,7 @@ int tp_tc_dw_splits(int64_t S, int n_jobs);  /* split partials per job that tp_t
  * [splits][n_jobs][256][256] with splits = tp_tc_dw_splits(S, n_jobs).  a_slots/b_slots: HOST arrays.
  * Reduce with tp_reduce_partials(partial, splits, n_jobs*65536, ...). */
 int tp_tc_dw_gemm(const void* a_images, int a_nslots, const void* b_images, int b_nslots, const int32_t* a_slots,
-                  const int32_t* b_slots, int n_jobs, int64_t S, float* partial, int64_t partial_floats, int flags,
-                  void* stream);
+                  const int32_t* b_slots, int n_jobs, int64_t S, float* partial, int64_t partial_floats, void* stream);
 
 /* Backward of both heads on the images tp_tc_nerf_stl_forward saved, in five launches: the dX chain kernel also accumulates,
  * on the tensor pipe, every thin gradient -- bias gradients, output-layer weight gradients, the xyz / view-direction columns

@@ -1,6 +1,5 @@
 """Fused forward kernel at C3 size (4096 rays x 128): inference launch vs training launch (activation save + ReLU bitmasks).
-Kernel-only CUDA-event times around the C-ABI call; TEXPOSE_TC_FLAGS bits 14 / 15 switch off the activation-save stores /
-the ReLU bitmasks (timing only: the backward would read garbage).  Never a benchmark."""
+Kernel-only CUDA-event times around the C-ABI call.  Never a benchmark."""
 import os
 import sys
 
@@ -62,7 +61,3 @@ def run(train, iters=12):
 for label, train in (("inference", False), ("training (save)", True), ("inference", False), ("training (save)", True)):
     med, best = run(train)
     print(f"{label:18s} kernel median {med * 1e3:8.1f} us   best {best * 1e3:8.1f} us", flush=True)
-for fl, what in ((16384, "no save stores"), (32768, "no bitmasks"), (49152, "neither")):
-    os.environ["TEXPOSE_TC_FLAGS"] = str(fl)
-    med, best = run(True)
-    print(f"training, {what:16s} kernel median {med * 1e3:8.1f} us   best {best * 1e3:8.1f} us", flush=True)

@@ -1,5 +1,5 @@
 """Smoke-sized run of every hand-written synchronisation protocol, for compute-sanitizer (memcheck / racecheck / synccheck):
-the fused forward kernel in its three launch kinds (render <1,17,3>, per-sample inference <1,17,1>, training <1,17,2> with the
+the fused forward kernel in its three launch kinds (render <17,3>, per-sample inference <17,1>, training <17,2> with the
 activation save), the static-only instantiations, the fused backward chain + dW GEMM kernels, the fused loss, and the peer-window
 exchange / barrier kernels with two "ranks" on one device.
 usage: compute-sanitizer --tool racecheck python scripts/sanitize_target.py [what ...]   (what: render train split plain peer; default render train split plain)"""
@@ -36,11 +36,11 @@ if "render1" in what:      # the per-sample inference launch alone (multi-kernel
 
 if "render" in what:
     with torch.no_grad():
-        a = g.render(opt, pose, intr=intr, ray_idx=range(0, H * W), depth_range=dr, mode="val")                   # <1,17,3>
+        a = g.render(opt, pose, intr=intr, ray_idx=range(0, H * W), depth_range=dr, mode="val")                   # <17,3>
         o2 = AttrDict(opt); o2.b200 = AttrDict(opt.b200); o2.b200.fused_render = False
-        b = g.render(o2, pose, intr=intr, ray_idx=range(0, H * W), depth_range=dr, mode="val")                    # <1,17,1> + composite
+        b = g.render(o2, pose, intr=intr, ray_idx=range(0, H * W), depth_range=dr, mode="val")                    # <17,1> + composite
         o3 = AttrDict(opt); o3.b200 = AttrDict(opt.b200); o3.b200.static_only = True
-        c = g.render(o3, pose[:1], intr=intr[:1], ray_idx=range(0, H * W), depth_range=(dr[0][:1], dr[1][:1]), sample_idx=torch.tensor(0, device=dev), mode="eval")   # <1,13,3>
+        c = g.render(o3, pose[:1], intr=intr[:1], ray_idx=range(0, H * W), depth_range=(dr[0][:1], dr[1][:1]), sample_idx=torch.tensor(0, device=dev), mode="eval")   # <13,3>
         opt64 = adapt_gan_opt(H=H, W=W, sample_intvs=64, device=dev); opt64.b200 = AttrDict(mlp="bf16", rng="torch")
         d = g.render(opt64, pose, intr=intr, ray_idx=torch.randperm(H * W, device=dev)[None, :300].expand(2, -1).contiguous(), depth_range=dr, mode="val")   # 2 rays per tile
     torch.cuda.synchronize()
@@ -86,7 +86,7 @@ if "train" in what:
     idx = torch.arange(B, device=dev)
     var = AttrDict(idx=idx, image=torch.rand(B, 3, 64, 64, device=dev), obj_mask=(torch.rand(B, 64, 64, device=dev) > 0.3).float(), ray_idx=coords)
     g.train()
-    ret = g.render(opt_t, pose_t, intr=intr_t, ray_idx=coords, depth_range=(zn_t[:, :, None], zf_t[:, :, None]), sample_idx=idx, mode="train")   # <1,17,2>
+    ret = g.render(opt_t, pose_t, intr=intr_t, ray_idx=coords, depth_range=(zn_t[:, :, None], zf_t[:, :, None]), sample_idx=idx, mode="train")   # <17,2>
     var.update(ret)
     summarize_loss(opt_t, var, g.compute_loss(opt_t, var, mode="train"))["all"].backward()      # chain + dW + finish kernels
     torch.cuda.synchronize()

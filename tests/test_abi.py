@@ -46,6 +46,21 @@ def test_host_side_helpers_without_gpu():
     assert lib.tp_tc_heads_backward_supported(0, 128) == 0
 
 
+def test_forward_rejects_unknown_flags_before_the_device():
+    """tp_tc_nerf_stl_forward takes only flags bit 17 (static only); any other bit is a bad argument, reported before the
+    device check.  S = 0, so no argument combination can launch anything."""
+    lib = _C.load()
+    p = 0x10000      # non-null, 16-byte aligned; never dereferenced
+
+    def fwd(flags):
+        return lib.tp_tc_nerf_stl_forward(p, p, p, 0, 32, 32, p, p, p, p, p, p, p, p, 1 << 30, None, flags, None)
+
+    for flags in (0, 1 << 17):
+        assert fwd(flags) in (0, -4)      # the dummy arguments pass every argument check (-4: no sm_100 device)
+    for flags in (2, 0x20, 0x40):
+        assert fwd(flags) == -1
+
+
 def test_peer_window_layout_helpers_without_gpu():
     """Pure host arithmetic of the gradient-exchange window (csrc/peer.cu): [1 KB header | buffer 0 | buffer 1], buffers
     padded to 256 B; argument errors are reported before any CUDA call."""

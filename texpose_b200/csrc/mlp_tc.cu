@@ -36,9 +36,9 @@
 
 namespace tc {
 
-// kHalves epilogue warps per (tile, TMEM lane quarter): kHalves = 1 -> 8 epilogue warps (256 columns per thread),
-// kHalves = 2 -> 16 epilogue warps (128 columns per thread).  Then one TMA producer warp and one MMA issuer warp.
-template <int kHalves> constexpr int num_threads() { return (8 * kHalves + 2) * 32; }
+// 8 epilogue warps (one per tile and TMEM lane quarter: 256 accumulator columns per thread), then one TMA producer warp and one
+// MMA issuer warp
+constexpr int kEpiWarps = 8, kProducerWarp = kEpiWarps, kMmaWarp = kEpiWarps + 1, kThreads = (kEpiWarps + 2) * 32;
 constexpr int kStages = 4;
 constexpr uint32_t kOffA = 0, kOffE = 2 * kABytes, kOffRing = kOffE + 2 * kEBytes;
 constexpr uint32_t kOffBar = kOffRing + kStages * kChunkBytes;
@@ -324,24 +324,21 @@ __device__ __noinline__ void render_composite(const Params& p, float* sc, int t,
 
 // kNL: number of stages run (kNumLayers = all; kStaticLayers = static-only rendering).  A template parameter, not a field of
 // Params: a run-time stage count costs 0.3 ms per C2 frame (same-box A/B).
-// kMode: 0 = general (debug tap, any tile skew, any N); 1 = the plain inference launch (per-sample outputs, no activation save);
-// 2 = the plain training launch (activation save + ReLU bitmasks); 3 = the fused render launch (rays, depths, view bias and
-// compositing in-kernel; per-ray outputs).  Modes 1-3 have every debug branch compiled out and the default tile skew as a
-// constant: the same code with those decisions left to run time is 6 % slower (same-box A/B).
+// kMode: 0 = general (any N: the per-sample launches, with or without the activation save, whose N is not a multiple of 32);
+// 1 = the plain inference launch (per-sample outputs, no activation save); 2 = the plain training launch (activation save + ReLU
+// bitmasks); 3 = the fused render launch (rays, depths, view bias and compositing in-kernel; per-ray outputs).  Modes 1-3 are
+// launched only when N % 32 == 0 and compile the branches of the other launch kinds out.
 // kSmemBias: the launch has one ray per tile (N = 128, hence also one image per tile): the per-ray / per-image bias row of the
 // two table-bias stages sits in shared memory and the drain reads it with broadcast loads instead of warp shuffles.
-template <int kHalves, int kNL = kNumLayers, int kMode = 0, bool kSmemBias = false>
+template <int kNL = kNumLayers, int kMode = 0, bool kSmemBias = false>
 // (320 threads allocate registers as 12 warps -- warps are allocated in fours -- so the cap is 168 registers per thread; the render
 // launch keeps its look-ahead state (next sample's encoding, finished sample) partly in local memory: a few dozen L1-resident
 // STL / LDL per super-tile, cheaper than recomputing it on the critical path)
-__global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_kernel(const Params p) {
+__global__ void __launch_bounds__(kThreads, 1) nerf_stl_forward_kernel(const Params p) {
   constexpr bool kRender = kMode == 3;
-  static_assert(!kRender || kHalves == 1, "the render launch uses the 8-warp drain");
-  static_assert(!kSmemBias || (kHalves == 1 && kMode != 0), "shared-memory bias rows: lean 8-warp launches");
-  const int p_skew = kMode ? 1 : p.skew;
+  static_assert(!kSmemBias || kMode != 0, "shared-memory bias rows: launches with N % 32 == 0 only");
   uint8_t* const p_save = (kMode == 1 || kRender) ? nullptr : p.save;
-  constexpr int kEpiWarps = 8 * kHalves, kProducerWarp = kEpiWarps, kMmaWarp = kEpiWarps + 1;
-  constexpr int kTileThreads = 128 * kHalves;     // epilogue threads working on one tile
+  constexpr int kTileThreads = 128;     // epilogue threads working on one tile
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);   // provably warp-uniform role index
@@ -404,9 +401,9 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
     }
   } else if (warp == kMmaWarp) {
     // ================================================================ MMA issuer (converged warp, one lane issues)
-    // Inside a stage tile 0 runs `skew` weight chunks ahead of tile 1 (both still consume every chunk from the same ring
-    // slot): T0's accumulator completes 256*(skew+1) cycles before T1's, so T0's epilogue -- and T0's first MMAs of the next
-    // stage -- overlap T1's MMAs / epilogue instead of leaving the tensor pipe idle.
+    // Inside a stage tile 0 runs one weight chunk ahead of tile 1 (both still consume every chunk from the same ring slot):
+    // T0's accumulator completes 512 cycles before T1's, so T0's epilogue -- and T0's first MMAs of the next stage -- overlap
+    // T1's MMAs / epilogue instead of leaving the tensor pipe idle.
     {
       uint32_t chunk_base = 0, ready_ph = 0, reload_ph = 0;   // per-tile phase bits (bit t)
 #ifdef TP_FWD_PROF
@@ -419,11 +416,10 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
         for (int L = 0; L < kNL; ++L) {
           const Layer ly = kLayers[L];
           const int nch = ly.small ? 1 : ly.a_chunks + ly.e_chunks + ly.bias_chunk;
-          const int skew = p_skew < nch ? p_skew : nch;
-          for (int step = 0; step < nch + skew; ++step) {
+          for (int step = 0; step <= nch; ++step) {
 #pragma unroll
             for (int t = 0; t < 2; ++t) {
-              const int c = t == 0 ? step : step - skew;
+              const int c = step - t;
               if (c < 0 || c >= nch) continue;
               const uint32_t abs_chunk = chunk_base + c;
               const uint32_t stage = abs_chunk % kStages, phase = (abs_chunk / kStages) & 1u;
@@ -500,12 +496,10 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
     }
   } else {
     // ================================================================ encode + epilogue warps
-    // warp -> (TMEM lane quarter q = warp % 4, tile t, column half); half 0 also encodes and owns the per-sample outputs
-    const int q = warp & 3, t = (warp >> 2) & 1, half = warp >> 3, row = q * 32 + lane;
-    constexpr int kCols = 256 / kHalves;            // accumulator columns converted per thread
+    // warp -> (TMEM lane quarter q = warp % 4, tile t): a thread owns one row of its tile, all 256 accumulator columns
+    const int q = warp & 3, t = (warp >> 2) & 1, row = q * 32 + lane;
     const uint32_t a_smem = sbase + kOffA + t * kABytes, e_smem = sbase + kOffE + t * kEBytes;
     const uint32_t tmem_row = tmem_base + ((uint32_t)(q * 32) << 16) + t * 256;
-    const uint32_t tmem_d = tmem_row + half * kCols;
     uint8_t* my_scratch = p.scratch + ((size_t)blockIdx.x * 2 + t) * kABytes;
     // render launch: view-bias rows of this tile's rays (<= 4 rays x 1 KB), behind the parked features of all CTAs
     float* vb_slot = reinterpret_cast<float*>(p.scratch + (size_t)gridDim.x * 2 * kABytes) + ((size_t)blockIdx.x * 2 + t) * 4 * 256;
@@ -532,9 +526,10 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
         if (kRender) {
           rs = render_fetch(p, st * 2 + t, row, lane);
           render_encode(rs.xyz[0], rs.xyz[1], rs.xyz[2], e_smem, row);
-        } else if (half == 0) {
-          if (kMode == 0 || kHalves != 1 || iter == 0) encode_sample(p, s, e_smem, row);
-          else store_encoding(enc_next, e_smem, row);      // worked out during the previous super-tile (below)
+        } else if (kMode == 0 || iter == 0) {
+          encode_sample(p, s, e_smem, row);
+        } else {
+          store_encoding(enc_next, e_smem, row);      // worked out during the previous super-tile (below)
         }
         fence_proxy_async_smem();
         tc_fence_before();
@@ -567,9 +562,9 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
             wb[1] = __ldcg(reinterpret_cast<const float4*>(brow + 128) + lane);
           } else {
             const long long img = kRender ? (long long)rs.img : s / p.per_image;
-            const float* brow = (ly.bias_kind == BIAS_RAY ? p.raybias + (s / p.N) * 256 : p.imgbias + img * 256) + half * kCols;
+            const float* brow = ly.bias_kind == BIAS_RAY ? p.raybias + (s / p.N) * 256 : p.imgbias + img * 256;
             wb[0] = __ldg(reinterpret_cast<const float4*>(brow) + lane);
-            if (kCols == 256) wb[1] = __ldg(reinterpret_cast<const float4*>(brow + 128) + lane);
+            wb[1] = __ldg(reinterpret_cast<const float4*>(brow + 128) + lane);
           }
         }
         // Two windows in which both tiles and the tensor pipe wait whatever the epilogue warps do (scripts/fwd_prof.py): right after
@@ -617,7 +612,7 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
             }
           }
         }
-        if (!kRender && kMode != 0 && kHalves == 1 && L == kNL - 2 && st + gridDim.x < n_super) {      // (8-warp drain: registers to spare)
+        if (!kRender && kMode != 0 && L == kNL - 2 && st + gridDim.x < n_super) {
           // per-sample launches: the same for the next sample's loads (ray, depth) and its sixty sines
           const long long sn_raw = ((st + gridDim.x) * 2 + t) * 128 + row, sn = sn_raw < p.S ? sn_raw : p.S - 1, rn = sn / p.N;
           const float cn[3] = {p.center[rn * 3], p.center[rn * 3 + 1], p.center[rn * 3 + 2]};
@@ -628,11 +623,11 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
         acc_ph ^= 1;
         tc_fence_after();
         if (ly.epi == EPI_HIDDEN && store_pending) {   // the previous bulk store must have finished reading A_t
-          if (row == 0 && half == 0) bulk_wait_read();
+          if (row == 0) bulk_wait_read();
           named_bar_sync(1 + t, kTileThreads);
           store_pending = false;
         }
-        if (L == kReloadIssueLayer && kNL > kStaticLayers && row == 0 && half == 0) {
+        if (L == kReloadIssueLayer && kNL > kStaticLayers && row == 0) {
           // every MMA that reads A_t has retired (acc barrier) -> bring the trunk feature back for the transient head
           bulk_wait_all();
           fence_proxy_async_all();
@@ -641,8 +636,7 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
         }
         if (copy_row) named_bar_sync(1 + t, kTileThreads);      // the tile's 128 threads wrote the row before the accumulator wait
         if (ly.epi == EPI_HIDDEN) {
-          float* dbg_row = (kMode == 0 && (L == p.dbg_layer) && live && p.dbg_out) ? p.dbg_out + s * 256 + half * kCols : nullptr;
-          const uint32_t a_row = a_smem + half * (kCols / 8) * 2048 + row * 16;
+          const uint32_t a_row = a_smem + row * 16;
           const bool train_stage = p_save && L != kSpillLayer && kSaveSlot[L] >= 0;
           if (train_stage) {
             // training: h1 / h2 of either head also leave a ReLU bitmask [128 rows][256 bits] for the backward chain (word
@@ -651,37 +645,34 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
             // 16-byte groups cover 512 contiguous bytes and nothing re-reads the A tile
             const int mslot = kMaskBitSlot[L];
             uint32_t* words = mslot < 0 ? nullptr
-                                        : reinterpret_cast<uint32_t*>(p.bits + ((size_t)(st * 2 + t) * 4 + mslot) * kMaskBitBytes) +
-                                              half * (kCols / 32) * 128 + row;
-            uint8_t* g_row = p_save + ((size_t)(st * 2 + t) * kSaveSlots + kSaveSlot[L]) * kABytes + half * (kCols / 8) * 2048 + row * 16;
+                                        : reinterpret_cast<uint32_t*>(p.bits + ((size_t)(st * 2 + t) * 4 + mslot) * kMaskBitBytes) + row;
+            uint8_t* g_row = p_save + ((size_t)(st * 2 + t) * kSaveSlots + kSaveSlot[L]) * kABytes + row * 16;
             if (ly.bias_kind == BIAS_MMA) {
-              hidden_epilogue<false, kCols / 32, true>(tmem_d, nullptr, a_row, dbg_row, words, g_row);
+              hidden_epilogue<false, 8, true>(tmem_row, nullptr, a_row, words, g_row);
             } else if (kSmemBias) {
-              hidden_epilogue_sbias<kCols / 32, true>(tmem_d, bias_sm, a_row, dbg_row, words, g_row);
+              hidden_epilogue_sbias<8, true>(tmem_row, bias_sm, a_row, words, g_row);
             } else if (warp_bias) {
-              hidden_epilogue_wbias<kCols / 32, true>(tmem_d, wb, a_row, dbg_row, words, g_row);
+              hidden_epilogue_wbias<8, true>(tmem_row, wb, a_row, words, g_row);
             } else {
-              const float* bias = (ly.bias_kind == BIAS_RAY ? p.raybias + (s / p.N) * 256 : p.imgbias + (s / p.per_image) * 256) +
-                                  half * kCols;
-              hidden_epilogue<true, kCols / 32, true>(tmem_d, bias, a_row, dbg_row, words, g_row);
+              const float* bias = ly.bias_kind == BIAS_RAY ? p.raybias + (s / p.N) * 256 : p.imgbias + (s / p.per_image) * 256;
+              hidden_epilogue<true, 8, true>(tmem_row, bias, a_row, words, g_row);
             }
           } else if (ly.bias_kind == BIAS_MMA) {
-            hidden_epilogue<false, kCols / 32>(tmem_d, nullptr, a_row, dbg_row);
+            hidden_epilogue<false, 8>(tmem_row, nullptr, a_row);
           } else if (kSmemBias) {
-            hidden_epilogue_sbias<kCols / 32>(tmem_d, bias_sm, a_row, dbg_row);
+            hidden_epilogue_sbias<8>(tmem_row, bias_sm, a_row);
           } else if (warp_bias) {
-            hidden_epilogue_wbias<kCols / 32>(tmem_d, wb, a_row, dbg_row);
+            hidden_epilogue_wbias<8>(tmem_row, wb, a_row);
           } else {
-            const float* bias = (ly.bias_kind == BIAS_RAY ? p.raybias + (s / p.N) * 256 : p.imgbias + (s / p.per_image) * 256) +
-                                half * kCols;
-            hidden_epilogue<true, kCols / 32>(tmem_d, bias, a_row, dbg_row);
+            const float* bias = ly.bias_kind == BIAS_RAY ? p.raybias + (s / p.N) * 256 : p.imgbias + (s / p.per_image) * 256;
+            hidden_epilogue<true, 8>(tmem_row, bias, a_row);
           }
           fence_proxy_async_smem();
           if (L == kSpillLayer && kNL > kStaticLayers) {      // static only: no second head, nothing to park
             // park the trunk feature (bf16 tile image) in the L2 scratch (training: in its slot of the save buffer, where
             // the backward also reads it) -- the bulk store overlaps the next stage's MMAs
             named_bar_sync(1 + t, kTileThreads);
-            if (row == 0 && half == 0) {
+            if (row == 0) {
               uint8_t* dst = p_save ? p_save + ((size_t)(st * 2 + t) * kSaveSlots + kSaveSlot[L]) * kABytes : my_scratch;
               bulk_s2g(dst, a_smem, kABytes);
               bulk_commit();
@@ -690,7 +681,7 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
           } else if (kRender && L == kSpillLayer) {
             named_bar_sync(1 + t, kTileThreads);      // static only: nothing is parked, but the view-bias rows need the tile barrier
           }
-        } else if (half == 0) {
+        } else {
           // N=16 output stage: columns 0..7 = x . bf16(W rows), columns 8..15 = x . bf16(W - bf16(W)) of the same rows
           uint32_t v[16];
           TP_TMEM_LD16(tmem_row, v);
@@ -741,7 +732,7 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
             }
           }
         }
-        if (L != kNL - 1 && !(ly.small && half == 0)) {   // (output stages arrived above; the next super-tile's encode covers the last stage)
+        if (L != kNL - 1 && !ly.small) {   // (output stages arrived above; the next super-tile's encode covers the last stage)
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(bar_ready(t));
@@ -753,7 +744,7 @@ __global__ void __launch_bounds__(num_threads<kHalves>(), 1) nerf_stl_forward_ke
       render_composite(p, sc, t, q, lane, done_ray, done_k, done_d, done_dist, done_live, done_v[0], done_v[1], done_v[2], done_v[3],
                        done_v[4], done_v[5], done_v[6], done_v[7], done_v[8]);
     }
-    if (row == 0 && half == 0) bulk_wait_all();
+    if (row == 0) bulk_wait_all();
   }
 
   tc_fence_before();
@@ -800,19 +791,8 @@ __global__ void pack_weights_kernel(const long long* __restrict__ desc, __nv_bfl
   }
 }
 
-// out[b, n] = bias[n] + sum_j W[n, col0 + j] * latent[b, j]
-__global__ void image_bias_kernel(const float* __restrict__ W, long long ldw, int col0, int ncols,
-                                  const float* __restrict__ bias, const float* __restrict__ latent, int nout,
-                                  float* __restrict__ out) {
-  const int b = blockIdx.x;
-  for (int n = threadIdx.x; n < nout; n += blockDim.x) {
-    float acc = bias ? bias[n] : 0.f;
-    for (int j = 0; j < ncols; ++j) acc = fmaf(W[n * ldw + col0 + j], latent[(long long)b * ncols + j], acc);
-    out[(long long)b * nout + n] = acc;
-  }
-}
-
-// both heads in one launch: blocks [0, B) the rgb head's rows, [B, 2B) the transient head's
+// out[b, n] = bias[n] + sum_j W[n, col0 + j] * latent[b, j] for both heads in one launch: blocks [0, B) the rgb head's rows,
+// [B, 2B) the transient head's
 __global__ void image_biases_kernel(const float* __restrict__ W_r, long long ld_r, int col_r, int n_r, const float* __restrict__ b_r,
                                     const float* __restrict__ lat_r, const float* __restrict__ W_t, long long ld_t, int col_t, int n_t,
                                     const float* __restrict__ b_t, const float* __restrict__ lat_t, int B, float* __restrict__ out_r,
@@ -920,14 +900,6 @@ TP_API int tp_tc_pack_weights(const int64_t* chunk_desc, int n_chunks, void* pac
   return tp_launch_status();
 }
 
-TP_API int tp_tc_image_bias(const float* W, int64_t ldw, int col0, int ncols, const float* bias, const float* latent,
-                            int B, int nout, float* out, void* stream) {
-  if (!W || !latent || !out) return TP_ERR_BAD_ARG;
-  if (B < 1 || nout < 1 || ncols < 0) return TP_ERR_BAD_SHAPE;
-  tc::image_bias_kernel<<<B, 256, 0, (cudaStream_t)stream>>>(W, ldw, col0, ncols, bias, latent, nout, out);
-  return tp_launch_status();
-}
-
 TP_API int tp_tc_image_biases(const float* W_rgb, int64_t ld_rgb, int col_rgb, int n_light, const float* b_rgb, const float* light,
                               const float* W_trans, int64_t ld_trans, int col_trans, int n_trans, const float* b_trans,
                               const float* trans, int B, float* out_rgb, float* out_trans, void* stream) {
@@ -949,24 +921,27 @@ TP_API int tp_tc_ray_bias(const float* ray, int64_t R, int64_t rays_per_image, i
   return tp_launch_status();
 }
 
-static int tc_launch(void (*kern)(const tc::Params), const tc::Params& p, int grid, int threads, cudaStream_t stream) {
+// 8 epilogue warps drain the accumulators (256 columns per thread, 320 threads per CTA): the same tensor-pipe time as 16 warps,
+// but the narrower CTA draws less power and the capped clock settles higher -- 2 % faster for the C2 frame, 1.7 % for the C3
+// training step (same-box A/B, profiles/r01f_summary.md section 9).
+static int tc_launch(void (*kern)(const tc::Params), const tc::Params& p, int grid, cudaStream_t stream) {
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::kSmemBytes);
   if (e != cudaSuccess) return (int)e;
-  kern<<<grid, threads, tc::kSmemBytes, stream>>>(p);
+  kern<<<grid, tc::kThreads, tc::kSmemBytes, stream>>>(p);
   return tp_launch_status();
 }
 
 TP_API int tp_tc_nerf_stl_forward(const float* center, const float* ray, const float* depth, int64_t S, int N,
                                   int64_t per_image, const void* packed, const float* biasbuf, const float* raybias,
                                   const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,
-                                  int64_t scratch_bytes, void* save, int dbg_layer, float* dbg_out, int flags, void* stream) {
+                                  int64_t scratch_bytes, void* save, int flags, void* stream) {
   if (!center || !ray || !depth || !packed || !biasbuf || !raybias || !imgbias || !rgb || !density || !uncert || !scratch)
     return TP_ERR_BAD_ARG;
   if (S < 0 || N < 1 || per_image < 1) return TP_ERR_BAD_SHAPE;
   if (((uintptr_t)packed & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)biasbuf & 15) || ((uintptr_t)raybias & 15) ||
       ((uintptr_t)imgbias & 15) || ((uintptr_t)rgb & 7) || ((uintptr_t)density & 7) || ((uintptr_t)save & 15))
     return TP_ERR_ALIGN;
-  if (flags & ~((1 << 1) | (3 << 5) | (1 << 17))) return TP_ERR_BAD_ARG;
+  if (flags & ~(1 << 17)) return TP_ERR_BAD_ARG;
   if (!tp_device_is_sm100()) return TP_ERR_ARCH;
   if (S == 0) return TP_OK;
   const long long n_super = (S + 255) / 256;
@@ -979,26 +954,17 @@ TP_API int tp_tc_nerf_stl_forward(const float* center, const float* ray, const f
   p.rgb = rgb; p.density = density; p.uncert = uncert; p.scratch = reinterpret_cast<uint8_t*>(scratch);
   p.save = reinterpret_cast<uint8_t*>(save);
   p.bits = save ? p.save + ((S + 255) / 256) * 2 * tc::kSaveSlots * (size_t)tc::kABytes : nullptr;
-  p.dbg_layer = dbg_layer; p.dbg_out = dbg_out; p.prof_offset = tp_tc_prof_offset();
+  p.prof_offset = tp_tc_prof_offset();
   p.n_layers = (flags & (1 << 17)) ? tc::kStaticLayers : tc::kNumLayers;      // flags bit 17: static-only rendering
   if ((flags & (1 << 17)) && save) return TP_ERR_BAD_ARG;                     // inference launches only
-  p.skew = ((flags >> 5) & 3) ? ((flags >> 5) & 3) - 1 : 1;      // default skew 1; flags bits 5-6 = skew+1 override (A/B)
-  // drain width: 8 epilogue warps (256 accumulator columns per thread, 320 threads per CTA) by default -- same tensor-pipe
-  // time as 16 warps, but the narrower CTA draws less power and the capped clock settles higher: 2 % faster for the C2 frame,
-  // 1.7 % for the C3 training step (same-box A/B, profiles/r01f_summary.md section 9).  flags bit 1 selects 16 warps.
-  const bool wide = (flags & 2) != 0;
   const bool stat = p.n_layers == tc::kStaticLayers;
-  const bool plain = dbg_layer < 0 && !dbg_out && p.skew == 1 && N % 32 == 0;
   const bool n128 = N == 128;      // one ray (and one image) per tile: bias rows in shared memory
   void (*kern)(const tc::Params) =
-      plain && !save && !wide ? (stat ? (n128 ? tc::nerf_stl_forward_kernel<1, tc::kStaticLayers, 1, true> : tc::nerf_stl_forward_kernel<1, tc::kStaticLayers, 1>)
-                                      : (n128 ? tc::nerf_stl_forward_kernel<1, tc::kNumLayers, 1, true> : tc::nerf_stl_forward_kernel<1, tc::kNumLayers, 1>))
-      : plain && !save        ? (stat ? tc::nerf_stl_forward_kernel<2, tc::kStaticLayers, 1> : tc::nerf_stl_forward_kernel<2, tc::kNumLayers, 1>)
-      : plain && wide         ? tc::nerf_stl_forward_kernel<2, tc::kNumLayers, 2>
-      : plain                 ? (n128 ? tc::nerf_stl_forward_kernel<1, tc::kNumLayers, 2, true> : tc::nerf_stl_forward_kernel<1, tc::kNumLayers, 2>)
-      : wide ? (stat ? tc::nerf_stl_forward_kernel<2, tc::kStaticLayers> : tc::nerf_stl_forward_kernel<2, tc::kNumLayers>)
-             : (stat ? tc::nerf_stl_forward_kernel<1, tc::kStaticLayers> : tc::nerf_stl_forward_kernel<1, tc::kNumLayers>);
-  return tc_launch(kern, p, grid, wide ? tc::num_threads<2>() : tc::num_threads<1>(), (cudaStream_t)stream);
+      N % 32 != 0 ? (stat ? tc::nerf_stl_forward_kernel<tc::kStaticLayers> : tc::nerf_stl_forward_kernel<tc::kNumLayers>)
+      : !save     ? (stat ? (n128 ? tc::nerf_stl_forward_kernel<tc::kStaticLayers, 1, true> : tc::nerf_stl_forward_kernel<tc::kStaticLayers, 1>)
+                          : (n128 ? tc::nerf_stl_forward_kernel<tc::kNumLayers, 1, true> : tc::nerf_stl_forward_kernel<tc::kNumLayers, 1>))
+                  : (n128 ? tc::nerf_stl_forward_kernel<tc::kNumLayers, 2, true> : tc::nerf_stl_forward_kernel<tc::kNumLayers, 2>);
+  return tc_launch(kern, p, grid, (cudaStream_t)stream);
 }
 
 // Graph.render after ray selection (model/nerf_adapt_st_gan.py:565-631) as ONE launch.
@@ -1031,7 +997,7 @@ TP_API int tp_render_fused_forward(const float* kinv, const float* pose_inv, int
   p.S = S; p.N = N; p.per_image = R * N;
   p.packed = reinterpret_cast<const uint8_t*>(packed); p.biasbuf = biasbuf; p.imgbias = imgbias_trans;
   p.density = density; p.scratch = reinterpret_cast<uint8_t*>(scratch);
-  p.dbg_layer = -1; p.skew = 1; p.prof_offset = tp_tc_prof_offset();
+  p.prof_offset = tp_tc_prof_offset();
   p.n_layers = (flags & (1 << 17)) ? tc::kStaticLayers : tc::kNumLayers;
   p.kinv = kinv; p.pinv = pose_inv; p.H = H; p.W = W; p.pix_offset = pix_offset;
   p.ray_idx = reinterpret_cast<const long long*>(ray_idx); p.R = R; p.ray0 = ray0;
@@ -1041,7 +1007,7 @@ TP_API int tp_render_fused_forward(const float* kinv, const float* pose_inv, int
   p.o_op_s = opacity_static; p.o_op_t = opacity_transient; p.o_unc = uncert; p.o_as = alpha_static; p.o_at = alpha_transient;
   const bool stat = p.n_layers == tc::kStaticLayers, n128 = N == 128;
   void (*kern)(const tc::Params) =
-      stat ? (n128 ? tc::nerf_stl_forward_kernel<1, tc::kStaticLayers, 3, true> : tc::nerf_stl_forward_kernel<1, tc::kStaticLayers, 3>)
-           : (n128 ? tc::nerf_stl_forward_kernel<1, tc::kNumLayers, 3, true> : tc::nerf_stl_forward_kernel<1, tc::kNumLayers, 3>);
-  return tc_launch(kern, p, grid, tc::num_threads<1>(), (cudaStream_t)stream);
+      stat ? (n128 ? tc::nerf_stl_forward_kernel<tc::kStaticLayers, 3, true> : tc::nerf_stl_forward_kernel<tc::kStaticLayers, 3>)
+           : (n128 ? tc::nerf_stl_forward_kernel<tc::kNumLayers, 3, true> : tc::nerf_stl_forward_kernel<tc::kNumLayers, 3>);
+  return tc_launch(kern, p, grid, (cudaStream_t)stream);
 }

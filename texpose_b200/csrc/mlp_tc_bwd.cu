@@ -514,7 +514,6 @@ struct DwParams {
   int n_jobs, splits;                                // CTA -> (job = blockIdx % n_jobs, split = blockIdx / n_jobs)
   long long n_tiles;
   float* partial;                                    // [splits][n_jobs][256][256]
-  int swap_strides;                                  // debug
 };
 
 
@@ -572,7 +571,7 @@ __global__ void __launch_bounds__(kThreads, 1) dw_gemm_kernel(const DwParams p) 
     const uint32_t idesc = umma_idesc_mn(128, 256);
     // MN-major canonical layout of a tile image: 8 (K=s) x 8 (MN) core matrices, K-block stride (LBO) 128 B,
     // MN-block stride (SBO) 2048 B
-    const uint32_t lbo = p.swap_strides ? 2048u : 128u, sbo = p.swap_strides ? 128u : 2048u;
+    constexpr uint32_t lbo = 128u, sbo = 2048u;
     const uint32_t hi = (sbo >> 4) | (1u << 14);
     for (long long t = t0; t < t1; ++t) {
       const uint32_t sa = slot, pa = phase;
@@ -930,8 +929,7 @@ TP_API int tp_tc_dw_splits(int64_t S, int n_jobs) {
 }
 
 TP_API int tp_tc_dw_gemm(const void* a_images, int a_nslots, const void* b_images, int b_nslots, const int32_t* a_slots,
-                         const int32_t* b_slots, int n_jobs, int64_t S, float* partial, int64_t partial_floats, int flags,
-                         void* stream) {
+                         const int32_t* b_slots, int n_jobs, int64_t S, float* partial, int64_t partial_floats, void* stream) {
   if (!a_images || !b_images || !partial || !a_slots || !b_slots) return TP_ERR_BAD_ARG;
   if (S < 1 || n_jobs < 1 || n_jobs > tcb::kDwMaxJobs) return TP_ERR_BAD_SHAPE;
   if (((uintptr_t)a_images & 15) || ((uintptr_t)b_images & 15) || ((uintptr_t)partial & 15)) return TP_ERR_ALIGN;
@@ -946,7 +944,7 @@ TP_API int tp_tc_dw_gemm(const void* a_images, int a_nslots, const void* b_image
   }
   p.n_jobs = n_jobs; p.splits = tp_tc_dw_splits(S, n_jobs);
   if (partial_floats < (int64_t)p.splits * n_jobs * 65536) return TP_ERR_WORKSPACE;
-  p.n_tiles = (S + 127) / 128; p.partial = partial; p.swap_strides = flags & 1;
+  p.n_tiles = (S + 127) / 128; p.partial = partial;
   cudaError_t e = cudaFuncSetAttribute(tcb::dw_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)tcb::kDwSmemBytes);
   if (e != cudaSuccess) return (int)e;
@@ -1078,7 +1076,7 @@ TP_API int tp_tc_heads_backward(const float* dz_rgb, const float* dz_trans, int6
   p.b_images = reinterpret_cast<const uint8_t*>(saved); p.b_nslots = tcb::kFwdSlots;
   const int a_slot[6] = {0, 1, 2, 3, 4, 5}, b_slot[6] = {2, 1, 0, 5, 4, 0};
   for (int j = 0; j < 6; ++j) { p.a_slot[j] = a_slot[j]; p.b_slot[j] = b_slot[j]; }
-  p.n_jobs = 6; p.splits = tp_tc_dw_splits(S, 6); p.n_tiles = n_tiles; p.partial = partial; p.swap_strides = 0;
+  p.n_jobs = 6; p.splits = tp_tc_dw_splits(S, 6); p.n_tiles = n_tiles; p.partial = partial;
   e = cudaFuncSetAttribute(tcb::dw_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcb::kDwSmemBytes);
   if (e != cudaSuccess) return (int)e;
   tcb::dw_gemm_kernel<<<p.splits * 6, tcb::kThreads, tcb::kDwSmemBytes, st>>>(p);

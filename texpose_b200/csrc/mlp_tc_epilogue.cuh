@@ -13,8 +13,7 @@ namespace tc {
 // stores are streaming (st.global.cs, evict-first): 1.9 GB per C3 step pass through L2 once and must not displace the 2 MB
 // weight image every CTA keeps re-reading (measured: 1 130 us with bulk stores -> 1 058 us direct -> 970 us streaming).
 template <bool kBias, bool kBits = false>
-__device__ __forceinline__ uint32_t hidden_slab(const uint32_t (&v)[32], const float* bias, uint32_t a_dst, float* dbg_row,
-                                                uint8_t* g_dst = nullptr) {
+__device__ __forceinline__ uint32_t hidden_slab(const uint32_t (&v)[32], const float* bias, uint32_t a_dst, uint8_t* g_dst = nullptr) {
   uint32_t signs = 0u;
 #pragma unroll
   for (int i = 0; i < 32; i += 8) {
@@ -35,10 +34,6 @@ __device__ __forceinline__ uint32_t hidden_slab(const uint32_t (&v)[32], const f
                    q3 = pack_relu_bf16(x[6], x[7]);
     st_shared_v4(a_dst + (i >> 3) * 2048, q0, q1, q2, q3);
     if (kBits && g_dst) st_global_cs_v4(g_dst + (i >> 3) * 2048, q0, q1, q2, q3);
-    if (dbg_row) {
-#pragma unroll
-      for (int e = 0; e < 8; ++e) dbg_row[i + e] = fmaxf(x[e], 0.f);
-    }
   }
   return __brev(~signs);      // element 0 was shifted in first: reverse; positive = sign bit clear
 }
@@ -48,7 +43,7 @@ __device__ __forceinline__ uint32_t hidden_slab(const uint32_t (&v)[32], const f
 // bias row (N % 32 == 0).  8 shuffles per 8 columns replace 2 dependent L2 round trips.
 template <bool kBits = false>
 __device__ __forceinline__ uint32_t hidden_slab_wbias(const uint32_t (&v)[32], const float4 (&mine)[2], int col0, uint32_t a_dst,
-                                                      float* dbg_row, uint8_t* g_dst = nullptr) {
+                                                      uint8_t* g_dst = nullptr) {
   uint32_t signs = 0u;
 #pragma unroll
   for (int i = 0; i < 32; i += 8) {
@@ -72,10 +67,6 @@ __device__ __forceinline__ uint32_t hidden_slab_wbias(const uint32_t (&v)[32], c
                    q3 = pack_relu_bf16(x[6], x[7]);
     st_shared_v4(a_dst + (i >> 3) * 2048, q0, q1, q2, q3);
     if (kBits && g_dst) st_global_cs_v4(g_dst + (i >> 3) * 2048, q0, q1, q2, q3);
-    if (dbg_row) {
-#pragma unroll
-      for (int e = 0; e < 8; ++e) dbg_row[i + e] = fmaxf(x[e], 0.f);
-    }
   }
   return __brev(~signs);
 }
@@ -85,7 +76,7 @@ __device__ __forceinline__ uint32_t hidden_slab_wbias(const uint32_t (&v)[32], c
 // shuffle form costs ~2 000 cycles per table-bias stage (256 warp shuffles per thread against a shuffle unit that serves one
 // warp per cycle): 4 % of a super-tile (scripts/fwd_prof.py: the MMA warp waits 2 700 cycles for the stage after each of them).
 template <bool kBits = false>
-__device__ __forceinline__ uint32_t hidden_slab_sbias(const uint32_t (&v)[32], uint32_t bias_smem, uint32_t a_dst, float* dbg_row,
+__device__ __forceinline__ uint32_t hidden_slab_sbias(const uint32_t (&v)[32], uint32_t bias_smem, uint32_t a_dst,
                                                       uint8_t* g_dst = nullptr) {
   uint32_t signs = 0u;
 #pragma unroll
@@ -106,16 +97,12 @@ __device__ __forceinline__ uint32_t hidden_slab_sbias(const uint32_t (&v)[32], u
                    q3 = pack_relu_bf16(x[6], x[7]);
     st_shared_v4(a_dst + (i >> 3) * 2048, q0, q1, q2, q3);
     if (kBits && g_dst) st_global_cs_v4(g_dst + (i >> 3) * 2048, q0, q1, q2, q3);
-    if (dbg_row) {
-#pragma unroll
-      for (int e = 0; e < 8; ++e) dbg_row[i + e] = fmaxf(x[e], 0.f);
-    }
   }
   return __brev(~signs);
 }
 
 template <int kSlabs, bool kBits = false>
-__device__ __forceinline__ void hidden_epilogue_sbias(uint32_t tmem_d, uint32_t bias_smem, uint32_t a_row, float* dbg_row,
+__device__ __forceinline__ void hidden_epilogue_sbias(uint32_t tmem_d, uint32_t bias_smem, uint32_t a_row,
                                                       uint32_t* words = nullptr, uint8_t* g_row = nullptr) {
   uint32_t va[32], vb[32];
   TP_TMEM_LD32(tmem_d, va);
@@ -123,18 +110,17 @@ __device__ __forceinline__ void hidden_epilogue_sbias(uint32_t tmem_d, uint32_t 
   for (int j = 0; j < kSlabs; j += 2) {
     TP_TMEM_WAIT32(va);
     TP_TMEM_LD32(tmem_d + (j + 1) * 32, vb);
-    const uint32_t w0 = hidden_slab_sbias<kBits>(va, bias_smem + j * 128, a_row + j * 4 * 2048, dbg_row ? dbg_row + j * 32 : nullptr,
-                                                 g_row ? g_row + j * 4 * 2048 : nullptr);
+    const uint32_t w0 = hidden_slab_sbias<kBits>(va, bias_smem + j * 128, a_row + j * 4 * 2048, g_row ? g_row + j * 4 * 2048 : nullptr);
     TP_TMEM_WAIT32(vb);
     if (j + 2 < kSlabs) TP_TMEM_LD32(tmem_d + (j + 2) * 32, va);
     const uint32_t w1 = hidden_slab_sbias<kBits>(vb, bias_smem + (j + 1) * 128, a_row + (j + 1) * 4 * 2048,
-                                                 dbg_row ? dbg_row + (j + 1) * 32 : nullptr, g_row ? g_row + (j + 1) * 4 * 2048 : nullptr);
+                                                 g_row ? g_row + (j + 1) * 4 * 2048 : nullptr);
     if (kBits && words) { __stcs(words + j * 128, w0); __stcs(words + (j + 1) * 128, w1); }
   }
 }
 
 template <int kSlabs, bool kBits = false>
-__device__ __forceinline__ void hidden_epilogue_wbias(uint32_t tmem_d, const float4 (&mine)[2], uint32_t a_row, float* dbg_row,
+__device__ __forceinline__ void hidden_epilogue_wbias(uint32_t tmem_d, const float4 (&mine)[2], uint32_t a_row,
                                                       uint32_t* words = nullptr,        // words: plane j at words[j * 128]
                                                       uint8_t* g_row = nullptr) {       // g_row: this row in the saved tile image
   uint32_t va[32], vb[32];
@@ -143,12 +129,11 @@ __device__ __forceinline__ void hidden_epilogue_wbias(uint32_t tmem_d, const flo
   for (int j = 0; j < kSlabs; j += 2) {
     TP_TMEM_WAIT32(va);
     TP_TMEM_LD32(tmem_d + (j + 1) * 32, vb);
-    const uint32_t w0 = hidden_slab_wbias<kBits>(va, mine, j * 32, a_row + j * 4 * 2048, dbg_row ? dbg_row + j * 32 : nullptr,
-                                                 g_row ? g_row + j * 4 * 2048 : nullptr);
+    const uint32_t w0 = hidden_slab_wbias<kBits>(va, mine, j * 32, a_row + j * 4 * 2048, g_row ? g_row + j * 4 * 2048 : nullptr);
     TP_TMEM_WAIT32(vb);
     if (j + 2 < kSlabs) TP_TMEM_LD32(tmem_d + (j + 2) * 32, va);
     const uint32_t w1 = hidden_slab_wbias<kBits>(vb, mine, (j + 1) * 32, a_row + (j + 1) * 4 * 2048,
-                                                 dbg_row ? dbg_row + (j + 1) * 32 : nullptr, g_row ? g_row + (j + 1) * 4 * 2048 : nullptr);
+                                                 g_row ? g_row + (j + 1) * 4 * 2048 : nullptr);
     if (kBits && words) { __stcs(words + j * 128, w0); __stcs(words + (j + 1) * 128, w1); }
   }
 }
@@ -156,7 +141,7 @@ __device__ __forceinline__ void hidden_epilogue_wbias(uint32_t tmem_d, const flo
 // Whole 128x256 accumulator row of one thread: TMEM loads are software-pipelined (slab j+1 in flight while slab j is
 // converted), ping-ponging two register slabs.
 template <bool kBias, int kSlabs, bool kBits = false>
-__device__ __forceinline__ void hidden_epilogue(uint32_t tmem_d, const float* bias, uint32_t a_row, float* dbg_row,
+__device__ __forceinline__ void hidden_epilogue(uint32_t tmem_d, const float* bias, uint32_t a_row,
                                                 uint32_t* words = nullptr, uint8_t* g_row = nullptr) {
   uint32_t va[32], vb[32];
   TP_TMEM_LD32(tmem_d, va);
@@ -164,12 +149,11 @@ __device__ __forceinline__ void hidden_epilogue(uint32_t tmem_d, const float* bi
   for (int j = 0; j < kSlabs; j += 2) {
     TP_TMEM_WAIT32(va);
     TP_TMEM_LD32(tmem_d + (j + 1) * 32, vb);
-    const uint32_t w0 = hidden_slab<kBias, kBits>(va, bias + j * 32, a_row + j * 4 * 2048, dbg_row ? dbg_row + j * 32 : nullptr,
-                                                  g_row ? g_row + j * 4 * 2048 : nullptr);
+    const uint32_t w0 = hidden_slab<kBias, kBits>(va, bias + j * 32, a_row + j * 4 * 2048, g_row ? g_row + j * 4 * 2048 : nullptr);
     TP_TMEM_WAIT32(vb);
     if (j + 2 < kSlabs) TP_TMEM_LD32(tmem_d + (j + 2) * 32, va);
     const uint32_t w1 = hidden_slab<kBias, kBits>(vb, bias + (j + 1) * 32, a_row + (j + 1) * 4 * 2048,
-                                                  dbg_row ? dbg_row + (j + 1) * 32 : nullptr, g_row ? g_row + (j + 1) * 4 * 2048 : nullptr);
+                                                  g_row ? g_row + (j + 1) * 4 * 2048 : nullptr);
     if (kBits && words) { __stcs(words + j * 128, w0); __stcs(words + (j + 1) * 128, w1); }
   }
 }

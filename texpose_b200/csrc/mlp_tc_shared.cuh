@@ -73,9 +73,6 @@ struct Params {
   uint8_t* scratch;          // gridDim.x x 2 x 64 KB (parked features)
   uint8_t* bits;             // optional [tiles][4][8 planes][128 rows] ReLU bitmask words (training; lives behind `save`)
   uint8_t* save;             // optional [tiles][7][64 KB]: feat, rgb h1..h3, trans h1..h3 tile images for the backward
-  int dbg_layer;
-  float* dbg_out;            // [S,256] post-activation of stage dbg_layer (debug only)
-  int skew;                  // weight chunks tile 0 runs ahead of tile 1 inside a stage (0..2)
   long long prof_offset;     // byte offset of the cycle counters inside `scratch` (-DTP_FWD_PROF builds only)
   int n_layers;              // 17 = all stages; 13 = static only (rendering that needs neither the transient head nor uncert):
                              // the stage list stops after the rgb output, transient outputs are written as zeros.  Host side only:
@@ -95,7 +92,7 @@ struct Params {
   unsigned long long seed;
   const float* wview;        // [3+6L][256] fp32: columns 256.. of mlp_rgb[0].weight, transposed (view-direction inputs)
   int L_view;
-  const float* imgbias_rgb;  // [B,256] rgb-0 bias + light-latent part (tp_tc_image_bias)
+  const float* imgbias_rgb;  // [B,256] rgb-0 bias + light-latent part (tp_tc_image_biases)
   float min_uncert;
   float* o_rgb;              // per-ray outputs (any may be NULL): [B*R,3] x 3, [B*R] x 5
   float* o_rgb_s;

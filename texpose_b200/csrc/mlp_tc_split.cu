@@ -19,7 +19,7 @@
 //     A operand in eight 32-column groups (one mbarrier each): the MMAs of stage L+1 start as soon as the first group is
 //     written and overlap the rest of the drain -- the tensor pipe only idles for the first slab of every drain;
 //   * biases are added in fp32 by the drain (static vectors, the per-ray row of tp_tc_ray_bias, the per-image row of
-//     tp_tc_image_bias): no bf16 rounding of any bias;
+//     tp_tc_image_biases): no bf16 rounding of any bias;
 //   * the stage list is DATA (tp_tc32_forward's `stages`): trunk depth, skip positions and head depths come from the caller's
 //     architecture, not from a table compiled into the kernel.
 //

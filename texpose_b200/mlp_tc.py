@@ -5,8 +5,6 @@ parameter's `_version` changes (SURVEY.md 8b: "re-packed when param._version cha
 """
 from __future__ import annotations
 
-import os
-
 import torch
 
 from . import _C, ops
@@ -162,10 +160,8 @@ def image_biases(cfg, B, lat_trans, lat_light, rgb_p, trans_p):
     return img_r, img_t
 
 
-def forward(cfg, geom, lat_trans, lat_light, feat_p, rgb_p, trans_p, dbg_layer=-1, flags=0, save=False, static_only=False):
-    flags = flags or int(os.environ.get("TEXPOSE_TC_FLAGS", "0"))     # bit 1: 16-epilogue-warp drain instead of the default 8 (A/B)
-    if static_only and not save:
-        flags |= STATIC_ONLY
+def forward(cfg, geom, lat_trans, lat_light, feat_p, rgb_p, trans_p, save=False, static_only=False):
+    flags = STATIC_ONLY if static_only and not save else 0
     if geom.get("mode") != "rays":
         raise NotImplementedError("the fused bf16 kernel is ray-parameterised (forward_samples)")
     if not supported(cfg, feat_p, rgb_p, trans_p):
@@ -186,13 +182,10 @@ def forward(cfg, geom, lat_trans, lat_light, feat_p, rgb_p, trans_p, dbg_layer=-
     density = torch.empty(S, 2, device=dev)
     uncert = torch.empty(S, device=dev)
     scratch = _scratch_for(dev)
-    dbg = torch.zeros(S, _F, device=dev) if dbg_layer >= 0 else None
     images = torch.empty(_C.load().tp_tc_save_bytes(S), dtype=torch.uint8, device=dev) if save else None
     _C.call("tp_tc_nerf_stl_forward", ops._p(center), ops._p(ray), ops._p(depth), S, N, per_image, ops._p(pk.weights),
             ops._p(pk.biasbuf), ops._p(raybias), ops._p(img_t), ops._p(rgb), ops._p(density), ops._p(uncert),
-            ops._p(scratch), scratch.numel(), ops._p(images), dbg_layer, ops._p(dbg), flags, ops._stream())
-    if dbg_layer >= 0:
-        return rgb, density, uncert, dbg
+            ops._p(scratch), scratch.numel(), ops._p(images), flags, ops._stream())
     if save:
         return rgb, density, uncert, images
     return rgb, density, uncert

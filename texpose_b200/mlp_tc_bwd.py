@@ -59,7 +59,7 @@ def reduce_partials(partial, splits, count, out=None):
     return out
 
 
-def dw_gemm(a_images, a_nslots, b_images, b_nslots, pairs, S, flags=0):
+def dw_gemm(a_images, a_nslots, b_images, b_nslots, pairs, S):
     """[len(pairs),256,256] fp32: job j = dz[a]^T x[b] over all samples -- one launch, split over tiles, fixed-order reduce."""
     n = len(pairs)
     splits = _C.load().tp_tc_dw_splits(S, n)
@@ -67,7 +67,7 @@ def dw_gemm(a_images, a_nslots, b_images, b_nslots, pairs, S, flags=0):
     a_s = (ctypes.c_int32 * n)(*[a for a, _ in pairs])
     b_s = (ctypes.c_int32 * n)(*[b for _, b in pairs])
     _C.call("tp_tc_dw_gemm", ops._p(a_images), a_nslots, ops._p(b_images), b_nslots, a_s, b_s, n, S, ops._p(partial),
-            partial.numel(), flags, ops._stream())
+            partial.numel(), ops._stream())
     return reduce_partials(partial, splits, n * 65536).view(n, 256, 256)
 
 
