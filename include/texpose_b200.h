@@ -262,6 +262,18 @@ int tp_tc32_forward(const float* center, const float* ray, const float* depth, i
                     const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
                     const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,
                     int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot, void* stream);
+/* The split-mode forward (precision 0 arithmetic, outputs bit-identical to tp_tc32_forward's) of a <= 1e-4 TRAINING step
+ * (autograd of layers/nerf.py:61-99 and layers/nerf_static_transient_light.py:104-137 at fp32 parity): `save` (required, n_save >= 1)
+ * [ceil(S/128)][2 n_save][64 KB] receives every save-slot activation, and slot enc_slot the encoding tile [xyz, enc(xyz), 1, 0...],
+ * as bf16 hi / lo tile images (slot 2k = bf16(x), 2k + 1 = bf16(x - hi)), then [ceil(S/128)][n_save][4 KB] ReLU bitmasks -- the
+ * operands of tp_tc_chain_backward_split and of tp_tc_dw_gemm / tp_tc_images_colsum / tp_tc_thin_dw / tp_tc_image_ray_sums, which
+ * address hi and lo as ordinary slots.  bf16 rather than the forward's fp16: the backward's operands need fp32's exponent range.
+ * Same stage list, checks, scratch and status word as tp_tc32_forward. */
+int64_t tp_tc32_split_save_bytes(int64_t S, int n_save);
+int tp_tc32_forward_split_save(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
+                               const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
+                               const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,
+                               int64_t scratch_bytes, void* save, int n_save, int enc_slot, void* stream);
 
 /* ---- tensor-core backward of the two heads on the saved tile images (K2b, bf16 mode) ------------------------- */
 
@@ -351,6 +363,18 @@ int tp_tc_chain_max_stages(void);
 int tp_tc_chain_backward(const float* thin0, int cols0, const float* thin1, int cols1, int64_t S, const void* packed_bwd,
                          int n_chunks, const int32_t* stages, int n_stages, const void* mask_bits, int n_saved, void* dz_out,
                          int n_out, void* stream);
+/* The same dX chain at fp32 parity (K2c, csrc/mlp_tc_chain.cu): dz, the thin operands and the weights carried as bf16 hi + lo,
+ * three tcgen05.mma passes per K = 16 step (dz_hi W_hi + dz_hi W_lo + dz_lo W_hi, fp32 accumulate).  packed_bwd: n_chunks x 16 KB
+ * K = 16 slots [W^T hi 8 KB | W^T lo 8 KB] from tp_tc_pack_weights_split; stage rows as tp_tc_chain_backward's, except that the
+ * number of chunks a stage reads against the previous output is 0 | 16 (K = 16 slots) and the thin operand's chunk is one slot.
+ * mask_bits: the bitmasks of tp_tc32_forward_split_save (at byte offset tiles * 2 * n_save * 65536 of its save buffer);
+ * dz_out [tiles][2 n_out][64 KB]: stage output slot k is written as hi (image 2k) and lo (image 2k + 1). */
+int tp_tc_chain_backward_split(const float* thin0, int cols0, const float* thin1, int cols1, int64_t S, const void* packed_bwd,
+                               int n_chunks, const int32_t* stages, int n_stages, const void* mask_bits, int n_saved, void* dz_out,
+                               int n_out, void* stream);
+/* chunk_desc: DEVICE int64 [n_chunks,10] rows as tp_tc_pack_weights' with n_layout 256 and no bias; each row is ONE K = 16 step
+ * (cols_valid <= 16): 8 KB bf16(W) then 8 KB bf16(W - bf16(W)), each [2 k8][256 n][8]. */
+int tp_tc_pack_weights_split(const int64_t* chunk_desc, int n_chunks, void* packed, void* stream);
 
 /* ---- K7: mesh depth / NOCS / colour rasteriser (SURVEY 8 f4) --------------------------------------------------------
  * tools/mvrenderer.py:33-178 as compute_surfelinfo.py:114-116 calls it (pytorch3d MeshRasterizer, faces_per_pixel 1, blur 0,

@@ -108,8 +108,13 @@ __device__ __forceinline__ void umma3(uint32_t d, uint32_t ah, uint32_t al, uint
 // kSingle = false: the fp32-parity mode (fp16 hi + lo, three passes).  kSingle = true: ONE pass with bf16 operands -- the general-
 // architecture bf16 forward (any stage list; <= 1e-2 like mlp_tc.cu, which stays the fast path for the yaml's architecture), whose
 // drain can also keep every hidden activation as a bf16 tile image for the tensor-core backward (training of layers/nerf.py).
-template <bool kSingle>
-__global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const Params p) {
+// kSplitSave (with kSingle = false): the parity-mode arithmetic unchanged, and the drain also keeps every save-slot activation and
+// the encoding tile as bf16 hi + lo tile images (slots 2k, 2k + 1) plus the ReLU bitmasks: the operands of the split backward.
+template <bool kSingle, bool kSplitSave>
+__device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
+  static_assert(!(kSingle && kSplitSave), "the split save belongs to the three-pass arithmetic");
+  constexpr bool kSave = kSingle || kSplitSave;      // the launch can write tile images
+  constexpr int kImgPerSlot = kSplitSave ? 2 : 1;     // tile images per save slot (hi, lo)
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
@@ -280,7 +285,9 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const P
           v[3 + j * 2 * kEncL + kEncL + k] = cs;
         }
       }
-      uint8_t* const g_enc = (kSingle && p.save && p.enc_slot >= 0) ? p.save + ((size_t)tile * p.n_save + p.enc_slot) * kABytes + row * 16 : nullptr;
+      uint8_t* const g_enc = (kSave && p.save && p.enc_slot >= 0)
+                                 ? p.save + ((size_t)tile * kImgPerSlot * p.n_save + kImgPerSlot * p.enc_slot) * kABytes + row * 16
+                                 : nullptr;
       v[63] = g_enc ? 1.f : 0.f;      // (no layer has a weight column 63: the packed images hold zeros there)
 #pragma unroll
       for (int k8 = 0; k8 < 8; ++k8) {
@@ -292,11 +299,22 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const P
         }
         st_shared_v4(sbase + kOffEhi + k8 * 2048 + row * 16, h[0], h[1], h[2], h[3]);
         if (!kSingle) st_shared_v4(sbase + kOffElo + k8 * 2048 + row * 16, l[0], l[1], l[2], l[3]);
-        if (g_enc) st_global_cs_v4(g_enc + k8 * 2048, h[0], h[1], h[2], h[3]);
+        if (kSplitSave && g_enc) {
+#pragma unroll
+          for (int e = 0; e < 4; ++e) split2_bf16(v[k8 * 8 + 2 * e], v[k8 * 8 + 2 * e + 1], h[e], l[e]);
+          st_global_cs_v4(g_enc + k8 * 2048, h[0], h[1], h[2], h[3]);
+          st_global_cs_v4(g_enc + kABytes + k8 * 2048, l[0], l[1], l[2], l[3]);
+        } else if (g_enc) {
+          st_global_cs_v4(g_enc + k8 * 2048, h[0], h[1], h[2], h[3]);
+        }
       }
       if (g_enc) {
 #pragma unroll 4
         for (int k8 = 8; k8 < 32; ++k8) st_global_cs_v4(g_enc + k8 * 2048, 0u, 0u, 0u, 0u);
+        if (kSplitSave) {
+#pragma unroll 4
+          for (int k8 = 8; k8 < 32; ++k8) st_global_cs_v4(g_enc + kABytes + k8 * 2048, 0u, 0u, 0u, 0u);
+        }
       }
       fence_proxy_async_smem();
       __syncwarp();
@@ -330,7 +348,9 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const P
                                                            : p.imgbias + (s / p.per_image) * 256) + half * 128;
           const uint32_t tmem_d = tmem_row + (uint32_t)(L & 1) * 256 + half * 128;
           const bool do_park = (sg.flags & F_PARK) != 0;
-          uint8_t* const g_save = (kSingle && p.save && sg.save_slot >= 0) ? p.save + ((size_t)tile * p.n_save + sg.save_slot) * kABytes : nullptr;
+          uint8_t* const g_save = (kSave && p.save && sg.save_slot >= 0)
+                                      ? p.save + ((size_t)tile * kImgPerSlot * p.n_save + kImgPerSlot * sg.save_slot) * kABytes
+                                      : nullptr;
           uint32_t* const g_bits = g_save ? p.save_bits + ((size_t)tile * p.n_save + sg.save_slot) * 1024 + half * 4 * 128 + row : nullptr;
           // one 32-column slab: + bias, ReLU, hi / lo split, 4 core-matrix rows of A_hi and A_lo (and of the parked copy)
           // the slab's 32 bias values are fetched one slab ahead (beside the TMEM load): loads issued inside the conversion loop
@@ -367,7 +387,19 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const P
                 st_global_v4(park + off, h[0], h[1], h[2], h[3]);
                 if (!kSingle) st_global_v4(park + kABytes + off, l[0], l[1], l[2], l[3]);
               }
-              if (g_save) st_global_cs_v4(g_save + off, h[0], h[1], h[2], h[3]);
+              if (kSplitSave && g_save) {      // (recomputed here, after the fp16 words are stored: fewer live registers)
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                  const float x0 = __uint_as_float(v[i * 8 + 2 * e]) + bb[2 * e], x1 = __uint_as_float(v[i * 8 + 2 * e + 1]) + bb[2 * e + 1];
+                  split2_bf16(fmaxf(x0, 0.f), fmaxf(x1, 0.f), h[e], l[e]);
+                  positive = __funnelshift_l(__float_as_uint(x0), positive, 1);
+                  positive = __funnelshift_l(__float_as_uint(x1), positive, 1);
+                }
+                st_global_cs_v4(g_save + off, h[0], h[1], h[2], h[3]);
+                st_global_cs_v4(g_save + kABytes + off, l[0], l[1], l[2], l[3]);
+              } else if (g_save) {
+                st_global_cs_v4(g_save + off, h[0], h[1], h[2], h[3]);
+              }
             }
             if (g_bits) g_bits[j * 128] = __brev(~positive);      // bit c = column c of the slab is positive (sign bit clear)
             if (do_park) __threadfence();      // the parked copy is read back through the async proxy (bulk load) four stages later
@@ -437,6 +469,15 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const P
   }
 }
 
+template <bool kSingle>
+__global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const Params p) {
+  nerf_forward_split_body<kSingle, false>(p);
+}
+// the parity-mode forward of a training step: tile images and ReLU bitmasks in the split backward's format
+__global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_save_kernel(const Params p) {
+  nerf_forward_split_body<false, true>(p);
+}
+
 // slot_desc row: [W ptr, ld, row0, rows_valid, col0, cols_valid, kind (256 | 16), unused]
 //   kind 256: slot = [hi | lo], each [2 k8][256 rows][8]: element (n, kl) = W[row0 + n][col0 + kl], kl < 16
 //   kind 16:  first 8 KB = [32 k8][16 rows][8]: rows 0..7 hi, rows 8..15 lo of W[row0 + (n & 7)][col0 + kl], kl < 256
@@ -492,13 +533,17 @@ TP_API int tp_tc32_pack_weights(const int64_t* slot_desc, int n_slots, int preci
   return tp_launch_status();
 }
 
-TP_API int tp_tc32_forward(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
-                           const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
-                           const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert,
-                           void* scratch, int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot, void* stream) {
-  if (!center || !ray || !depth || !image || !stages || !bias || !rgb || !density || !uncert || !scratch) return TP_ERR_BAD_ARG;
-  if (S < 0 || N < 1 || per_image < 1 || n_stages < 1 || n_stages > tcs::kMaxStages) return TP_ERR_BAD_SHAPE;
-  if ((precision != 0 && precision != 1) || (save && (precision != 1 || n_save < 1)) || ((uintptr_t)save & 15)) return TP_ERR_BAD_ARG;
+/* bytes of the save buffer of a split-save launch: [tiles][2 n_save][64 KB] hi / lo tile images, then [tiles][n_save][4 KB] bitmasks */
+TP_API int64_t tp_tc32_split_save_bytes(int64_t S, int n_save) {
+  return ((S + 127) / 128) * (int64_t)n_save * (2 * tc::kABytes + 4096);
+}
+
+// shared by tp_tc32_forward and tp_tc32_forward_split_save: the argument and stage-list checks, then the launch
+static int tc32_forward_launch(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
+                               const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
+                               const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert,
+                               void* scratch, int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot,
+                               bool split_save, void* stream) {
   if (enc_slot < -1 || (enc_slot >= 0 && (!save || enc_slot >= n_save))) return TP_ERR_BAD_ARG;
   if (((uintptr_t)image & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)bias & 15) || ((uintptr_t)raybias & 15) ||
       ((uintptr_t)imgbias & 15) || ((uintptr_t)rgb & 7) || ((uintptr_t)density & 7))
@@ -553,10 +598,35 @@ TP_API int tp_tc32_forward(const float* center, const float* ray, const float* d
   p.status = reinterpret_cast<unsigned int*>(p.scratch + tp_tc32_status_offset());
   p.n_stages = n_stages;
   p.save = reinterpret_cast<uint8_t*>(save); p.n_save = n_save; p.enc_slot = save ? enc_slot : -1;
-  p.save_bits = save ? reinterpret_cast<uint32_t*>(p.save + (size_t)((S + 127) / 128) * n_save * tc::kABytes) : nullptr;
-  void (*kern)(const tcs::Params) = precision ? tcs::nerf_forward_split_kernel<true> : tcs::nerf_forward_split_kernel<false>;
+  const size_t images_per_slot = split_save ? 2 : 1;
+  p.save_bits = save ? reinterpret_cast<uint32_t*>(p.save + (size_t)((S + 127) / 128) * n_save * images_per_slot * tc::kABytes) : nullptr;
+  void (*kern)(const tcs::Params) = split_save ? tcs::nerf_forward_split_save_kernel
+                                    : precision ? tcs::nerf_forward_split_kernel<true> : tcs::nerf_forward_split_kernel<false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcs::kSmemBytes);
   if (e != cudaSuccess) return (int)e;
   kern<<<grid, tcs::kThreads, tcs::kSmemBytes, (cudaStream_t)stream>>>(p);
   return tp_launch_status();
+}
+
+TP_API int tp_tc32_forward(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
+                           const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
+                           const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert,
+                           void* scratch, int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot, void* stream) {
+  if (!center || !ray || !depth || !image || !stages || !bias || !rgb || !density || !uncert || !scratch) return TP_ERR_BAD_ARG;
+  if (S < 0 || N < 1 || per_image < 1 || n_stages < 1 || n_stages > tcs::kMaxStages) return TP_ERR_BAD_SHAPE;
+  if ((precision != 0 && precision != 1) || (save && (precision != 1 || n_save < 1)) || ((uintptr_t)save & 15)) return TP_ERR_BAD_ARG;
+  return tc32_forward_launch(center, ray, depth, S, N, per_image, image, n_slots, stages, n_stages, bias, raybias, imgbias, rgb,
+                             density, uncert, scratch, scratch_bytes, precision, save, n_save, enc_slot, false, stream);
+}
+
+TP_API int tp_tc32_forward_split_save(const float* center, const float* ray, const float* depth, int64_t S, int N,
+                                      int64_t per_image, const void* image, int n_slots, const int32_t* stages, int n_stages,
+                                      const float* bias, const float* raybias, const float* imgbias, float* rgb, float* density,
+                                      float* uncert, void* scratch, int64_t scratch_bytes, void* save, int n_save, int enc_slot,
+                                      void* stream) {
+  if (!center || !ray || !depth || !image || !stages || !bias || !rgb || !density || !uncert || !scratch || !save) return TP_ERR_BAD_ARG;
+  if (S < 0 || N < 1 || per_image < 1 || n_stages < 1 || n_stages > tcs::kMaxStages || n_save < 1) return TP_ERR_BAD_SHAPE;
+  if ((uintptr_t)save & 15) return TP_ERR_ALIGN;
+  return tc32_forward_launch(center, ray, depth, S, N, per_image, image, n_slots, stages, n_stages, bias, raybias, imgbias, rgb,
+                             density, uncert, scratch, scratch_bytes, 0, save, n_save, enc_slot, true, stream);
 }

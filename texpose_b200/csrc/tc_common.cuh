@@ -179,6 +179,12 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
   return d;
 }
+// hi / lo bf16 words of two fp32 values (x0 in the low half): hi = bf16(x), lo = bf16(x - hi) -> x to ~16 significand bits, with
+// fp32's exponent range (the operand format of the fp32-parity backward: gradients far below fp16's normal range keep their bits)
+__device__ __forceinline__ void split2_bf16(float x0, float x1, uint32_t& hi, uint32_t& lo) {
+  hi = pack_bf16(x0, x1);
+  lo = pack_bf16(x0 - __uint_as_float(hi << 16), x1 - __uint_as_float(hi & 0xffff0000u));
+}
 __device__ __forceinline__ uint4 ld_shared_v4(uint32_t addr) {
   uint4 v;
   asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");

@@ -6,8 +6,10 @@ reference are never materialised: each layer reads a *segmented* input (see tp_l
 
 Two arithmetic modes:
   fp32  -- the <=1e-4 parity mode: SIMT FFMA kernels (mlp_simt.cu), forward and backward; calls that record no gradient
-           (rendering) run on the tensor cores with split-bf16 operands instead (mlp_tc_split.cu, three MMA passes per K
+           (rendering) run on the tensor cores with split-fp16 operands instead (mlp_tc_split.cu, three MMA passes per K
            step), for any 256-wide static/transient/light architecture (opt.b200.fp32_engine = 'simt' keeps them on SIMT);
+           with opt.b200.fp32_engine = 'tc' a gradient-recording ray-mode call trains the heads on the tensor cores too (split
+           forward with bf16 hi / lo activation save, split dX chain, dW GEMMs on the hi / lo images: mlp_tc_bwd, split flag);
   bf16  -- fused tcgen05/TMEM forward (mlp_tc.cu) for the static/transient/light model; in training it also saves
            the head activations (bf16 tile images) that the backward consumes.
 """
@@ -39,6 +41,7 @@ class MLPConfig:
     packed: object = None       # bf16 weight image for the tcgen05 kernel (mlp_tc.pack), or None
     static_only: bool = False   # rendering only: skip the transient head (its outputs come back as zeros), fused kernel only
     fp32_tc: bool = True        # fp32 mode, no gradient wanted: split-bf16 tensor-core kernel (mlp_tc32) instead of SIMT FFMA
+    fp32_train_tc: bool = False  # fp32 mode, gradient wanted: split staged kernels instead of SIMT (opt.b200.fp32_engine = 'tc')
 
     @property
     def stl(self) -> bool:
@@ -247,7 +250,7 @@ class NerfMLP(torch.autograd.Function):
                     and mlp_tc32.supported(cfg, feat_p, rgb_p, trans_p):
                 # bf16 on an architecture the lock-step kernel is not specialised for: single-pass launch of the staged kernel
                 use_tc32, single, use_tc = True, 1, False
-        staged_train = False
+        staged_train = split_train = False
         if sv is not None and cfg.stl and not trunk_grad and cfg.precision in ("bf16", "auto") and geom.get("mode") == "rays":
             from .. import mlp_tc, mlp_tc32, mlp_tc_bwd
             # training on the staged kernels: an architecture the lock-step kernel / fused backward are not specialised for, or
@@ -255,11 +258,18 @@ class NerfMLP(torch.autograd.Function):
             lockstep = mlp_tc.supported(cfg, feat_p, rgb_p, trans_p) and mlp_tc_bwd.fused_supported(S, per_image)
             staged_train = not lockstep and mlp_tc32.supported(cfg, feat_p, rgb_p, trans_p) \
                 and (len(rgb_p) - 1) + (len(trans_p) - 1) + 1 <= 16
+        if sv is not None and cfg.stl and not trunk_grad and cfg.precision == "fp32" and cfg.fp32_train_tc \
+                and geom.get("mode") == "rays":
+            from .. import mlp_tc32
+            # the <= 1e-4 training step on the tensor cores: the staged kernels in their split form
+            staged_train = split_train = mlp_tc32.supported(cfg, feat_p, rgb_p, trans_p) \
+                and (len(rgb_p) - 1) + (len(trans_p) - 1) + 1 <= 16
         if staged_train:
             from .. import mlp_tc32
-            rgb, density, uncert, (images, n_save) = mlp_tc32.forward(cfg, geom, lt, ll, feat_p, rgb_p, trans_p, precision=1,
-                                                                      save="heads")
+            rgb, density, uncert, (images, n_save) = mlp_tc32.forward(cfg, geom, lt, ll, feat_p, rgb_p, trans_p,
+                                                                      precision=0 if split_train else 1, save="heads")
             sv.images, sv.n_save, sv.staged, sv.geom, sv.lat = images, n_save, True, geom, (lt, ll)
+            sv.split = split_train
             sv.rgb, sv.density, sv.uncert = rgb, density, uncert
         elif use_tc32:
             from .. import mlp_tc32
@@ -296,12 +306,16 @@ class NerfMLP(torch.autograd.Function):
         need = ctx.needs_input_grad[4:]
         g = lambda t: t.contiguous().float() if t is not None else None
         if getattr(sv, "images", None) is not None:
-            # bf16 mode: the backward of whichever kernels the forward chose -- the fused backward on the tile images the lock-step
-            # forward saved (csrc/mlp_tc_bwd.cu), or the staged kernels (csrc/mlp_tc_chain.cu)
+            # tensor-core training: the backward of whichever kernels the forward chose -- the fused backward on the tile images the
+            # lock-step forward saved (csrc/mlp_tc_bwd.cu), or the staged kernels (csrc/mlp_tc_chain.cu; split = the fp32 step)
             from .. import mlp_tc_bwd
-            fn = mlp_tc_bwd.heads_backward_staged if getattr(sv, "staged", False) else mlp_tc_bwd.heads_backward
-            gr, gt, d_lt, d_ll = fn(cfg, sv, S, ctx.per_image, rgb_p, trans_p, g(g_rgb), g(g_density),
-                                    g(g_uncert), bool(ctx.needs_input_grad[2]), bool(ctx.needs_input_grad[3]))
+            if getattr(sv, "staged", False):
+                gr, gt, d_lt, d_ll = mlp_tc_bwd.heads_backward_staged(
+                    cfg, sv, S, ctx.per_image, rgb_p, trans_p, g(g_rgb), g(g_density), g(g_uncert),
+                    bool(ctx.needs_input_grad[2]), bool(ctx.needs_input_grad[3]), split=sv.split)
+            else:
+                gr, gt, d_lt, d_ll = mlp_tc_bwd.heads_backward(cfg, sv, S, ctx.per_image, rgb_p, trans_p, g(g_rgb), g(g_density),
+                                                               g(g_uncert), bool(ctx.needs_input_grad[2]), bool(ctx.needs_input_grad[3]))
             out = [None] * n_f
             for layers in (gr, gt):
                 for pair in layers:

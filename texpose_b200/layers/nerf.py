@@ -61,7 +61,8 @@ class NeRF(torch.nn.Module):
 
     def forward_samples(self, opt, center, ray, depth_samples, mode=None):
         """layers/nerf.py:101-115.  Rendering (no gradient needed) with opt.b200.mlp 'bf16' / 'auto' runs on the fused
-        tcgen05 kernel; training the plain model needs the trunk's backward and stays on the fp32 kernels."""
+        tcgen05 kernel, with 'fp32' on the split-fp16 kernel; training runs on the tensor cores with 'bf16' / 'auto', and with
+        'fp32' when opt.b200.fp32_engine = 'tc' (trains_on_tensor_cores); otherwise on the fp32 SIMT kernels."""
         cfg = self._config(opt, mode)
         geom = _common.ray_geometry(cfg, center, ray, depth_samples)
         if geom["S"] > 0 and self.uses_tensor_cores(opt):
@@ -70,7 +71,8 @@ class NeRF(torch.nn.Module):
             return self._forward_tc32(cfg, geom)
         if geom["S"] > 0 and self.trains_on_tensor_cores(opt, cfg):
             from .. import mlp_tc_plain
-            return mlp_tc_plain.PlainTC.apply(cfg, geom, len(self.mlp_feat), *_common.flat_params(self.mlp_feat, self.mlp_rgb))
+            split = _common.mlp_precision(opt) == "fp32"
+            return mlp_tc_plain.PlainTC.apply(cfg, geom, len(self.mlp_feat), split, *_common.flat_params(self.mlp_feat, self.mlp_rgb))
         return run_mlp(cfg, geom, None, None, *_common.flat_params(self.mlp_feat, self.mlp_rgb))
 
     # ------------------------------------------------------------------ tensor-core rendering path
@@ -137,8 +139,11 @@ class NeRF(torch.nn.Module):
 
     def trains_on_tensor_cores(self, opt, cfg=None) -> bool:
         """True when a gradient-recording forward_samples takes the tensor-core training path (mlp_tc_plain: single-pass bf16
-        forward with saved activations, staged dX chain, dW GEMMs): opt.b200.mlp 'bf16' / 'auto' and a supported architecture."""
-        if _common.mlp_precision(opt) == "fp32" or not torch.is_grad_enabled():
+        forward with saved activations, staged dX chain, dW GEMMs): opt.b200.mlp 'bf16' / 'auto', or 'fp32' with
+        opt.b200.fp32_engine = 'tc' (the split kernels, <= 1e-4), and a supported architecture."""
+        if not torch.is_grad_enabled():
+            return False
+        if _common.mlp_precision(opt) == "fp32" and _common.b200_option(opt, "fp32_engine", "auto") != "tc":
             return False
         from .. import mlp_tc_plain
         cfg = cfg or self._config(opt, None)

@@ -75,7 +75,8 @@ class NeRF(torch.nn.Module):
                          n_latent_trans=opt.nerf.N_latent_trans, precision=_common.mlp_precision(opt),
                          save_for_backward=torch.is_grad_enabled(), packed=self,
                          static_only=bool(mode == "eval" and _common.b200_option(opt, "static_only", False)),
-                         fp32_tc=_common.b200_option(opt, "fp32_engine", "auto") != "simt")
+                         fp32_tc=_common.b200_option(opt, "fp32_engine", "auto") != "simt",
+                         fp32_train_tc=_common.b200_option(opt, "fp32_engine", "auto") == "tc")
 
     def uses_tensor_cores(self, opt, mode="val") -> bool:
         """True when forward_samples of this module will take the fused tcgen05 path under `opt` (opt.b200.mlp)."""

@@ -2,8 +2,9 @@
 
 The kernel takes its stage list as data, so this module derives it from the caller's architecture (trunk depth, skip
 positions, head depths: `opt.arch` of the reference yaml files) instead of relying on a table compiled into the kernel.
-Every layer is carried as hi + lo bf16 (three MMA passes per K step): <= 1e-4 against the reference where the bf16
-kernel (mlp_tc.py) is <= 1e-2.  Inference only (no activation save); training in the parity mode stays on mlp_simt.cu.
+Every layer is carried as hi + lo fp16 (three MMA passes per K step): <= 1e-4 against the reference where the bf16
+kernel (mlp_tc.py) is <= 1e-2.  A training step in the parity mode (opt.b200.fp32_engine = 'tc') uses the split-save launch,
+which also keeps the activations as bf16 hi + lo tile images for the split backward (mlp_tc_plain, mlp_tc_bwd).
 """
 from __future__ import annotations
 
@@ -172,7 +173,8 @@ def check_range(device=None):
 
 def forward(cfg, geom, lat_trans, lat_light, feat_p, rgb_p, trans_p, static_only=False, precision=0, save=False):
     """NeRF.forward_samples (layers/nerf_static_transient_light.py:147-166) -> rgb [S,3,2], density [S,2], uncert [S]
-    (+ (images, n_save) with save: the bf16 tile images of every hidden activation, single-pass launch only)."""
+    (+ (images, n_save) with save: the tile images of every hidden activation -- bf16 for the single-pass launch (precision 1),
+    bf16 hi / lo pairs, images 2k and 2k + 1 of save slot k, for the split launch (precision 0, tp_tc32_forward_split_save))."""
     if geom.get("mode") != "rays":
         raise NotImplementedError("the tensor-core kernels are ray-parameterised (forward_samples)")
     if not supported(cfg, feat_p, rgb_p, trans_p):
@@ -193,8 +195,15 @@ def forward(cfg, geom, lat_trans, lat_light, feat_p, rgb_p, trans_p, static_only
     scratch = _scratch_for(dev)
     images = None
     if save:
-        assert precision == 1, "activations are saved by the single-pass (bf16) launch"
-        images = torch.empty(_C.load().tp_tc32_save_bytes(S, pk.n_save), dtype=torch.uint8, device=dev)      # tile images, then ReLU bitmasks
+        lib = _C.load()
+        nbytes = lib.tp_tc32_save_bytes(S, pk.n_save) if precision else lib.tp_tc32_split_save_bytes(S, pk.n_save)
+        images = torch.empty(nbytes, dtype=torch.uint8, device=dev)      # tile images, then ReLU bitmasks
+    if save and precision == 0:
+        _C.call("tp_tc32_forward_split_save", ops._p(center), ops._p(ray), ops._p(depth), S, N, per_image, ops._p(pk.image),
+                pk.n_slots, ops._p(pk.stages), pk.stages.shape[0], ops._p(pk.bias), ops._p(raybias), ops._p(img_t), ops._p(rgb),
+                ops._p(density), ops._p(uncert), ops._p(scratch), scratch.numel(), ops._p(images), pk.n_save, pk.n_save - 1,
+                ops._stream())
+        return rgb, density, uncert, (images, pk.n_save)
     _C.call("tp_tc32_forward", ops._p(center), ops._p(ray), ops._p(depth), S, N, per_image, ops._p(pk.image), pk.n_slots,
             ops._p(pk.stages), pk.stages.shape[0], ops._p(pk.bias), ops._p(raybias), ops._p(img_t), ops._p(rgb),
             ops._p(density), ops._p(uncert), ops._p(scratch), scratch.numel(), int(precision), ops._p(images), pk.n_save if save else 0,

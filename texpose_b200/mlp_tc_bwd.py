@@ -1,8 +1,9 @@
 """Host side of the tensor-core backward of the two heads (bf16 mode): transposed weight image, kernel sequencing.
 
 Two backwards, one per forward: `heads_backward` (csrc/mlp_tc_bwd.cu, tp_tc_heads_backward) after the lock-step forward, and
-`heads_backward_staged` (csrc/mlp_tc_chain.cu + the dW GEMM and thin helpers here) after the single-pass staged forward.
-NerfMLP.forward picks the forward, and with it the backward.
+`heads_backward_staged` (csrc/mlp_tc_chain.cu + the dW GEMM and thin helpers here) after the single-pass staged forward -- or,
+with split = True, after the split-save forward of the fp32-parity step.  NerfMLP.forward picks the forward, and with it the
+backward.
 
 Gradient sinks are the reference's: mlp_rgb.*, mlp_trans.*, the two latents (model/nerf_adapt_st_gan.py:56-69,108-127);
 the trunk is frozen (layers/nerf_static_transient_light.py:34).
@@ -59,8 +60,18 @@ def reduce_partials(partial, splits, count, out=None):
     return out
 
 
-def dw_gemm(a_images, a_nslots, b_images, b_nslots, pairs, S):
-    """[len(pairs),256,256] fp32: job j = dz[a]^T x[b] over all samples -- one launch, split over tiles, fixed-order reduce."""
+# split = True: the images are the fp32-parity backward's (tp_tc32_forward_split_save, tp_tc_chain_backward_split): every logical
+# slot k is the pair of bf16 images 2k (hi) and 2k + 1 (lo), and the helpers below run the bf16 kernels on both and add the parts
+# in a fixed order (tp_reduce_partials).  Slot numbers and slot counts passed in are logical.
+
+def dw_gemm(a_images, a_nslots, b_images, b_nslots, pairs, S, split=False):
+    """[len(pairs),256,256] fp32: job j = dz[a]^T x[b] over all samples -- one launch per 12 jobs, split over tiles, fixed-order
+    reduce.  split: three jobs per pair, (dz_hi, x_hi) + (dz_hi, x_lo) + (dz_lo, x_hi) (the dropped lo x lo term is ~2^-17)."""
+    if split:
+        n = len(pairs)
+        jobs = [(2 * a + i, 2 * b + j) for i, j in ((0, 0), (0, 1), (1, 0)) for a, b in pairs]      # term-major
+        parts = torch.cat([dw_gemm(a_images, 2 * a_nslots, b_images, 2 * b_nslots, jobs[k:k + 12], S) for k in range(0, len(jobs), 12)])
+        return reduce_partials(parts, 3, n * 65536).view(n, 256, 256)
     n = len(pairs)
     splits = _C.load().tp_tc_dw_splits(S, n)
     partial = torch.empty(splits * n * 65536, device=a_images.device)
@@ -71,20 +82,29 @@ def dw_gemm(a_images, a_nslots, b_images, b_nslots, pairs, S):
     return reduce_partials(partial, splits, n * 65536).view(n, 256, 256)
 
 
-def images_colsum(images, n_slots, S, slots):
+def images_colsum(images, n_slots, S, slots, split=False):
     """[len(slots),256]: column sums over all samples of the selected image slots (bias gradients), one launch + one reduce."""
     lib = _C.load()
-    blocks, n = lib.tp_tc_images_colsum_blocks(), len(slots)
-    sel = ops.device_table(list(slots), torch.int32, images.device)
-    partial = torch.empty(blocks * n * 256, device=images.device)
-    _C.call("tp_tc_images_colsum", ops._p(images), n_slots, S, ops._p(sel), n, ops._p(partial), partial.numel(), ops._stream())
-    return reduce_partials(partial, blocks, n * 256).view(n, 256)
+    n = len(slots)
+    sel_slots = [2 * s for s in slots] + [2 * s + 1 for s in slots] if split else list(slots)
+    blocks, n_sel = lib.tp_tc_images_colsum_blocks(), len(sel_slots)
+    sel = ops.device_table(sel_slots, torch.int32, images.device)
+    partial = torch.empty(blocks * n_sel * 256, device=images.device)
+    _C.call("tp_tc_images_colsum", ops._p(images), n_slots * (2 if split else 1), S, ops._p(sel), n_sel, ops._p(partial),
+            partial.numel(), ops._stream())
+    return reduce_partials(partial, blocks * (n_sel // n), n * 256).view(n, 256)      # [blocks][hi | lo][n][256]
 
 
-def image_ray_sums(images, slot, n_slots, S, N):
-    out = torch.empty((S + N - 1) // N, 256, device=images.device)
-    _C.call("tp_tc_image_ray_sums", ops._p(images), slot, n_slots, S, N, ops._p(out), ops._stream())
-    return out
+def image_ray_sums(images, slot, n_slots, S, N, split=False):
+    rays = (S + N - 1) // N
+    if not split:
+        out = torch.empty(rays, 256, device=images.device)
+        _C.call("tp_tc_image_ray_sums", ops._p(images), slot, n_slots, S, N, ops._p(out), ops._stream())
+        return out
+    parts = torch.empty(2, rays, 256, device=images.device)
+    for i in range(2):
+        _C.call("tp_tc_image_ray_sums", ops._p(images), 2 * slot + i, 2 * n_slots, S, N, ops._p(parts[i]), ops._stream())
+    return reduce_partials(parts, 2, rays * 256).view(rays, 256)
 
 
 def thin_colsum(x, S):
@@ -95,15 +115,19 @@ def thin_colsum(x, S):
     return out
 
 
-def thin_dw(thin, images, slot, n_slots, S):
+def thin_dw(thin, images, slot, n_slots, S, split=False):
     """[M,256] = thin^T x for a thin fp32 operand [S,M] (M in 1,3,5) and an image slot x."""
     M = thin.shape[1]
     max_blocks = 148 * 4 + 8
-    partial = torch.empty(max_blocks * M * 256, device=thin.device)
-    nb = ctypes.c_int(0)
-    _C.call("tp_tc_thin_dw", ops._p(thin), M, ops._p(images), slot, n_slots, S, ops._p(partial), partial.numel(),
-            ctypes.byref(nb), ops._stream())
-    return reduce_partials(partial, nb.value, M * 256).view(M, 256)
+    parts = 2 if split else 1
+    partial = torch.empty(parts * max_blocks * M * 256, device=thin.device)
+    used = 0
+    for i in range(parts):
+        nb = ctypes.c_int(0)
+        _C.call("tp_tc_thin_dw", ops._p(thin), M, ops._p(images), parts * slot + i, parts * n_slots, S,
+                ops._p(partial[used * M * 256:]), partial.numel() - used * M * 256, ctypes.byref(nb), ops._stream())
+        used += nb.value
+    return reduce_partials(partial, used, M * 256).view(M, 256)
 
 
 def fused_supported(S, per_image) -> bool:
@@ -149,13 +173,15 @@ def heads_backward(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_un
     return pairs[:4], pairs[4:], d_lt, d_ll
 
 
-def heads_backward_staged(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans, need_lat_light):
+def heads_backward_staged(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_density, g_uncert, need_lat_trans, need_lat_light,
+                          split=False):
     """The two heads' backward for ANY head depth (256-wide layers), on the staged kernels: the activations are the tile images /
     ReLU bitmasks the single-pass staged forward saved (slots: feature, rgb hidden 1.., transient hidden 1.., encoding tile), the
     dX chains are two tp_tc_chain_backward launches (one per head: its output layer's dz enters as the thin operand), the
     256 x 256 weight gradients one tp_tc_dw_gemm launch, the thin pieces the helpers above.  Used when tp_tc_heads_backward's
     fixed stage table (the yaml's 3 x 256 heads) does not describe the architecture, or when its images are too small for it
-    (fused_supported is false)."""
+    (fused_supported is false).  split: the fp32-parity step -- the images are the bf16 hi / lo pairs of the split-save forward,
+    the chains tp_tc_chain_backward_split launches over K = 16 hi | lo weight slots."""
     from . import mlp_tc32  # noqa: F401  (save layout)
     dev = sv.rgb.device
     geom = sv.geom
@@ -167,13 +193,15 @@ def heads_backward_staged(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_densit
     slot_r = lambda i: i                  # rgb hidden activation h_i (output of rgb layer i-1), i = 1 .. nr-1
     slot_t = lambda i: (nr - 1) + i       # transient hidden activation, i = 1 .. nt-1
     lib = _C.load()
+    parts = 2 if split else 1             # tile images per slot (split: hi, lo)
+    k = 16 if split else 32               # K rows of W per packed chunk
     dz_rgb, dz_trans = torch.empty(S, 3, device=dev), torch.empty(S, 5, device=dev)
     _C.call("tp_stl_output_grad", ops._p(sv.rgb), ops._p(sv.density), ops._p(sv.uncert), ops._p(g_rgb), ops._p(g_density),
             ops._p(g_uncert), S, ops._p(dz_rgb), ops._p(dz_trans), None, ops._stream())
     n_tiles = (S + 127) // 128
     n_dz = (nr - 1) + (nt - 1)            # dz of every hidden layer's pre-activation: rgb nr-2 .. 0, then transient nt-2 .. 0
-    dz = torch.empty(n_tiles * n_dz * 65536, dtype=torch.uint8, device=dev)
-    bits = images[n_tiles * n_save * 65536:]
+    dz = torch.empty(n_tiles * parts * n_dz * 65536, dtype=torch.uint8, device=dev)
+    bits = images[n_tiles * parts * n_save * 65536:]
     rows = []
 
     def chain(layers, thin, slot_h, dz0):
@@ -185,44 +213,47 @@ def heads_backward_staged(cfg, sv, S, per_image, rgb_p, trans_p, g_rgb, g_densit
         for j, li in enumerate(range(n - 2, 0, -1)):
             c0 = len(rows)
             W = layers[li][0]
-            for c in range(0, 256, 32):
-                rows.append([W.data_ptr(), W.stride(0), 0, 256, c, 32, 256, 0, -1, 1])
-            stages.append([-1, 0, c0, 8, slot_h(li), dz0 + 1 + j])
+            for c in range(0, 256, k):
+                rows.append([W.data_ptr(), W.stride(0), 0, 256, c, k, 256, 0, -1, 1])
+            stages.append([-1, 0, c0, 256 // k, slot_h(li), dz0 + 1 + j])
         return thin, stages
 
     jobs = [chain(rgb_p, dz_rgb, slot_r, 0), chain(trans_p, dz_trans, slot_t, nr - 1)]
     desc = ops.device_table(rows, torch.int64, dev)
     packed = torch.empty(len(rows) * lib.tp_tc_chunk_bytes(), dtype=torch.uint8, device=dev)
-    _C.call("tp_tc_pack_weights", ops._p(desc), len(rows), ops._p(packed), ops._stream())
+    _C.call("tp_tc_pack_weights_split" if split else "tp_tc_pack_weights", ops._p(desc), len(rows), ops._p(packed), ops._stream())
     for thin, stages in jobs:
         st = torch.tensor(stages, dtype=torch.int32)
-        _C.call("tp_tc_chain_backward", ops._p(thin), thin.shape[1], None, 0, S, ops._p(packed), len(rows), ops._p(st), len(stages),
-                ops._p(bits), n_save, ops._p(dz), n_dz, ops._stream())
+        _C.call("tp_tc_chain_backward_split" if split else "tp_tc_chain_backward", ops._p(thin), thin.shape[1], None, 0, S,
+                ops._p(packed), len(rows), ops._p(st), len(stages), ops._p(bits), n_save, ops._p(dz), n_dz, ops._stream())
     # dz slot of layer li's pre-activation (li = 0 .. n-2)
     dzr = lambda li: (nr - 2) - li
     dzt = lambda li: (nr - 1) + (nt - 2) - li
     pairs = [(dzr(li), slot_r(li) if li else slot_feat) for li in range(nr - 2, -1, -1)] + \
             [(dzt(li), slot_t(li) if li else slot_feat) for li in range(nt - 2, -1, -1)]
-    big = torch.cat([dw_gemm(dz, n_dz, images, n_save, pairs[i:i + 12], S) for i in range(0, len(pairs), 12)], dim=0)
+    if split:
+        big = dw_gemm(dz, n_dz, images, n_save, pairs, S, split=True)
+    else:
+        big = torch.cat([dw_gemm(dz, n_dz, images, n_save, pairs[i:i + 12], S) for i in range(0, len(pairs), 12)], dim=0)
     big_r = {li: big[j] for j, li in enumerate(range(nr - 2, -1, -1))}
     big_t = {li: big[(nr - 1) + j] for j, li in enumerate(range(nt - 2, -1, -1))}
-    sums = images_colsum(dz, n_dz, S, list(range(n_dz)))                                   # bias gradients of every hidden layer
+    sums = images_colsum(dz, n_dz, S, list(range(n_dz)), split=split)                     # bias gradients of every hidden layer
     grads_r, grads_t = [None] * nr, [None] * nt
-    grads_r[nr - 1] = (thin_dw(dz_rgb, images, slot_r(nr - 1), n_save, S), thin_colsum(dz_rgb, S))
-    grads_t[nt - 1] = (thin_dw(dz_trans, images, slot_t(nt - 1), n_save, S), thin_colsum(dz_trans, S))
+    grads_r[nr - 1] = (thin_dw(dz_rgb, images, slot_r(nr - 1), n_save, S, split=split), thin_colsum(dz_rgb, S))
+    grads_t[nt - 1] = (thin_dw(dz_trans, images, slot_t(nt - 1), n_save, S, split=split), thin_colsum(dz_trans, S))
     for li in range(1, nr - 1):
         grads_r[li] = (big_r[li], sums[dzr(li)])
     for li in range(1, nt - 1):
         grads_t[li] = (big_t[li], sums[dzt(li)])
     # ---- layer 0 of each head: feature columns from the GEMM, per-ray view / per-sample xyz / per-image latent columns
     W_r0, W_t0 = rgb_p[0][0], trans_p[0][0]
-    g_ray = image_ray_sums(dz, dzr(0), n_dz, S, N)                                         # [B*R,256]
+    g_ray = image_ray_sums(dz, dzr(0), n_dz, S, N, split=split)                            # [B*R,256]
     g_img = ops.group_colsum(g_ray, B * R, R)                                              # [B,256]
-    g_timg = ops.group_colsum(image_ray_sums(dz, dzt(0), n_dz, S, N), B * R, R)
+    g_timg = ops.group_colsum(image_ray_sums(dz, dzt(0), n_dz, S, N, split=split), B * R, R)
     view_t, _, vc = geom["view_seg"]()
     dW_view, _ = ops.linear_backward_weight(g_ray, [(view_t, 1, vc)], B * R, want_bias=False)
     xyz = ops.points_from_depth(geom["center"], geom["ray"], geom["depth"]).view(S, 3)
-    dW_xyz = thin_dw(xyz, dz, dzr(0), n_dz, S).t().contiguous()
+    dW_xyz = thin_dw(xyz, dz, dzr(0), n_dz, S, split=split).t().contiguous()
     dW_light, _ = ops.linear_backward_weight(g_img, [(ll, 1, cfg.n_latent_light)], B, want_bias=False)
     grads_r[0] = (torch.cat([big_r[0], dW_view, dW_xyz, dW_light], dim=1), sums[dzr(0)])
     d_ll = ops.linear_backward_input(g_img, W_r0, B, cfg.n_latent_light, None, w_col0=256 + vc + 3) if need_lat_light else None

@@ -6,6 +6,11 @@ hidden layer -> trunk feature -> trunk layers, with the raw-density gradient ent
 GEMMs on the tile images (tp_tc_dw_gemm, eight 256 x 256 jobs in one launch) and the thin pieces (bias sums, the 63 encoding
 columns of trunk layers 0 / skip, the view / xyz columns of the rgb head, the output rows) from the existing helpers.
 Tolerance: the bf16 contract (<= 1e-2 on outputs and gradients).
+
+split = True is the same step at the fp32-parity contract (<= 1e-4; opt.b200.mlp = 'fp32' with opt.b200.fp32_engine = 'tc'): the
+split-fp16 forward (three passes) saves the activations as bf16 hi + lo image pairs (tp_tc32_forward_split_save), the dX chain
+carries dz and the weights as bf16 hi + lo with three passes per K = 16 step (tp_tc_chain_backward_split), and every image helper
+runs on the hi and lo images and adds the parts (mlp_tc_bwd, split flag).
 """
 from __future__ import annotations
 
@@ -70,7 +75,7 @@ class _Holder:
     """Cache slot for the packed images of one forward / backward pair (the padded tensors are rebuilt per call)."""
 
 
-def forward_train(cfg, geom, feat_p, rgb_p):
+def forward_train(cfg, geom, feat_p, rgb_p, split=False):
     """-> rgb [S,3], density [S], ctx for `backward`."""
     dev = geom["depth"].device
     B, R, N = geom["shape"]
@@ -80,25 +85,28 @@ def forward_train(cfg, geom, feat_p, rgb_p):
     stl = _stl_config(cfg, holder, len(feat_p))
     none = none1.expand(B, 0)
     rgb2, den2, _, (images, n_save) = mlp_tc32.forward(stl, geom, none, none, feat_p, rgb_pad, trans_dummy, static_only=True,
-                                                       precision=1, save=True)
+                                                       precision=0 if split else 1, save=True)
     rgb, density = rgb2[:, :, 0].contiguous(), den2[:, 0].contiguous()
-    ctx = dict(images=images, n_save=n_save, rgb=rgb, density=density, geom=geom, rgb_pad=rgb_pad, cfg=cfg)
+    ctx = dict(images=images, n_save=n_save, rgb=rgb, density=density, geom=geom, rgb_pad=rgb_pad, cfg=cfg, split=split)
     return rgb, density, ctx
 
 
-def _bwd_chunks(cfg, feat_p, rgb_pad):
-    """Transposed weight chunks of the chain, in stage order; returns (desc rows, chain stage rows)."""
+def _bwd_chunks(cfg, feat_p, rgb_pad, split=False):
+    """Transposed weight chunks of the chain, in stage order; returns (desc rows, chain stage rows).  split: the chunks of
+    tp_tc_pack_weights_split, one K = 16 step (hi | lo) each, sixteen per layer."""
     nf = len(feat_p)
     rows, stages = [], []
+    k = 16 if split else 32             # K rows of W per chunk
+    per_layer = _F // k
 
     def thin_chunk(W, n_rows):          # K = 16 step: chunk element (n, kl) = W[kl][n], kl < n_rows
         rows.append([W.data_ptr(), W.stride(0), 0, _F, 0, n_rows, 256, 0, -1, 1])
         return len(rows) - 1
 
-    def big(W, row0=0):                 # eight K = 32 chunks: element (n, kl) = W[row0 + 32 c + kl][n], n < 256
+    def big(W, row0=0):                 # K = 32 (16) chunks: element (n, kl) = W[row0 + k c + kl][n], n < 256
         c0 = len(rows)
-        for c in range(0, _F, 32):
-            rows.append([W.data_ptr(), W.stride(0), 0, _F, row0 + c, 32, 256, 0, -1, 1])
+        for c in range(0, _F, k):
+            rows.append([W.data_ptr(), W.stride(0), 0, _F, row0 + c, k, 256, 0, -1, 1])
         return c0
 
     slot_h = lambda li: li              # saved slot of trunk activation h_li (output of trunk layer li), li < nf - 1
@@ -107,67 +115,71 @@ def _bwd_chunks(cfg, feat_p, rgb_pad):
     # stage 0: dz_rgb (thin 0) x W_out -> masked by the rgb hidden activation -> dz slot 0
     stages.append([0, thin_chunk(W_out, 3), 0, 0, slot_rgb_h, 0])
     # stage 1: x W_r0[:, :256] -> masked by the trunk feature -> dz slot 1 (gradient of the feature rows of the last trunk layer)
-    stages.append([-1, 0, big(W_r0), 8, slot_feat, 1])
+    stages.append([-1, 0, big(W_r0), per_layer, slot_feat, 1])
     # stage 2: x W_last[1:] + dz_sigma (thin 1) x W_last[0] -> masked by h_{nf-2} -> dz slot 2; then down the trunk
     W_last = feat_p[nf - 1][0]
     tc = thin_chunk(W_last, 1)
-    stages.append([1, tc, big(W_last, row0=1), 8, slot_h(nf - 2), 2])
+    stages.append([1, tc, big(W_last, row0=1), per_layer, slot_h(nf - 2), 2])
     for li in range(nf - 2, 0, -1):     # layer li maps h_{li-1} -> h_li: dz_{li-1} = (dz_li W_li[:, :256]) * [h_{li-1} > 0]
-        stages.append([-1, 0, big(feat_p[li][0]), 8, slot_h(li - 1), 2 + (nf - 1 - li)])
+        stages.append([-1, 0, big(feat_p[li][0]), per_layer, slot_h(li - 1), 2 + (nf - 1 - li)])
     return rows, stages
 
 
 def backward(ctx, g_rgb, g_density, feat_p, rgb_p):
     """-> ([(dW, db)] per trunk layer, [(dW, db)] per rgb layer)."""
     cfg, geom, images, n_save = ctx["cfg"], ctx["geom"], ctx["images"], ctx["n_save"]
-    rgb_pad = ctx["rgb_pad"]
+    rgb_pad, split = ctx["rgb_pad"], ctx["split"]
     B, R, N = geom["shape"]
     S = geom["S"]
     dev = images.device
     nf = len(feat_p)
     lib = _C.load()
+    parts = 2 if split else 1           # tile images per slot (split: hi, lo)
     dz_rgb, dz_sigma = torch.empty(S, 3, device=dev), torch.empty(S, 1, device=dev)
     _C.call("tp_plain_output_grad", ops._p(ctx["rgb"]), ops._p(ctx["density"]), ops._p(ops._f32(g_rgb).reshape(S, 3)),
             ops._p(ops._f32(g_density).reshape(S)), S, ops._p(dz_rgb), ops._p(dz_sigma), ops._stream())
-    rows, stages = _bwd_chunks(cfg, feat_p, rgb_pad)
+    rows, stages = _bwd_chunks(cfg, feat_p, rgb_pad, split)
     desc = ops.device_table(rows, torch.int64, dev)
     packed = torch.empty(len(rows) * lib.tp_tc_chunk_bytes(), dtype=torch.uint8, device=dev)
-    _C.call("tp_tc_pack_weights", ops._p(desc), len(rows), ops._p(packed), ops._stream())
+    _C.call("tp_tc_pack_weights_split" if split else "tp_tc_pack_weights", ops._p(desc), len(rows), ops._p(packed), ops._stream())
     n_dz = len(stages)
     n_tiles = (S + 127) // 128
-    dz = torch.empty(n_tiles * n_dz * 65536, dtype=torch.uint8, device=dev)
+    dz = torch.empty(n_tiles * parts * n_dz * 65536, dtype=torch.uint8, device=dev)
     st = torch.tensor(stages, dtype=torch.int32)
-    bits = images[n_tiles * n_save * 65536:]          # the ReLU bitmasks the forward wrote behind the tile images
-    _C.call("tp_tc_chain_backward", ops._p(dz_rgb), 3, ops._p(dz_sigma), 1, S, ops._p(packed), len(rows), ops._p(st), n_dz,
-            ops._p(bits), n_save, ops._p(dz), n_dz, ops._stream())
+    bits = images[n_tiles * parts * n_save * 65536:]          # the ReLU bitmasks the forward wrote behind the tile images
+    _C.call("tp_tc_chain_backward_split" if split else "tp_tc_chain_backward", ops._p(dz_rgb), 3, ops._p(dz_sigma), 1, S,
+            ops._p(packed), len(rows), ops._p(st), n_dz, ops._p(bits), n_save, ops._p(dz), n_dz, ops._stream())
     # ---- 256 x 256 weight gradients: (dz slot, saved activation slot) per layer; the layers that read the encoding (layer 0, skip
     # layers) add a job against the saved encoding tile, whose column 63 is a constant 1: dz^T of it = [dW encoding columns | db]
     slot_feat, slot_rgb_h, slot_enc = nf - 1, nf, n_save - 1
     dz_slot = lambda li: 2 + (nf - 2 - li) if li < nf - 1 else 1      # dz of trunk layer li's pre-activation (the last layer: its feature rows)
     enc_layers = [0] + sorted(set(cfg.skip))
     pairs = [(0, slot_feat), (1, nf - 2)] + [(dz_slot(li), li - 1) for li in range(nf - 2, 0, -1)] + [(dz_slot(li), slot_enc) for li in enc_layers]
-    big = torch.cat([mlp_tc_bwd.dw_gemm(dz, n_dz, images, n_save, pairs[i:i + 12], S) for i in range(0, len(pairs), 12)], dim=0)      # one launch for <= 12 jobs
+    if split:
+        big = mlp_tc_bwd.dw_gemm(dz, n_dz, images, n_save, pairs, S, split=True)
+    else:
+        big = torch.cat([mlp_tc_bwd.dw_gemm(dz, n_dz, images, n_save, pairs[i:i + 12], S) for i in range(0, len(pairs), 12)], dim=0)      # one launch for <= 12 jobs
     enc_grad = {li: big[nf + j] for j, li in enumerate(enc_layers)}       # [256, 256]: columns 0..62 encoding, 63 bias sum
     # ---- column sums of the dz images whose bias gradient does not come out of an encoding job
     want = [0, 1] + [dz_slot(li) for li in range(nf - 2, 0, -1) if li not in enc_grad]
-    sums = mlp_tc_bwd.images_colsum(dz, n_dz, S, want)
+    sums = mlp_tc_bwd.images_colsum(dz, n_dz, S, want, split=split)
     colsum = lambda slot: sums[want.index(slot)]
     # ---- thin pieces
     h = rgb_p[0][0].shape[0]
-    dW_out = mlp_tc_bwd.thin_dw(dz_rgb, images, slot_rgb_h, n_save, S)[:, :h].contiguous()
+    dW_out = mlp_tc_bwd.thin_dw(dz_rgb, images, slot_rgb_h, n_save, S, split=split)[:, :h].contiguous()
     db_out = mlp_tc_bwd.thin_colsum(dz_rgb, S)
-    ray_sums0 = mlp_tc_bwd.image_ray_sums(dz, 0, n_dz, S, N)                                   # [B*R,256] of the rgb hidden dz
+    ray_sums0 = mlp_tc_bwd.image_ray_sums(dz, 0, n_dz, S, N, split=split)                    # [B*R,256] of the rgb hidden dz
     view_t, _, vc = geom["view_seg"]()
     dW_view, _ = ops.linear_backward_weight(ray_sums0, [(view_t, 1, vc)], B * R, want_bias=False)          # [256, vc]
     xyz = ops.points_from_depth(geom["center"], geom["ray"], geom["depth"]).view(S, 3)
-    dW_xyz = mlp_tc_bwd.thin_dw(xyz, dz, 0, n_dz, S).t()                                                   # [256, 3]
+    dW_xyz = mlp_tc_bwd.thin_dw(xyz, dz, 0, n_dz, S, split=split).t()                                     # [256, 3]
     dW_r0 = torch.cat([big[0], dW_view, dW_xyz], dim=1)[:h].contiguous()
     db_r0 = colsum(0)[:h].contiguous()
     g_rgb_layers = [(dW_r0, db_r0), (dW_out, db_out)]
     # ---- trunk
     ec = cfg.enc_cols
     g_feat = [None] * nf
-    dW_sigma = mlp_tc_bwd.thin_dw(dz_sigma, images, nf - 2, n_save, S)                          # [1,256]: row 0 of the last layer
+    dW_sigma = mlp_tc_bwd.thin_dw(dz_sigma, images, nf - 2, n_save, S, split=split)            # [1,256]: row 0 of the last layer
     g_feat[nf - 1] = (torch.cat([dW_sigma, big[1]], dim=0), torch.cat([mlp_tc_bwd.thin_colsum(dz_sigma, S), colsum(1)]))
     for j, li in enumerate(range(nf - 2, 0, -1)):
         if li in enc_grad:
@@ -179,13 +191,14 @@ def backward(ctx, g_rgb, g_density, feat_p, rgb_p):
 
 
 class PlainTC(torch.autograd.Function):
-    """(geom, *trunk and head parameters) -> (rgb [B,R,N,3], density [B,R,N]) with the tensor-core backward."""
+    """(geom, split, *trunk and head parameters) -> (rgb [B,R,N,3], density [B,R,N]) with the tensor-core backward; split = the
+    fp32-parity step (<= 1e-4), else bf16 (<= 1e-2)."""
 
     @staticmethod
-    def forward(ctx, cfg, geom, n_feat, *params):
+    def forward(ctx, cfg, geom, n_feat, split, *params):
         pairs = [(params[i].detach().float().contiguous(), params[i + 1].detach().float().contiguous()) for i in range(0, len(params), 2)]
         feat_p, rgb_p = pairs[:n_feat], pairs[n_feat:]
-        rgb, density, saved = forward_train(cfg, geom, feat_p, rgb_p)
+        rgb, density, saved = forward_train(cfg, geom, feat_p, rgb_p, split)
         ctx.saved, ctx.layers = saved, (feat_p, rgb_p)
         B, R, N = geom["shape"]
         return rgb.view(B, R, N, 3), density.view(B, R, N)
@@ -202,5 +215,5 @@ class PlainTC(torch.autograd.Function):
         out = []
         for dW, db in g_feat + g_rgb_layers:
             out += [dW, db]
-        need = ctx.needs_input_grad[3:]
-        return (None, None, None, *[o if need[i] else None for i, o in enumerate(out)])
+        need = ctx.needs_input_grad[4:]
+        return (None, None, None, None, *[o if need[i] else None for i, o in enumerate(out)])
