@@ -270,6 +270,29 @@ int tp_tc32_forward(const float* center, const float* ray, const float* depth, i
  * address hi and lo as ordinary slots.  bf16 rather than the forward's fp16: the backward's operands need fp32's exponent range.
  * Same stage list, checks, scratch and status word as tp_tc32_forward. */
 int64_t tp_tc32_split_save_bytes(int64_t S, int n_save);
+/* Graph.render after ray selection as ONE launch of the staged kernel, for inference, in either arithmetic (precision 0 split
+ * <= 1e-4, 1 single-pass bf16) and for any stage list tp_tc32_forward takes: what tp_raygen + tp_sample_depth + tp_tc_ray_bias +
+ * tp_tc32_forward + tp_composite_{plain,stl}_forward compute (pre-training engine, model/nerf_pretrain.py:588-627 with the plain
+ * layers/nerf.py model; adaptation engine, model/nerf_adapt_st_gan.py:565-631), with no per-sample tensor and no bias table in HBM.
+ *   kinv, pose_inv, B, H, W, pix_offset, ray_idx / R / ray0, z_near / z_far, N in {32, 64, 128}, depth_mode / rand / seed and
+ *   min_uncert as for tp_render_fused_forward (rays and depths have the bits of tp_raygen and tp_sample_depth);
+ *   image, n_slots, stages, n_stages, bias, precision as for tp_tc32_forward (no save slot is written); a BIAS_RAY stage's row is
+ *   imgbias_rgb[view] + wview^T [u, enc(u)] computed in-kernel with tp_tc_ray_bias's bits: wview [3+6*L_view,256] = the view-encoding
+ *   columns of the rgb-0 layer, transposed; imgbias_rgb [B,256] and imgbias [B,256] (BIAS_IMAGE stages; may be NULL without one)
+ *   from tp_tc_image_biases or the layer-0 biases of the two heads.
+ *   chains 3 (static / transient / light, layers/nerf_static_transient_light.py:168-212): outputs as tp_render_fused_forward's,
+ *   density [B*R*N,2]; chains 1 (plain model, single-chain compositing of layers/nerf.py:117-136, no background colour): rgb [B*R,3],
+ *   depth and opacity [B*R], density [B*R*N] -- the other outputs must be NULL.  Any output may be NULL and may address a peer
+ *   GPU's memory.  scratch >= tp_tc32_render_scratch_bytes(); the fp16-range status word is tp_tc32_forward's (same offset). */
+int64_t tp_tc32_render_scratch_bytes(void);
+int tp_tc32_render_forward(const float* kinv, const float* pose_inv, int B, int H, int W, float pix_offset, const int64_t* ray_idx,
+                           int64_t R, int64_t ray0, const float* z_near, const float* z_far, int N, int depth_mode,
+                           const float* rand, uint64_t seed, const void* image, int n_slots, const int32_t* stages, int n_stages,
+                           const float* bias, const float* wview, int L_view, const float* imgbias_rgb, const float* imgbias,
+                           int chains, float min_uncert, float* rgb, float* rgb_static, float* rgb_transient, float* depth,
+                           float* opacity, float* opacity_static, float* opacity_transient, float* uncert,
+                           float* alpha_static, float* alpha_transient, float* density, void* scratch,
+                           int64_t scratch_bytes, int precision, void* stream);
 int tp_tc32_forward_split_save(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
                                const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
                                const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,

@@ -23,9 +23,17 @@
 //   * the stage list is DATA (tp_tc32_forward's `stages`): trunk depth, skip positions and head depths come from the caller's
 //     architecture, not from a table compiled into the kernel.
 //
-// SMEM: A_hi 64K | A_lo 64K | E_hi 16K | E_lo 16K | ring 4 x 16K | barriers = 229 632 B.  TMEM: 512 columns.
+// Render launch (tp_tc32_render_forward, either arithmetic): the tile's rows make their own samples from the pixel index (rays,
+// bounds, jitter, depths: the bits of tp_raygen + tp_sample_depth), the rgb-0 stage's per-ray bias row is computed by the warps
+// that read it (tp_tc_ray_bias's bits, in a per-warp slot of the L2-resident scratch), and the last stage's samples are
+// composited in the epilogue (row = sample: warp scan + cross-warp carry) -- no per-sample tensor and no bias table in HBM.
+//
+// SMEM: A_hi 64K | A_lo 64K | E_hi 16K | E_lo 16K | ring 4 x 16K | barriers = 229 632 B (+ 512 B compositing scratch in the
+// render launch).  TMEM: 512 columns.
+#include <type_traits>
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
+#include "rays.cuh"
 #include "../../include/texpose_b200.h"
 
 namespace tcs {
@@ -82,6 +90,33 @@ struct Params {
   Stage st[kMaxStages];
 };
 
+// The render launch's parameters: the staged kernel's, minus the per-sample inputs / outputs (center, ray, depth, raybias, rgb,
+// density, uncert stay unused), plus what a row needs to make its sample and what the compositing writes.
+constexpr uint32_t kOffComp = kSmemBytes;                 // [4 warps][3] scan totals, then [4 warps][14] per-ray partial sums
+constexpr uint32_t kSmemRender = kOffComp + 512;
+static_assert(kSmemRender <= 232448, "227 KB of shared memory per CTA");
+constexpr int kViewRowFloats = 128;                       // per drain warp: its column half of the ray's rgb-0 bias row
+struct RenderParams : Params {
+  const float* kinv;         // [B,9]
+  const float* pinv;         // [B,12]
+  int H, W;
+  float pix_offset;
+  const long long* ray_idx;  // [B,R] pixel indices, or NULL: ray r of every view is pixel ray0 + r
+  long long R, ray0;
+  const float* z_near;       // [B,H*W]
+  const float* z_far;
+  int depth_mode;            // 0 injected rand [B*R*N], 1 midpoints, 2 Philox (tp_sample_depth's stream)
+  const float* rand;
+  unsigned long long seed;
+  const float* wview;        // [3+6L,256]: the view-encoding columns of the rgb-0 layer, transposed
+  int L_view;
+  const float* imgbias_rgb;  // [B,256]
+  int chains;                // 1: plain model (per-sample density is [S]); 3: static / transient / light ([S,2])
+  float min_uncert;
+  float *o_rgb, *o_rgb_s, *o_rgb_t, *o_depth, *o_op, *o_op_s, *o_op_t, *o_unc, *o_as, *o_at, *o_density;
+  long long vrow_off;        // byte offset in scratch of the view-bias rows: [CTA][8 drain warps][128] floats
+};
+
 // hi / lo fp16 words of two fp32 values (x0 in the low half): hi = fp16(x), lo = fp16(x - hi) -> x to ~22 mantissa bits
 __device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
   uint32_t d;
@@ -105,15 +140,275 @@ __device__ __forceinline__ void umma3(uint32_t d, uint32_t ah, uint32_t al, uint
   umma_bf16_lohi(d, al, a_hi, bh, b_hi, idesc, 1u);
 }
 
+// ------------------------------------------------------------------------------------------ render pieces
+// One row's sample: ray from the pixel index (camera.py:292-314, unproject = tp_raygen's arithmetic), depth from the ray's bounds
+// (model/nerf_adapt_st_gan.py:682-700, tp_sample_depth's arithmetic and Philox stream), the interval to the next sample of the
+// ray and the point.  Rows past the last ray take the last ray (a tile holds whole rays: they are never composited into output).
+struct RenderSample {
+  long long ray;
+  int k;
+  bool live;
+  float d, dist, xyz[3];
+};
+
+__device__ __forceinline__ long long render_ray(const RenderParams& p, long long tile, int row, bool& live) {
+  const long long n_rays = p.S / p.N, ray_raw = tile * (128 / p.N) + row / p.N;
+  live = ray_raw < n_rays;
+  return live ? ray_raw : n_rays - 1;
+}
+__device__ __forceinline__ void render_unproject(const RenderParams& p, long long ray, long long& b, long long& pix, float c[3],
+                                                 float dir[3]) {
+  b = ray / p.R;
+  pix = p.ray_idx ? p.ray_idx[ray] : p.ray0 + (ray - b * p.R);
+  unproject(p.kinv + b * 9, p.pinv + b * 12, __fadd_rn((float)(pix % p.W), p.pix_offset), __fadd_rn((float)(pix / p.W), p.pix_offset),
+            c, dir);
+}
+
+// jitter of this lane's sample and of the next sample of its ray.  A warp holds 32 consecutive samples of one ray = 8 Philox
+// quads (counter = sample / 4): lanes 0..8 evaluate quads 0..8 once (quad 8: the next warp's first sample), shuffles hand out.
+__device__ __forceinline__ void render_jitter_pair(const RenderParams& p, long long s, int lane, bool has_next, float& u0, float& u1) {
+  if (p.depth_mode == 1) {
+    u0 = u1 = 0.5f;
+    return;
+  }
+  if (p.depth_mode == 0) {
+    u0 = p.rand[s];
+    u1 = __shfl_down_sync(0xffffffffu, u0, 1);
+    if (lane == 31 && has_next) u1 = p.rand[s + 1];
+    return;
+  }
+  const long long qd = ((s - lane) >> 2) + lane;      // (s - lane): the warp's first sample, a multiple of 32
+  const uint4 x = tp_philox((uint32_t)qd, (uint32_t)(qd >> 32), (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
+  const int src = lane >> 2, e = lane & 3;
+  const float c0 = __shfl_sync(0xffffffffu, tp_u01(x.x), src), c1 = __shfl_sync(0xffffffffu, tp_u01(x.y), src),
+              c2 = __shfl_sync(0xffffffffu, tp_u01(x.z), src), c3 = __shfl_sync(0xffffffffu, tp_u01(x.w), src);
+  u0 = e == 0 ? c0 : e == 1 ? c1 : e == 2 ? c2 : c3;
+  const float nq = __shfl_sync(0xffffffffu, tp_u01(x.x), 8);
+  u1 = __shfl_down_sync(0xffffffffu, u0, 1);
+  if (lane == 31) u1 = nq;
+}
+
+__device__ __noinline__ RenderSample render_sample(const RenderParams& p, long long tile, int row, int lane) {
+  RenderSample o;
+  const int N = p.N;                                       // 32, 64 or 128: divides 128
+  o.k = row & (N - 1);
+  o.ray = render_ray(p, tile, row, o.live);
+  long long b, pix;
+  float c[3], dir[3];
+  render_unproject(p, o.ray, b, pix, c, dir);
+  const long long zi = b * (long long)p.H * p.W + pix;
+  const float lo = p.z_near[zi], hi = p.z_far[zi];
+  float u0, u1;
+  render_jitter_pair(p, o.ray * N + o.k, lane, o.k + 1 < N, u0, u1);
+  // stratified_depth with N = 2^m: (u + k) / N is an exact scaling, so the multiplication gives the division's bits
+  const float inv_n = 1.f / (float)N;
+  o.d = __fadd_rn(__fmul_rn(__fmul_rn(__fadd_rn(u0, (float)o.k), inv_n), __fsub_rn(hi, lo)), lo);
+  const float dn = __fadd_rn(__fmul_rn(__fmul_rn(__fadd_rn(u1, (float)(o.k + 1)), inv_n), __fsub_rn(hi, lo)), lo);
+  const float len = sqrtf(dir[0] * dir[0] + dir[1] * dir[1] + dir[2] * dir[2]);      // composite.cu's |ray|
+  o.dist = __fmul_rn(o.k + 1 < N ? __fsub_rn(dn, o.d) : 1e10f, len);
+#pragma unroll
+  for (int j = 0; j < 3; ++j) o.xyz[j] = __fadd_rn(c[j], __fmul_rn(dir[j], o.d));      // camera.py:317-322
+  return o;
+}
+
+// The E tile row of the sample: the same fp32 encoding as the per-sample launch's encode_tile (no save slot).
+template <bool kSingle>
+__device__ __noinline__ void render_encode(const RenderParams& p, long long tile, int row, int lane, uint32_t sbase) {
+  const RenderSample rs = render_sample(p, tile, row, lane);
+  float v[64];
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    const float x = rs.xyz[j];
+    v[j] = x;
+#pragma unroll
+    for (int k = 0; k < kEncL; ++k) {
+      float sn, cs;
+      sincosf(__fmul_rn(x, ldexpf(3.14159265358979323846f, k)), &sn, &cs);
+      v[3 + j * 2 * kEncL + k] = sn;
+      v[3 + j * 2 * kEncL + kEncL + k] = cs;
+    }
+  }
+  v[63] = 0.f;
+#pragma unroll
+  for (int k8 = 0; k8 < 8; ++k8) {
+    uint32_t h[4], l[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      if (kSingle) h[e] = pack_bf16(v[k8 * 8 + 2 * e], v[k8 * 8 + 2 * e + 1]);
+      else split2(v[k8 * 8 + 2 * e], v[k8 * 8 + 2 * e + 1], h[e], l[e]);
+    }
+    st_shared_v4(sbase + kOffEhi + k8 * 2048 + row * 16, h[0], h[1], h[2], h[3]);
+    if (!kSingle) st_shared_v4(sbase + kOffElo + k8 * 2048 + row * 16, l[0], l[1], l[2], l[3]);
+  }
+}
+
+// Columns [half * 128, half * 128 + 128) of the rgb-0 bias row of the warp's ray (all 32 rows of a warp share it): imgbias_rgb[view]
+// + W_view [u, enc(u)], u = ray / |ray| (layers/nerf_static_transient_light.py:104-117), with tp_tc_ray_bias's operation order --
+// one fma chain per column, inputs ascending -- so the row has the table's bits.  Lane j holds input j, lane l computes columns
+// 4l .. 4l + 3 of the half; the row goes to the warp's slot `dst`, which the drain of this stage reads back.
+__device__ __noinline__ void render_view_row(const RenderParams& p, long long tile, int row, int lane, int half, float* dst) {
+  bool live;
+  const long long ray = render_ray(p, tile, row, live);
+  long long b, pix;
+  float c[3], dir[3];
+  render_unproject(p, ray, b, pix, c, dir);
+  const float len = unit_length(dir[0], dir[1], dir[2]);
+  const int L = p.L_view, vc = 3 + 6 * L;
+  float e = 0.f;
+  if (lane < vc) {
+    const int jj = lane - 3, cc = lane < 3 ? lane : jj / (2 * L);
+    const float uc = __fdiv_rn(cc == 0 ? dir[0] : cc == 1 ? dir[1] : dir[2], len);
+    e = uc;
+    if (lane >= 3) {
+      const int rem = jj - cc * 2 * L, k = rem < L ? rem : rem - L;
+      const float arg = __fmul_rn(uc, ldexpf(3.14159265358979323846f, k));
+      e = rem < L ? sinf(arg) : cosf(arg);
+    }
+  }
+  const int col = half * 128 + lane * 4;
+  float4 acc = __ldg(reinterpret_cast<const float4*>(p.imgbias_rgb + b * 256 + col));
+  // inputs nine at a time: the nine weight loads of a batch are independent (one L2 round trip per batch, not per input)
+#pragma unroll 1
+  for (int j0 = 0; j0 < vc; j0 += 9) {
+    float4 w[9];
+#pragma unroll
+    for (int i = 0; i < 9; ++i)
+      if (j0 + i < vc) w[i] = __ldg(reinterpret_cast<const float4*>(p.wview + (j0 + i) * 256 + col));
+#pragma unroll
+    for (int i = 0; i < 9; ++i) {
+      const float ej = __shfl_sync(0xffffffffu, e, (j0 + i) & 31);
+      if (j0 + i < vc) {
+        acc.x = fmaf(w[i].x, ej, acc.x);
+        acc.y = fmaf(w[i].y, ej, acc.y);
+        acc.z = fmaf(w[i].z, ej, acc.z);
+        acc.w = fmaf(w[i].w, ej, acc.w);
+      }
+    }
+  }
+  *reinterpret_cast<float4*>(dst + lane * 4) = acc;
+}
+
+__device__ __forceinline__ float warp_scan(float v, int lane) {      // inclusive
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const float n = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v += n;
+  }
+  return v;
+}
+
+// Compositing of the tile's rays by the four column-half-0 warps (rows = samples; N / 32 warps per ray), arithmetic of
+// tp_composite_stl_forward (layers/nerf_static_transient_light.py:168-212, SURVEY appendix C): three exclusive cumulative sums
+// (warp scan + the totals of the ray's earlier warps, exchanged through `sc`), 14 per-ray sums (warp reduction + the same
+// exchange).  The plain model (layers/nerf.py:117-136) is the same arithmetic with a zero transient head: sig_t = 0 makes the
+// joint and static chains equal, rgb = sum c w, depth = sum d w, opacity = sum w with w = T (1 - exp(-sigma dist)) -- the weights
+// of tp_composite_plain_forward.
+__device__ __noinline__ void render_composite(const RenderParams& p, float* sc, int q, int lane, long long ray, int k, float d,
+                                              float dist, bool live, float sig_s, float sig_t, float cs0, float cs1, float cs2,
+                                              float ct0, float ct1, float ct2, float u) {
+  const float cs[3] = {cs0, cs1, cs2}, ct[3] = {ct0, ct1, ct2};
+  float* tot = sc;             // [4 warps][3]
+  float* red = sc + 12;        // [4 warps][14]
+  const float sd_s = __fmul_rn(sig_s, dist), sd_t = __fmul_rn(sig_t, dist), sd = __fadd_rn(sd_s, sd_t);
+  const float in_j = warp_scan(sd, lane), in_s = warp_scan(sd_s, lane), in_t = warp_scan(sd_t, lane);
+  if (lane == 31) {
+    tot[q * 3] = in_j;
+    tot[q * 3 + 1] = in_s;
+    tot[q * 3 + 2] = in_t;
+  }
+  const float pj = __shfl_up_sync(0xffffffffu, in_j, 1), ps_ = __shfl_up_sync(0xffffffffu, in_s, 1),
+              pt_ = __shfl_up_sync(0xffffffffu, in_t, 1);
+  named_bar_sync(1, 128);
+  const int wpr = p.N >> 5, q0 = q & ~(wpr - 1);      // warps per ray (1, 2, 4), first warp of this ray
+  float ex_j = lane ? pj : 0.f, ex_s = lane ? ps_ : 0.f, ex_t = lane ? pt_ : 0.f;
+  {
+    float cj = 0.f, c_s = 0.f, c_t = 0.f;
+    for (int w = q0; w < q; ++w) {
+      cj += tot[w * 3];
+      c_s += tot[w * 3 + 1];
+      c_t += tot[w * 3 + 2];
+    }
+    ex_j += cj;
+    ex_s += c_s;
+    ex_t += c_t;
+  }
+  const float Es = expf(-sd_s), Et = expf(-sd_t), E = expf(-sd);
+  const float T = expf(-ex_j), Ts = expf(-ex_s), Tt = expf(-ex_t);
+  const float as = 1.f - Es, at = 1.f - Et, a = 1.f - E;
+  const float w_ps = T * as, w_pt = T * at, w_p = T * a, w_qs = Ts * as, w_qt = Tt * at;
+  float v16[16];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    v16[c] = cs[c] * w_ps + ct[c] * w_pt;
+    v16[3 + c] = w_qs * cs[c];
+    v16[6 + c] = w_qt * ct[c];
+  }
+  v16[9] = d * w_qs;
+  v16[10] = w_p;
+  v16[11] = w_qs;
+  v16[12] = w_qt;
+  v16[13] = u * w_pt;
+  v16[14] = v16[15] = 0.f;
+  // warp totals of the 16 values by recursive halving (8 + 4 + 2 + 1 + 1 shuffles): a lane keeps one half and adds the partner's
+  float v8[8], v4[4], v2[2];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const bool up = (lane & 16) != 0;
+    v8[i] = (up ? v16[i + 8] : v16[i]) + __shfl_xor_sync(0xffffffffu, up ? v16[i] : v16[i + 8], 16);
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const bool up = (lane & 8) != 0;
+    v4[i] = (up ? v8[i + 4] : v8[i]) + __shfl_xor_sync(0xffffffffu, up ? v8[i] : v8[i + 4], 8);
+  }
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    const bool up = (lane & 4) != 0;
+    v2[i] = (up ? v4[i + 2] : v4[i]) + __shfl_xor_sync(0xffffffffu, up ? v4[i] : v4[i + 2], 4);
+  }
+  const bool up2 = (lane & 2) != 0;
+  float v1 = (up2 ? v2[1] : v2[0]) + __shfl_xor_sync(0xffffffffu, up2 ? v2[0] : v2[1], 2);
+  v1 += __shfl_xor_sync(0xffffffffu, v1, 1);
+  const int vidx = ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1);
+  if ((lane & 1) == 0 && vidx < 14) red[q * 14 + vidx] = v1;
+  if (live) {
+    const long long s = ray * p.N + k;
+    if (p.o_as) __stcs(p.o_as + s, as);
+    if (p.o_at) __stcs(p.o_at + s, at);
+    if (p.o_density) {
+      if (p.chains == 1) __stcs(p.o_density + s, sig_s);
+      else __stcs(reinterpret_cast<float2*>(p.o_density) + s, make_float2(sig_s, sig_t));
+    }
+  }
+  named_bar_sync(1, 128);
+  if (q == q0 && lane < 14 && live) {
+    float v = 0.f;
+    for (int w = q0; w < q0 + wpr; ++w) v += red[w * 14 + lane];
+    float* dst = lane < 3 ? (p.o_rgb ? p.o_rgb + ray * 3 + lane : nullptr)
+               : lane < 6 ? (p.o_rgb_s ? p.o_rgb_s + ray * 3 + lane - 3 : nullptr)
+               : lane < 9 ? (p.o_rgb_t ? p.o_rgb_t + ray * 3 + lane - 6 : nullptr)
+               : lane == 9 ? (p.o_depth ? p.o_depth + ray : nullptr)
+               : lane == 10 ? (p.o_op ? p.o_op + ray : nullptr)
+               : lane == 11 ? (p.o_op_s ? p.o_op_s + ray : nullptr)
+               : lane == 12 ? (p.o_op_t ? p.o_op_t + ray : nullptr)
+                            : (p.o_unc ? p.o_unc + ray : nullptr);
+    if (lane == 13) v += p.min_uncert;
+    if (dst) *dst = v;
+  }
+}
+
 // kSingle = false: the fp32-parity mode (fp16 hi + lo, three passes).  kSingle = true: ONE pass with bf16 operands -- the general-
 // architecture bf16 forward (any stage list; <= 1e-2 like mlp_tc.cu, which stays the fast path for the yaml's architecture), whose
 // drain can also keep every hidden activation as a bf16 tile image for the tensor-core backward (training of layers/nerf.py).
 // kSplitSave (with kSingle = false): the parity-mode arithmetic unchanged, and the drain also keeps every save-slot activation and
 // the encoding tile as bf16 hi + lo tile images (slots 2k, 2k + 1) plus the ReLU bitmasks: the operands of the split backward.
-template <bool kSingle, bool kSplitSave>
-__device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
+// P = RenderParams: the render launch (samples made in-kernel, per-ray outputs; no save).
+template <bool kSingle, bool kSplitSave, class P = Params>
+__device__ __forceinline__ void nerf_forward_split_body(const P& p) {
   static_assert(!(kSingle && kSplitSave), "the split save belongs to the three-pass arithmetic");
-  constexpr bool kSave = kSingle || kSplitSave;      // the launch can write tile images
+  constexpr bool kRender = std::is_same<P, RenderParams>::value;
+  static_assert(!(kRender && kSplitSave), "the render launch keeps no activations");
+  constexpr bool kSave = (kSingle || kSplitSave) && !kRender;      // the launch can write tile images
   constexpr int kImgPerSlot = kSplitSave ? 2 : 1;     // tile images per save slot (hi, lo)
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
@@ -270,6 +565,13 @@ __device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
     // takes sin / cos of the ROUNDED product -- its own encoding differs from the exact one by up to 6e-5 at k = 9, so the
     // parity mode must round where it rounds), split into E_hi / E_lo.  Done by the column-half-1 warps (row = sample).
     auto encode_tile = [&](long long tile) {
+      if constexpr (kRender) {
+        render_encode<kSingle>(p, tile, row, lane, sbase);
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(bar_enc);
+        return;
+      }
       const long long s_raw = tile * 128 + row, s = s_raw < p.S ? s_raw : p.S - 1, r = s / p.N;
       const float d = p.depth[s];
       float v[64];
@@ -321,6 +623,8 @@ __device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
       if (lane == 0) mbar_arrive(bar_enc);
     };
     if (half == 1 && (long long)blockIdx.x < n_tiles) encode_tile(blockIdx.x);
+    float* vrow = nullptr;      // render launch: this warp's slot for its half of the rgb-0 bias row
+    if constexpr (kRender) vrow = reinterpret_cast<float*>(p.scratch + p.vrow_off) + ((size_t)blockIdx.x * 8 + warp) * kViewRowFloats;
 
     for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
       const long long s_raw = tile * 128 + row;
@@ -329,6 +633,12 @@ __device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
       float sigma_s = 0.f, rgb_s[3] = {0.f, 0.f, 0.f}, rgb_t[3] = {0.f, 0.f, 0.f}, sigma_t = 0.f, unc = 0.f;
       for (int L = 0; L < n_stages; ++L) {
         const Stage sg = p.st[L];
+        if constexpr (kRender) {
+          if (sg.bias_kind == BIAS_RAY) {      // while the stage's MMAs run: the warp's half of its ray's bias row
+            render_view_row(p, tile, row, lane, half, vrow);
+            __syncwarp();
+          }
+        }
         mbar_wait(bar_acc(L & 1), (acc_ph >> (L & 1)) & 1u);
         acc_ph ^= 1u << (L & 1);
         tc_fence_after();
@@ -343,7 +653,8 @@ __device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
           }
         }
         if (sg.kind == KIND_HIDDEN) {
-          const float* brow = (sg.bias_kind == BIAS_STATIC ? p.bias + sg.bias_off
+          const float* brow = kRender && sg.bias_kind == BIAS_RAY ? vrow
+                            : (sg.bias_kind == BIAS_STATIC ? p.bias + sg.bias_off
                                : sg.bias_kind == BIAS_RAY  ? p.raybias + (s / p.N) * 256
                                                            : p.imgbias + (s / p.per_image) * 256) + half * 128;
           const uint32_t tmem_d = tmem_row + (uint32_t)(L & 1) * 256 + half * 128;
@@ -357,7 +668,10 @@ __device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
           // wait out their full latency behind the stores of the previous group (16 exposed load-use stalls per stage, ncu source page)
           auto load_bias = [&](float4 (&bq)[8], int j) {
 #pragma unroll
-            for (int i = 0; i < 8; ++i) bq[i] = __ldg(reinterpret_cast<const float4*>(brow + j * 32 + i * 4));
+            for (int i = 0; i < 8; ++i) {
+              const float4* a = reinterpret_cast<const float4*>(brow + j * 32 + i * 4);
+              bq[i] = kRender ? __ldcg(a) : __ldg(a);      // (the render launch's bias row was written by this kernel)
+            }
           };
           auto slab = [&](const uint32_t (&v)[32], const float4 (&bq)[8], int j) {
             uint32_t positive = 0u;
@@ -452,7 +766,13 @@ __device__ __forceinline__ void nerf_forward_split_body(const Params& p) {
         }
       }
       if (!kSingle && !(act_max <= 6.0e4f)) atomicOr(p.status, 1u);      // (also catches NaN)
-      if (half == 0 && live) {
+      if constexpr (kRender) {
+        if (half == 0) {
+          const RenderSample rs = render_sample(p, tile, row, lane);
+          render_composite(p, reinterpret_cast<float*>(smem + kOffComp), q, lane, rs.ray, rs.k, rs.d, rs.dist, rs.live, sigma_s,
+                           sigma_t, rgb_s[0], rgb_s[1], rgb_s[2], rgb_t[0], rgb_t[1], rgb_t[2], unc);
+        }
+      } else if (half == 0 && live) {
 #pragma unroll
         for (int c = 0; c < 3; ++c) *reinterpret_cast<float2*>(p.rgb + s * 6 + c * 2) = make_float2(rgb_s[c], rgb_t[c]);
         *reinterpret_cast<float2*>(p.density + s * 2) = make_float2(sigma_s, sigma_t);
@@ -476,6 +796,12 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_kernel(const P
 // the parity-mode forward of a training step: tile images and ReLU bitmasks in the split backward's format
 __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_save_kernel(const Params p) {
   nerf_forward_split_body<false, true>(p);
+}
+
+// the render launch in either arithmetic
+template <bool kSingle>
+__global__ void __launch_bounds__(kThreads, 1) nerf_render_split_kernel(const __grid_constant__ RenderParams p) {
+  nerf_forward_split_body<kSingle, false, RenderParams>(p);
 }
 
 // slot_desc row: [W ptr, ld, row0, rows_valid, col0, cols_valid, kind (256 | 16), unused]
@@ -538,19 +864,10 @@ TP_API int64_t tp_tc32_split_save_bytes(int64_t S, int n_save) {
   return ((S + 127) / 128) * (int64_t)n_save * (2 * tc::kABytes + 4096);
 }
 
-// shared by tp_tc32_forward and tp_tc32_forward_split_save: the argument and stage-list checks, then the launch
-static int tc32_forward_launch(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
-                               const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
-                               const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert,
-                               void* scratch, int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot,
-                               bool split_save, void* stream) {
-  if (enc_slot < -1 || (enc_slot >= 0 && (!save || enc_slot >= n_save))) return TP_ERR_BAD_ARG;
-  if (((uintptr_t)image & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)bias & 15) || ((uintptr_t)raybias & 15) ||
-      ((uintptr_t)imgbias & 15) || ((uintptr_t)rgb & 7) || ((uintptr_t)density & 7))
-    return TP_ERR_ALIGN;
-  if (!tp_device_is_sm100()) return TP_ERR_ARCH;
-  tcs::Params p = {};
-  // validate the stage list: it is the caller's architecture, and a malformed list would dead-lock the barrier protocol
+// The stage list into p.st: it is the caller's architecture, and a malformed list would dead-lock the barrier protocol.
+// has_raybias / has_imgbias: the launch has the per-ray / per-image bias rows that BIAS_RAY / BIAS_IMAGE stages read.
+static int tc32_parse_stages(tcs::Params& p, const int32_t* stages, int n_stages, int n_slots, bool has_raybias, bool has_imgbias,
+                             const void* save, int n_save, int enc_slot) {
   int slots = 0, pending_ready = 0, n_e_last = 0;
   bool parked = false;
   for (int L = 0; L < n_stages; ++L) {
@@ -570,8 +887,8 @@ static int tc32_forward_launch(const float* center, const float* ray, const floa
     if (wait) pending_ready = 0;
     if (reload && (!parked || L == 0 || p.st[L - 1].kind == tcs::KIND_HIDDEN || pending_ready)) return TP_ERR_BAD_ARG;
     if (sg.a_steps && !wait && !reload && (L == 0 || p.st[L - 1].kind == tcs::KIND_HIDDEN)) return TP_ERR_BAD_ARG;   // A would be stale
-    if (sg.bias_kind == tcs::BIAS_RAY && !raybias) return TP_ERR_BAD_ARG;
-    if (sg.bias_kind == tcs::BIAS_IMAGE && !imgbias) return TP_ERR_BAD_ARG;
+    if (sg.bias_kind == tcs::BIAS_RAY && !has_raybias) return TP_ERR_BAD_ARG;
+    if (sg.bias_kind == tcs::BIAS_IMAGE && !has_imgbias) return TP_ERR_BAD_ARG;
     if (hidden) {
       if (pending_ready) return TP_ERR_BAD_ARG;                          // the previous drain's arrivals were never consumed
       pending_ready = 1;
@@ -587,6 +904,24 @@ static int tc32_forward_launch(const float* center, const float* ray, const floa
   }
   if (n_e_last != 1 || pending_ready || p.st[0].e_steps == 0 || p.st[n_stages - 1].kind == tcs::KIND_HIDDEN) return TP_ERR_BAD_ARG;
   if (slots != n_slots) return TP_ERR_BAD_SHAPE;
+  p.n_stages = n_stages;
+  return TP_OK;
+}
+
+// shared by tp_tc32_forward and tp_tc32_forward_split_save: the argument and stage-list checks, then the launch
+static int tc32_forward_launch(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
+                               const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
+                               const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert,
+                               void* scratch, int64_t scratch_bytes, int precision, void* save, int n_save, int enc_slot,
+                               bool split_save, void* stream) {
+  if (enc_slot < -1 || (enc_slot >= 0 && (!save || enc_slot >= n_save))) return TP_ERR_BAD_ARG;
+  if (((uintptr_t)image & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)bias & 15) || ((uintptr_t)raybias & 15) ||
+      ((uintptr_t)imgbias & 15) || ((uintptr_t)rgb & 7) || ((uintptr_t)density & 7))
+    return TP_ERR_ALIGN;
+  if (!tp_device_is_sm100()) return TP_ERR_ARCH;
+  tcs::Params p = {};
+  const int err = tc32_parse_stages(p, stages, n_stages, n_slots, raybias != nullptr, imgbias != nullptr, save, n_save, enc_slot);
+  if (err != TP_OK) return err;
   if (S == 0) return TP_OK;
   const long long n_tiles = (S + 127) / 128;
   int grid = tp_num_sms();
@@ -596,7 +931,6 @@ static int tc32_forward_launch(const float* center, const float* ray, const floa
   p.image = reinterpret_cast<const uint8_t*>(image); p.bias = bias; p.raybias = raybias; p.imgbias = imgbias;
   p.rgb = rgb; p.density = density; p.uncert = uncert; p.scratch = reinterpret_cast<uint8_t*>(scratch);
   p.status = reinterpret_cast<unsigned int*>(p.scratch + tp_tc32_status_offset());
-  p.n_stages = n_stages;
   p.save = reinterpret_cast<uint8_t*>(save); p.n_save = n_save; p.enc_slot = save ? enc_slot : -1;
   const size_t images_per_slot = split_save ? 2 : 1;
   p.save_bits = save ? reinterpret_cast<uint32_t*>(p.save + (size_t)((S + 127) / 128) * n_save * images_per_slot * tc::kABytes) : nullptr;
@@ -629,4 +963,60 @@ TP_API int tp_tc32_forward_split_save(const float* center, const float* ray, con
   if ((uintptr_t)save & 15) return TP_ERR_ALIGN;
   return tc32_forward_launch(center, ray, depth, S, N, per_image, image, n_slots, stages, n_stages, bias, raybias, imgbias, rgb,
                              density, uncert, scratch, scratch_bytes, 0, save, n_save, enc_slot, true, stream);
+}
+
+/* scratch of the render launch: tp_tc32_forward's (parked features, status word), then 256 B, then the view-bias rows */
+TP_API int64_t tp_tc32_render_scratch_bytes(void) {
+  return tp_tc32_status_offset() + 256 + (int64_t)tp_num_sms() * 8 * tcs::kViewRowFloats * 4;
+}
+
+TP_API int tp_tc32_render_forward(const float* kinv, const float* pose_inv, int B, int H, int W, float pix_offset,
+                                  const int64_t* ray_idx, int64_t R, int64_t ray0, const float* z_near, const float* z_far, int N,
+                                  int depth_mode, const float* rand, uint64_t seed, const void* image, int n_slots,
+                                  const int32_t* stages, int n_stages, const float* bias, const float* wview, int L_view,
+                                  const float* imgbias_rgb, const float* imgbias, int chains, float min_uncert, float* rgb,
+                                  float* rgb_static, float* rgb_transient, float* depth, float* opacity, float* opacity_static,
+                                  float* opacity_transient, float* uncert, float* alpha_static, float* alpha_transient,
+                                  float* density, void* scratch, int64_t scratch_bytes, int precision, void* stream) {
+  if (!kinv || !pose_inv || !z_near || !z_far || !image || !stages || !bias || !wview || !imgbias_rgb || !scratch)
+    return TP_ERR_BAD_ARG;
+  if (B < 1 || H < 1 || W < 1 || R < 0 || L_view < 0 || L_view > 4 || n_stages < 1 || n_stages > tcs::kMaxStages)
+    return TP_ERR_BAD_SHAPE;
+  if (N != 32 && N != 64 && N != 128) return TP_ERR_BAD_SHAPE;      // a 128-row tile holds whole rays
+  if (!ray_idx && (ray0 < 0 || ray0 + R > (int64_t)H * W)) return TP_ERR_BAD_SHAPE;
+  if (depth_mode < 0 || depth_mode > 2 || (depth_mode == 0 && !rand)) return TP_ERR_BAD_ARG;
+  if ((precision != 0 && precision != 1) || (chains != 1 && chains != 3)) return TP_ERR_BAD_ARG;
+  if (chains == 1 && (rgb_static || rgb_transient || opacity_static || opacity_transient || uncert || alpha_static || alpha_transient))
+    return TP_ERR_BAD_ARG;      // the plain model has one chain: rgb, depth, opacity and the per-sample density
+  if (((uintptr_t)image & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)bias & 15) || ((uintptr_t)wview & 15) ||
+      ((uintptr_t)imgbias_rgb & 15) || ((uintptr_t)imgbias & 15) || ((uintptr_t)density & (chains == 1 ? 3 : 7)))
+    return TP_ERR_ALIGN;
+  if (!tp_device_is_sm100()) return TP_ERR_ARCH;
+  tcs::RenderParams p = {};
+  const int err = tc32_parse_stages(p, stages, n_stages, n_slots, true, imgbias != nullptr, nullptr, 0, -1);
+  if (err != TP_OK) return err;
+  const int64_t S = (int64_t)B * R * N;
+  if (S == 0) return TP_OK;
+  if (scratch_bytes < tp_tc32_render_scratch_bytes()) return TP_ERR_WORKSPACE;
+  const long long n_tiles = (S + 127) / 128;
+  int grid = tp_num_sms();
+  if (n_tiles < grid) grid = (int)n_tiles;
+  p.S = S; p.N = N; p.per_image = R * N;
+  p.image = reinterpret_cast<const uint8_t*>(image); p.bias = bias; p.imgbias = imgbias;
+  p.scratch = reinterpret_cast<uint8_t*>(scratch);
+  p.status = reinterpret_cast<unsigned int*>(p.scratch + tp_tc32_status_offset());
+  p.enc_slot = -1;
+  p.kinv = kinv; p.pinv = pose_inv; p.H = H; p.W = W; p.pix_offset = pix_offset;
+  p.ray_idx = reinterpret_cast<const long long*>(ray_idx); p.R = R; p.ray0 = ray0;
+  p.z_near = z_near; p.z_far = z_far; p.depth_mode = depth_mode; p.rand = rand; p.seed = seed;
+  p.wview = wview; p.L_view = L_view; p.imgbias_rgb = imgbias_rgb; p.chains = chains; p.min_uncert = min_uncert;
+  p.o_rgb = rgb; p.o_rgb_s = rgb_static; p.o_rgb_t = rgb_transient; p.o_depth = depth; p.o_op = opacity;
+  p.o_op_s = opacity_static; p.o_op_t = opacity_transient; p.o_unc = uncert; p.o_as = alpha_static; p.o_at = alpha_transient;
+  p.o_density = density;
+  p.vrow_off = tp_tc32_status_offset() + 256;
+  void (*kern)(const tcs::RenderParams) = precision ? tcs::nerf_render_split_kernel<true> : tcs::nerf_render_split_kernel<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcs::kSmemRender);
+  if (e != cudaSuccess) return (int)e;
+  kern<<<grid, tcs::kThreads, tcs::kSmemRender, (cudaStream_t)stream>>>(p);
+  return tp_launch_status();
 }

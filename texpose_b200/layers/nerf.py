@@ -159,6 +159,10 @@ class NeRF(torch.nn.Module):
             return False
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             return False
+        return self._staged_architecture(opt)
+
+    def _staged_architecture(self, opt) -> bool:
+        """The layer shapes the staged kernel (mlp_tc32) takes for this model."""
         if not (opt.nerf.view_dep and opt.arch.posenc and opt.arch.posenc.L_3D == 10 and 0 <= (opt.arch.posenc.L_view or 0) <= 4):
             return False
         nf, skip = len(self.mlp_feat), set(opt.arch.skip)
@@ -204,6 +208,49 @@ class NeRF(torch.nn.Module):
         none = torch.zeros(B, 0, device=dev)
         rgb, density, _ = mlp_tc32.forward(stl, geom, none, none, feat_p, rgb_p, trans_p, static_only=True)
         return rgb.view(B, R, N, 3, 2)[..., 0].contiguous(), density.view(B, R, N, 2)[..., 0].contiguous()
+
+    # ------------------------------------------------------------------ one-launch rendering (staged kernel, render mode)
+    def render_precision(self, opt) -> int:
+        """Arithmetic of render_rays: 0 = split hi + lo (<= 1e-4) for opt.b200.mlp 'fp32' and for 'auto' where the bf16 kernel does
+        not implement the architecture (what forward_samples computes then); 1 = single-pass bf16 (<= 1e-2) otherwise.  Raises
+        NotImplementedError when the staged launch cannot render this model under `opt`."""
+        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            raise NotImplementedError("render_rays is inference: call it under torch.no_grad()")
+        if opt.nerf.get("setbg_opaque"):
+            raise NotImplementedError("render_rays composites without a background colour (opt.nerf.setbg_opaque)")
+        if opt.camera.ndc:
+            raise NotImplementedError("camera.ndc is false in every reference yaml; not implemented")
+        if opt.nerf.depth.param != "metric":
+            raise NotImplementedError("nerf.depth.param is 'metric' in every reference yaml")
+        from .. import mlp_tc
+        if opt.nerf.sample_intvs not in mlp_tc.FUSED_N:
+            raise NotImplementedError(f"the render launch takes {mlp_tc.FUSED_N} samples per ray, not {opt.nerf.sample_intvs}")
+        prec = _common.mlp_precision(opt)
+        if prec == "fp32" and _common.b200_option(opt, "fp32_engine", "auto") == "simt":
+            raise NotImplementedError("opt.b200.fp32_engine = 'simt' keeps the fp32 mode off the tensor cores")
+        if not self._staged_architecture(opt):
+            raise NotImplementedError("the staged render launch takes 256-wide trunks with L_3D = 10 and rgb heads <= 256 wide")
+        if prec == "auto":
+            return 1 if self.uses_tensor_cores(opt) else 0
+        return 0 if prec == "fp32" else 1
+
+    def render_rays(self, opt, kinv, pinv, ray_idx, ray0, R, z_near, z_far, mode=None, rand=None, seed=0, want=None,
+                    out_ptrs=None):
+        """camera.get_center_and_ray + ray_batch_sample + sample_depth + forward_samples + composite (model/nerf_pretrain.py:588-627)
+        as ONE launch of the staged kernel (tp_tc32_render_forward) in render_precision(opt); returns {rgb [B,R,3], depth
+        [B,R,1], opacity [B,R,1], density [B,R,N]} (the `want` subset; outputs in out_ptrs are written there instead)."""
+        from .. import mlp_tc32
+        precision = self.render_precision(opt)
+        cfg = self._config(opt, mode)
+        feat_p, rgb_p, trans_p = self._tc32_parameters()
+        stl = MLPConfig(L_3D=cfg.L_3D, L_view=cfg.L_view, skip=cfg.skip, view_dep=True, n_feat=len(feat_p), n_rgb=len(rgb_p),
+                        n_trans=2, n_latent_light=0, n_latent_trans=0, precision="fp32" if precision == 0 else "bf16",
+                        save_for_backward=False, packed=self, static_only=True)
+        none = torch.zeros(len(kinv), 0, device=kinv.device)
+        return mlp_tc32.render(stl, kinv, pinv, opt.H, opt.W, ray_idx, ray0, R, ops._f32(z_near), ops._f32(z_far),
+                               opt.nerf.sample_intvs, none, none, feat_p, rgb_p, trans_p, 0.0, rand=rand,
+                               stratified=bool(opt.nerf.sample_stratified), seed=seed, static_only=True, precision=precision,
+                               want=want, out_ptrs=out_ptrs)
 
     @staticmethod
     def composite(opt, ray, rgb_samples, density_samples, depth_samples):

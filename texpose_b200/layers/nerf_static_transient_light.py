@@ -127,16 +127,56 @@ class NeRF(torch.nn.Module):
     def render_rays(self, opt, kinv, pinv, ray_idx, ray0, R, z_near, z_far, latent_variable_trans, latent_variable_light,
                     mode=None, rand=None, seed=0, want=None, out_ptrs=None):
         """get_center_and_ray + ray_batch_sample + sample_depth + forward_samples + composite (model/nerf_adapt_st_gan.py:565-631)
-        in one launch; returns the dict of the eleven outputs of Graph.render."""
+        in one launch; returns the dict of the eleven outputs of Graph.render.  The lock-step bf16 render launch
+        (tp_render_fused_forward) where it implements the precision and architecture; otherwise the staged kernel's render launch
+        (tp_tc32_render_forward, render_precision)."""
         from .. import mlp_tc
         cfg = self._config(opt, mode)
         pairs = lambda ml: [(l.weight.detach(), l.bias.detach()) for l in ml]
         lt = ops._f32(latent_variable_trans.detach())
         ll = ops._f32(latent_variable_light.detach())
+        if not self._lockstep_render_applies(opt, cfg):
+            from .. import mlp_tc32
+            precision = self.render_precision(opt, cfg)
+            return mlp_tc32.render(cfg, kinv, pinv, opt.H, opt.W, ray_idx, ray0, R, ops._f32(z_near), ops._f32(z_far),
+                                   opt.nerf.sample_intvs, lt, ll, pairs(self.mlp_feat), pairs(self.mlp_rgb), pairs(self.mlp_trans),
+                                   float(opt.nerf.min_uncert), rand=rand, stratified=bool(opt.nerf.sample_stratified), seed=seed,
+                                   precision=precision, want=want, out_ptrs=out_ptrs)
         return mlp_tc.render_fused(cfg, kinv, pinv, opt.H, opt.W, ray_idx, ray0, R, ops._f32(z_near), ops._f32(z_far),
                                    opt.nerf.sample_intvs, lt, ll, pairs(self.mlp_feat), pairs(self.mlp_rgb), pairs(self.mlp_trans),
                                    float(opt.nerf.min_uncert), rand=rand, stratified=bool(opt.nerf.sample_stratified), seed=seed,
                                    static_only=cfg.static_only, want=want or mlp_tc.RENDER_KEYS, out_ptrs=out_ptrs)
+
+    def _lockstep_render_applies(self, opt, cfg) -> bool:
+        """render_rays takes tp_render_fused_forward: bf16 / auto precision and the architecture the lock-step kernel implements."""
+        from .. import mlp_tc
+        if cfg.precision == "fp32":
+            return False
+        pairs = lambda ml: [(l.weight, l.bias) for l in ml]
+        return mlp_tc.supported(cfg, pairs(self.mlp_feat), pairs(self.mlp_rgb), pairs(self.mlp_trans))
+
+    def render_precision(self, opt, cfg=None) -> int:
+        """Arithmetic of the staged render launch: 0 = split hi + lo (<= 1e-4) for opt.b200.mlp 'fp32', 1 = single-pass bf16
+        (<= 1e-2) for 'bf16' / 'auto' -- what forward_samples computes for an architecture the lock-step kernel does not implement.
+        Raises NotImplementedError when the staged launch cannot render this model under `opt`."""
+        from .. import mlp_tc, mlp_tc32
+        cfg = cfg or self._config(opt, None)
+        if torch.is_grad_enabled():
+            raise NotImplementedError("render_rays is inference: call it under torch.no_grad()")
+        if opt.camera.ndc:
+            raise NotImplementedError("camera.ndc is false in every reference yaml; not implemented")
+        if opt.nerf.depth.param != "metric":
+            raise NotImplementedError("nerf.depth.param is 'metric' in every reference yaml")
+        if opt.nerf.sample_intvs not in mlp_tc.FUSED_N:
+            raise NotImplementedError(f"the render launch takes {mlp_tc.FUSED_N} samples per ray, not {opt.nerf.sample_intvs}")
+        if cfg.static_only:
+            raise NotImplementedError("static-only rendering (opt.b200.static_only) runs on the lock-step bf16 render launch only")
+        if cfg.precision == "fp32" and not cfg.fp32_tc:
+            raise NotImplementedError("opt.b200.fp32_engine = 'simt' keeps the fp32 mode off the tensor cores")
+        pairs = lambda ml: [(l.weight, l.bias) for l in ml]
+        if not mlp_tc32.supported(cfg, pairs(self.mlp_feat), pairs(self.mlp_rgb), pairs(self.mlp_trans)):
+            raise NotImplementedError("the staged render launch takes 256-wide static/transient/light layer lists with L_3D = 10")
+        return 0 if cfg.precision == "fp32" else 1
 
     @staticmethod
     def composite(opt, ray, rgb_samples, density_samples, depth_samples, uncert_samples=None):

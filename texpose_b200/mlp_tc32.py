@@ -114,7 +114,7 @@ def build_tables(cfg, feat_p, rgb_p, trans_p, static_only=False, save=False):
 
 
 class Packed:
-    __slots__ = ("key", "image", "n_slots", "stages", "bias", "keep", "n_save")
+    __slots__ = ("key", "image", "n_slots", "stages", "bias", "keep", "n_save", "wview")
 
 
 def pack(cfg, holder, feat_p, rgb_p, trans_p, static_only=False, precision=0, save=False) -> Packed:
@@ -136,6 +136,7 @@ def pack(cfg, holder, feat_p, rgb_p, trans_p, static_only=False, precision=0, sa
     out.bias = torch.cat([b.float() for b in biases]).contiguous()
     out.keep = desc
     out.n_save = sum(1 for st in stages if st[6] >= 0) + (1 if save else 0)      # + the encoding tile, in the last slot
+    out.wview = None          # the render launch's view-encoding weight columns (render(), built on first use)
     if holder is not None:
         try:
             setattr(holder, attr, out)
@@ -150,7 +151,9 @@ _scratch = {}
 def _scratch_for(dev):
     k = (dev.type, dev.index)
     if k not in _scratch:
-        _scratch[k] = torch.zeros(_C.load().tp_tc32_scratch_bytes(), dtype=torch.uint8, device=dev)      # (status word starts at 0)
+        lib = _C.load()      # one buffer for both launches: the render launch's is tp_tc32_forward's plus its view-bias rows
+        n = max(lib.tp_tc32_scratch_bytes(), lib.tp_tc32_render_scratch_bytes())
+        _scratch[k] = torch.zeros(n, dtype=torch.uint8, device=dev)      # (status word starts at 0)
     return _scratch[k]
 
 
@@ -211,3 +214,67 @@ def forward(cfg, geom, lat_trans, lat_light, feat_p, rgb_p, trans_p, static_only
     if save:
         return rgb, density, uncert, (images, pk.n_save)
     return rgb, density, uncert
+
+
+RENDER_KEYS = ("rgb", "rgb_static", "rgb_transient", "depth", "opacity", "opacity_static", "opacity_transient", "uncert",
+               "alpha_static", "alpha_transient", "density")
+PLAIN_RENDER_KEYS = ("rgb", "depth", "opacity", "density")      # the plain model (static_only): one compositing chain
+
+
+def render(cfg, kinv, pinv, H, W, ray_idx, ray0, R, z_near, z_far, N, lat_trans, lat_light, feat_p, rgb_p, trans_p, min_uncert,
+           rand=None, stratified=True, seed=0, static_only=False, precision=0, want=None, out_ptrs=None):
+    """Graph.render after ray selection as ONE launch of the staged kernel (tp_tc32_render_forward): rays, depths, the per-ray
+    bias row and the compositing happen in-kernel.  static_only=True: the plain layers/nerf.py model (its layer list as
+    NeRF._tc32_parameters builds it, one compositing chain, outputs PLAIN_RENDER_KEYS, density [B,R,N]); otherwise the static /
+    transient / light model (the eleven RENDER_KEYS).  precision 0: split hi + lo (<= 1e-4); 1: single-pass bf16 (<= 1e-2).
+    ray_idx / ray0 / R, z_near / z_far, rand / stratified / seed, want and out_ptrs as mlp_tc.render_fused."""
+    import ctypes
+    if N not in mlp_tc.FUSED_N:
+        raise NotImplementedError(f"the staged render launch takes {mlp_tc.FUSED_N} samples per ray")
+    if not supported(cfg, feat_p, rgb_p, trans_p):
+        raise NotImplementedError("staged render launch: 256-wide static/transient/light layer lists with L_3D = 10")
+    keys = PLAIN_RENDER_KEYS if static_only else RENDER_KEYS
+    want = tuple(keys if want is None else want)
+    out_ptrs = out_ptrs or {}
+    bad = [k for k in tuple(want) + tuple(out_ptrs) if k not in keys]
+    if bad:
+        raise ValueError(f"the {'plain' if static_only else 'static/transient/light'} render has no output {bad}")
+    B = kinv.shape[0]
+    dev = kinv.device
+    pk = pack(cfg, cfg.packed, feat_p, rgb_p, trans_p, static_only, precision)
+    if pk.wview is None:
+        pk.wview = rgb_p[0][0][:, _F:_F + cfg.view_cols].t().contiguous()
+    if cfg.n_latent_light or cfg.n_latent_trans:
+        img_r, img_t = mlp_tc.image_biases(cfg, B, lat_trans, lat_light, rgb_p, trans_p)
+    else:      # no latents: the per-image rows are the layer-0 biases (tp_tc_image_biases' bits: the bias, no products)
+        img_r = rgb_p[0][1].float().expand(B, _F).contiguous()
+        img_t = None if static_only else trans_p[0][1].float().expand(B, _F).contiguous()
+    shapes = dict(rgb=(B, R, 3), rgb_static=(B, R, 3), rgb_transient=(B, R, 3), depth=(B, R, 1), opacity=(B, R, 1),
+                  opacity_static=(B, R, 1), opacity_transient=(B, R, 1), uncert=(B, R, 1), alpha_static=(B, R, N),
+                  alpha_transient=(B, R, N), density=(B, R, N) if static_only else (B, R, N, 2))
+    ret = {k: torch.empty(shapes[k], device=dev) for k in want if k not in out_ptrs}
+    if B * R == 0:
+        return ret
+
+    def dst(k):
+        if k in out_ptrs:
+            return ctypes.c_void_p(int(out_ptrs[k]))
+        return ops._p(ret[k]) if k in ret else None
+
+    if rand is not None:
+        mode, rand_t = 0, ops._f32(rand)
+        assert rand_t.numel() == B * R * N
+    elif not stratified:
+        mode, rand_t = 1, None
+    else:
+        mode, rand_t = 2, None
+    if ray_idx is not None:
+        ray_idx = ray_idx.to(torch.int64).contiguous()
+        assert ray_idx.shape == (B, R)
+    scratch = _scratch_for(dev)
+    _C.call("tp_tc32_render_forward", ops._p(ops._f32(kinv)), ops._p(ops._f32(pinv)), B, H, W, 0.5, ops._p(ray_idx), R, int(ray0),
+            ops._p(z_near), ops._p(z_far), N, mode, ops._p(rand_t), int(seed), ops._p(pk.image), pk.n_slots, ops._p(pk.stages),
+            pk.stages.shape[0], ops._p(pk.bias), ops._p(pk.wview), cfg.L_view, ops._p(img_r), ops._p(img_t),
+            1 if static_only else 3, float(min_uncert), *[dst(k) for k in RENDER_KEYS], ops._p(scratch), scratch.numel(),
+            int(precision), ops._stream())
+    return ret

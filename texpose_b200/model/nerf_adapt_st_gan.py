@@ -29,6 +29,8 @@ def rotation_distance(R1, R2, eps=1e-7):
 
 
 class Graph(torch.nn.Module):
+    RENDER_KEYS = ("rgb", "rgb_static", "rgb_transient", "depth", "opacity", "opacity_static", "opacity_transient", "uncert",
+                   "alpha_static", "alpha_transient", "density")      # what _render_fused can produce
 
     def __init__(self, opt, n_train_images=None):
         super().__init__()

@@ -24,6 +24,7 @@ from ..layers.nerf import NeRF
 
 
 class Graph(torch.nn.Module):
+    RENDER_KEYS = ("rgb", "depth", "opacity", "density")      # what _render_fused can produce
 
     def __init__(self, opt):
         super().__init__()
@@ -88,6 +89,30 @@ class Graph(torch.nn.Module):
         rgb_samples, density_samples = self.nerf.forward_samples(opt, center, ray, depth_samples, mode=mode)
         rgb, depth, opacity, _prob = self.nerf.composite(opt, ray, rgb_samples, density_samples, depth_samples)
         return AttrDict(rgb=rgb, depth=depth, opacity=opacity)
+
+    def _render_fused(self, opt, pose, intr, ray_idx, depth_range, sample_idx=None, mode=None, want=None, out_ptrs=None):
+        """render() as ONE launch of the staged kernel (NeRF.render_rays): rays, depths and compositing in-kernel.  Same signature
+        as the adaptation Graph's, so that parallel.FrameGather renders either engine's frame; sample_idx is unused (no latents).
+        ray_idx: [B,R] tensor, or a `range` = contiguous row block.  The view matrices and the jitter draw are render()'s, so a
+        seeded call makes the same rays and depths."""
+        B = len(pose)
+        HW = opt.H * opt.W
+        kinv, pinv = camera.view_matrices(pose, intr, one_launch=camera.one_launch_matrices(opt))
+        zn, zf = depth_range[0].reshape(B, HW), depth_range[1].reshape(B, HW)
+        if isinstance(ray_idx, range):
+            assert ray_idx.step == 1
+            idx_t, ray0, R = None, ray_idx.start, len(ray_idx)
+        else:
+            idx_t, ray0, R = ray_idx, 0, ray_idx.shape[1]
+        rand, seed = None, 0
+        if opt.nerf.sample_stratified:
+            if self._b200(opt, "rng", "torch") == "philox":
+                seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+            else:
+                rand = torch.rand(B, R, opt.nerf.sample_intvs, 1, device=pose.device)      # sample_depth's draw (:707-728)
+        ret = self.nerf.render_rays(opt, kinv, pinv, idx_t, ray0, R, zn, zf, mode=mode, rand=rand, seed=seed, want=want,
+                                    out_ptrs=out_ptrs)
+        return AttrDict(ret)
 
     def _slice_rays(self, opt):
         """Rays per launch: the tensor-core kernels keep activations on chip, the fp32 SIMT path is bounded by its

@@ -245,6 +245,7 @@ class PeerGradExchange(GradBucket):
 
 
 PER_RAY_KEYS = ("rgb", "rgb_static", "rgb_transient", "depth", "opacity", "opacity_static", "opacity_transient", "uncert")
+PRETRAIN_KEYS = ("rgb", "depth", "opacity")      # the per-ray outputs of the pre-training engine (model.nerf_pretrain.Graph)
 _PER_RAY_CHANNELS = dict(rgb=3, rgb_static=3, rgb_transient=3, depth=1, opacity=1, opacity_static=1, opacity_transient=1, uncert=1)
 
 
@@ -268,7 +269,8 @@ def peer_barrier(window_ptrs: Sequence[int], rank: int, epoch: int, device, time
 
 class FrameGather:
     """ONE frame rendered by all ranks of a node (the north-star's 480x640x128 frame at 1/2/4/8 GPUs; the reference is
-    single-GPU, options.py:112).  Rank r renders the row block shard_rays(HW, r, world, align=W) with the fused render launch,
+    single-GPU, options.py:112).  Rank r renders the row block shard_rays(HW, r, world, align=W) with the graph's render launch
+    (`graph._render_fused`: the lock-step or the staged kernel's; keys=PRETRAIN_KEYS for the pre-training engine),
     whose compositing epilogue stores the 56 B/ray outputs STRAIGHT INTO THE ROOT RANK'S FRAME BUFFERS -- a CUDA-IPC window, so
     the stores of ranks != root travel over NVLink as they are produced: the gather is the kernel's own output write, there
     is no collective and no staging copy.  One tiny barrier kernel per frame (tp_peer_barrier) publishes completion.
@@ -313,6 +315,10 @@ class FrameGather:
         {key: [1,HW,C]} on the root (None elsewhere), `local` = the `local_keys` outputs of this rank's rows."""
         if len(pose) != 1:
             raise ValueError("FrameGather renders one view per call")
+        missing = [k for k in tuple(self.keys) + tuple(local_keys) if k not in getattr(graph, "RENDER_KEYS", ())]
+        if missing:
+            raise ValueError(f"{type(graph).__module__}.{type(graph).__name__} does not render {missing} "
+                             f"(it renders {getattr(graph, 'RENDER_KEYS', ())})")
         self.epoch += 1
         par = self.epoch & 1
         b, e = self.rows
