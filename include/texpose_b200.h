@@ -90,6 +90,30 @@ int tp_depth_guided_range(const float* depth, int64_t n, float bg_near, float bg
 int tp_normal_from_depth(const float* kinv, const float* pose_inv, const float* depth, int B, int H, int W,
                          float* normal, void* stream);
 
+/* ---- mask-prior frames (render_by_slices, model/nerf_adapt_st_gan.py:633-680, modes other than 'val') ---------------------- */
+
+/* Object-pixel ray list of B views for the list mode of the render launches (tp_render_fused_forward_list,
+ * tp_tc32_render_forward_list): mask [B,HW] fp32, object pixel = mask > 0 (the reference's test, :655).  list [list_cap] int64
+ * receives, view after view, the entries q = b*HW + pixel of the view's object pixels in ascending order (`nonzero`'s order),
+ * each view's run padded to a multiple of u = 256 / N entries (one super-tile of the lock-step kernel, two tiles of the staged
+ * one: no tile holds rays of two views) with pad entries ~(b*HW) (negative; rendered as pixel 0 of view b, never stored); an
+ * empty view has no entries.  DEVICE outputs: n_slots [1] = the number of entries, counts [B] = object pixels per view.  Nothing
+ * is read back; three launches, no atomics (the order is deterministic).  N in {32, 64, 128};
+ * list_cap >= tp_mask_ray_list_capacity(B, HW, N); workspace >= tp_mask_ray_list_workspace(B, HW) bytes, 8-byte aligned. */
+int64_t tp_mask_ray_list_capacity(int B, int64_t HW, int N);
+int64_t tp_mask_ray_list_workspace(int B, int64_t HW);
+int tp_mask_ray_list(const float* mask, int B, int64_t HW, int N, int64_t* list, int64_t list_cap, int64_t* n_slots,
+                     int64_t* counts, void* workspace, int64_t ws_bytes, void* stream);
+
+/* The defaults of :657-667 at the background pixels (mask <= 0) of pixels [pix0, pix1) of every view: rgb, rgb_static,
+ * rgb_transient [B*HW,3] = 0; depth, opacity, opacity_static, opacity_transient [B*HW] = 0; uncert [B*HW] = min_uncert;
+ * alpha_static, alpha_transient [B*HW*N] = 1; density [B*HW*N,2] = 1 (N a multiple of 4; these three 16-byte aligned).  Object
+ * pixels are never touched.  Any output may be NULL and may address a peer GPU's memory (the frame layout of a FrameGather window). */
+int tp_mask_defaults(const float* mask, int B, int64_t HW, int64_t pix0, int64_t pix1, int N, float min_uncert, float* rgb,
+                     float* rgb_static, float* rgb_transient, float* depth, float* opacity, float* opacity_static,
+                     float* opacity_transient, float* uncert, float* alpha_static, float* alpha_transient, float* density,
+                     void* stream);
+
 /* ---- compositing (K3) ----------------------------------------------------------------------------------- */
 
 /* NeRF.composite, static/transient/joint chains (layers/nerf_static_transient_light.py:168-212).
@@ -229,6 +253,21 @@ int tp_render_fused_forward(const float* kinv, const float* pose_inv, int B, int
                             float* opacity, float* opacity_static, float* opacity_transient, float* uncert,
                             float* alpha_static, float* alpha_transient, float* density, void* scratch,
                             int64_t scratch_bytes, int flags, void* stream);
+/* The same launch over an object-pixel list (tp_mask_ray_list): ray j is slot j of `list` [>= *n_slots], n_slots a DEVICE
+ * pointer read by the kernel (one CTA per SM: the host does not know the count; n_slots = 0 is a valid launch).  Rank shard_rank
+ * of shard_world renders super-tiles [floor(r*T/w), floor((r+1)*T/w)) of the T = n_slots / (256/N) in the list.  A sample's key
+ * is s = q*N + k for entry q: per-ray outputs are stored at row q of [B*HW,C] frame buffers, per-sample ones at s, and
+ * depth_mode 0 reads a frame-sized rand [B*HW*N] at s -- the key a full-frame launch (ray_idx NULL, ray0 0, R = HW) gives the same
+ * sample, for injected rand and Philox alike, so a list-mode sample is bit-identical to that launch's.  Every other argument,
+ * flags bit 17 included, as for tp_render_fused_forward. */
+int tp_render_fused_forward_list(const float* kinv, const float* pose_inv, int B, int H, int W, float pix_offset,
+                                 const int64_t* list, const int64_t* n_slots, int shard_rank, int shard_world,
+                                 const float* z_near, const float* z_far, int N, int depth_mode, const float* rand, uint64_t seed,
+                                 const void* packed, const float* biasbuf, const float* wview, int L_view,
+                                 const float* imgbias_rgb, const float* imgbias_trans, float min_uncert, float* rgb,
+                                 float* rgb_static, float* rgb_transient, float* depth, float* opacity, float* opacity_static,
+                                 float* opacity_transient, float* uncert, float* alpha_static, float* alpha_transient,
+                                 float* density, void* scratch, int64_t scratch_bytes, int flags, void* stream);
 /* ---- fp32-parity mode on the tensor cores (K2 split-bf16, csrc/mlp_tc_split.cu) --------------------------------
  * NeRF.forward_samples (layers/nerf_static_transient_light.py:76-166; layers/nerf.py:61-99 as a padded layer list) with every
  * operand carried as hi + lo bf16 and three tcgen05.mma passes per K step (A_hi W_hi + A_hi W_lo + A_lo W_hi, fp32 accumulate):
@@ -293,6 +332,17 @@ int tp_tc32_render_forward(const float* kinv, const float* pose_inv, int B, int 
                            float* opacity, float* opacity_static, float* opacity_transient, float* uncert,
                            float* alpha_static, float* alpha_transient, float* density, void* scratch,
                            int64_t scratch_bytes, int precision, void* stream);
+/* tp_tc32_render_forward over an object-pixel list: list, n_slots, shard_rank, shard_world, frame-sized rand and the frame layout
+ * of the outputs as tp_render_fused_forward_list (a shard's tiles are twice its super-tiles); n_weight_slots is tp_tc32_forward's
+ * n_slots.  chains must be 3 (static / transient / light); every other argument as for tp_tc32_render_forward. */
+int tp_tc32_render_forward_list(const float* kinv, const float* pose_inv, int B, int H, int W, float pix_offset, const int64_t* list,
+                                const int64_t* n_slots, int shard_rank, int shard_world, const float* z_near, const float* z_far,
+                                int N, int depth_mode, const float* rand, uint64_t seed, const void* image, int n_weight_slots,
+                                const int32_t* stages, int n_stages, const float* bias, const float* wview, int L_view,
+                                const float* imgbias_rgb, const float* imgbias, int chains, float min_uncert, float* rgb,
+                                float* rgb_static, float* rgb_transient, float* depth, float* opacity, float* opacity_static,
+                                float* opacity_transient, float* uncert, float* alpha_static, float* alpha_transient,
+                                float* density, void* scratch, int64_t scratch_bytes, int precision, void* stream);
 int tp_tc32_forward_split_save(const float* center, const float* ray, const float* depth, int64_t S, int N, int64_t per_image,
                                const void* image, int n_slots, const int32_t* stages, int n_stages, const float* bias,
                                const float* raybias, const float* imgbias, float* rgb, float* density, float* uncert, void* scratch,

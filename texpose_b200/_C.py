@@ -16,7 +16,7 @@ ROOT = os.path.dirname(_HERE)
 HEADER = os.path.join(ROOT, "include", "texpose_b200.h")
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("TEXPOSE_B200_LIB") or os.path.join(_HERE, "libtexpose_b200.so")      # override: A/B builds
-SOURCES = ["api.cu", "rays.cu", "composite.cu", "mlp_simt.cu", "mlp_tc.cu", "mlp_tc_split.cu", "mlp_tc_bwd.cu", "mlp_tc_chain.cu", "loss.cu", "peer.cu", "raster.cu"]
+SOURCES = ["api.cu", "rays.cu", "mask.cu", "composite.cu", "mlp_simt.cu", "mlp_tc.cu", "mlp_tc_split.cu", "mlp_tc_bwd.cu", "mlp_tc_chain.cu", "loss.cu", "peer.cu", "raster.cu"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

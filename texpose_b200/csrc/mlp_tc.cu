@@ -112,6 +112,24 @@ __device__ __forceinline__ float stratified_depth_pow2(float u, int k, float inv
   return __fadd_rn(__fmul_rn(__fmul_rn(__fadd_rn(u, (float)k), inv_n), __fsub_rn(hi, lo)), lo);
 }
 
+// pixel b, pix -> ray, bounds, jitter (key s), depth, interval, point of a sample whose k, ray, live and img are set
+__device__ __forceinline__ void render_fetch_at(const Params& p, long long b, long long pix, long long s, int lane, RenderSample& o) {
+  const int N = p.N;
+  float c[3];
+  unproject(p.kinv + b * 9, p.pinv + b * 12, __fadd_rn((float)(pix % p.W), p.pix_offset),
+            __fadd_rn((float)(pix / p.W), p.pix_offset), c, o.dir);
+  const long long zi = b * (long long)p.H * p.W + pix;
+  const float lo = p.z_near[zi], hi = p.z_far[zi];
+  float u0, u1;
+  render_jitter_pair(p, s, lane, o.k + 1 < N, u0, u1);
+  const float inv_n = 1.f / (float)N;                      // N in {32, 64, 128}: exact
+  o.d = stratified_depth_pow2(u0, o.k, inv_n, lo, hi);
+  const float dn = stratified_depth_pow2(u1, o.k + 1, inv_n, lo, hi);
+  const float len = sqrtf(o.dir[0] * o.dir[0] + o.dir[1] * o.dir[1] + o.dir[2] * o.dir[2]);
+  o.dist = __fmul_rn(o.k + 1 < N ? __fsub_rn(dn, o.d) : 1e10f, len);
+#pragma unroll
+  for (int j = 0; j < 3; ++j) o.xyz[j] = __fadd_rn(c[j], __fmul_rn(o.dir[j], o.d));      // camera.py:317-322
+}
 // Everything of a sample but its encoding: pixel -> ray, bounds, jitter, depth, interval, point.  A call, like the other render
 // pieces: the stage loop of the epilogue warps must stay small and spill-free -- local-memory traffic and instruction fetch share
 // the SM's data paths with the MMAs' operand reads, and every build that carried this code inside the loop was slower
@@ -127,21 +145,28 @@ __device__ __noinline__ RenderSample render_fetch(const Params& p, long long til
   const long long b = o.ray / p.R;
   o.img = (int)b;
   const long long pix = p.ray_idx ? p.ray_idx[o.ray] : p.ray0 + (o.ray - b * p.R);
-  float c[3];
-  unproject(p.kinv + b * 9, p.pinv + b * 12, __fadd_rn((float)(pix % p.W), p.pix_offset),
-            __fadd_rn((float)(pix / p.W), p.pix_offset), c, o.dir);
-  const long long zi = b * (long long)p.H * p.W + pix;
-  const float lo = p.z_near[zi], hi = p.z_far[zi];
-  float u0, u1;
-  render_jitter_pair(p, s, lane, o.k + 1 < N, u0, u1);
-  const float inv_n = 1.f / (float)N;                      // N in {32, 64, 128}: exact
-  o.d = stratified_depth_pow2(u0, o.k, inv_n, lo, hi);
-  const float dn = stratified_depth_pow2(u1, o.k + 1, inv_n, lo, hi);
-  const float len = sqrtf(o.dir[0] * o.dir[0] + o.dir[1] * o.dir[1] + o.dir[2] * o.dir[2]);
-  o.dist = __fmul_rn(o.k + 1 < N ? __fsub_rn(dn, o.d) : 1e10f, len);
-#pragma unroll
-  for (int j = 0; j < 3; ++j) o.xyz[j] = __fadd_rn(c[j], __fmul_rn(o.dir[j], o.d));      // camera.py:317-322
+  render_fetch_at(p, b, pix, s, lane, o);
   return o;
+}
+// List mode (kMode 4): ray j of the launch is slot j of the object-pixel list, entry q = view * HW + pixel; a pad entry ~(view * HW)
+// is rendered as pixel 0 of its view and stores nothing.  The sample's key -- its jitter and its output address -- is q * N + k: the
+// key a full-frame launch (ray_idx NULL, ray0 = 0, R = HW) gives the same pixel's sample, so the two render it bit for bit alike.
+__device__ __noinline__ RenderSample render_fetch_list(const Params& p, long long tile, int row, int lane) {
+  RenderSample o;
+  const int N = p.N;
+  o.k = row % N;
+  const long long q = p.list[tile * (128 / N) + row / N], HW = (long long)p.H * p.W;
+  o.live = q >= 0;
+  o.ray = o.live ? q : ~q;      // the frame position the outputs are stored at
+  const long long b = o.ray / HW;
+  o.img = (int)b;
+  render_fetch_at(p, b, o.ray - b * HW, o.ray * N + o.k, lane, o);
+  return o;
+}
+// first (end = 0) / one past the last (end = 1) super-tile of this rank's share of the list: rank r of w takes
+// [floor(r T / w), floor((r + 1) T / w)), T = n_slots / (256 / N)
+__device__ __forceinline__ long long list_shard(const Params& p, int end) {
+  return *p.n_slots / (256 / p.N) * (p.shard_rank + end) / p.shard_world;
 }
 __device__ __noinline__ void render_encode(const float x, const float y, const float z, uint32_t e_smem, int row) {
   const float xyz[3] = {x, y, z};
@@ -326,8 +351,9 @@ __device__ __noinline__ void render_composite(const Params& p, float* sc, int t,
 // Params: a run-time stage count costs 0.3 ms per C2 frame (same-box A/B).
 // kMode: 0 = general (any N: the per-sample launches, with or without the activation save, whose N is not a multiple of 32);
 // 1 = the plain inference launch (per-sample outputs, no activation save); 2 = the plain training launch (activation save + ReLU
-// bitmasks); 3 = the fused render launch (rays, depths, view bias and compositing in-kernel; per-ray outputs).  Modes 1-3 are
-// launched only when N % 32 == 0 and compile the branches of the other launch kinds out.
+// bitmasks); 3 = the fused render launch (rays, depths, view bias and compositing in-kernel; per-ray outputs); 4 = the render launch
+// over an object-pixel list, sharded over the ranks of a frame (render_fetch_list, list_shard).  Modes 1-4 are launched only when
+// N % 32 == 0 and compile the branches of the other launch kinds out.
 // kSmemBias: the launch has one ray per tile (N = 128, hence also one image per tile): the per-ray / per-image bias row of the
 // two table-bias stages sits in shared memory and the drain reads it with broadcast loads instead of warp shuffles.
 template <int kNL = kNumLayers, int kMode = 0, bool kSmemBias = false>
@@ -335,7 +361,7 @@ template <int kNL = kNumLayers, int kMode = 0, bool kSmemBias = false>
 // launch keeps its look-ahead state (next sample's encoding, finished sample) partly in local memory: a few dozen L1-resident
 // STL / LDL per super-tile, cheaper than recomputing it on the critical path)
 __global__ void __launch_bounds__(kThreads, 1) nerf_stl_forward_kernel(const Params p) {
-  constexpr bool kRender = kMode == 3;
+  constexpr bool kRender = kMode >= 3, kList = kMode == 4;
   static_assert(!kSmemBias || kMode != 0, "shared-memory bias rows: launches with N % 32 == 0 only");
   uint8_t* const p_save = (kMode == 1 || kRender) ? nullptr : p.save;
   constexpr int kTileThreads = 128;     // epilogue threads working on one tile
@@ -374,7 +400,8 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_stl_forward_kernel(const Par
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  const long long n_super = (p.S + 255) / 256;
+  // super-tiles of the launch; list mode: of this rank's share, whose first one is super-tile st0 of the list
+  const long long n_super = kList ? list_shard(p, 1) - list_shard(p, 0) : (p.S + 255) / 256;
 
   if (warp == kProducerWarp) {
     // ================================================================ weight producer (converged warp, one lane issues)
@@ -524,7 +551,8 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_stl_forward_kernel(const Par
       const long long s = live ? s_raw : p.S - 1;
       if (!kRender || iter == 0) {     // (the render launch encodes the next super-tile at the end of the last stage, below)
         if (kRender) {
-          rs = render_fetch(p, st * 2 + t, row, lane);
+          if constexpr (kList) rs = render_fetch_list(p, (list_shard(p, 0) + st) * 2 + t, row, lane);
+          else rs = render_fetch(p, st * 2 + t, row, lane);
           render_encode(rs.xyz[0], rs.xyz[1], rs.xyz[2], e_smem, row);
         } else if (kMode == 0 || iter == 0) {
           encode_sample(p, s, e_smem, row);
@@ -572,7 +600,10 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_stl_forward_kernel(const Par
         // (~2 700 cycles), and the trans-0 stage waits for the 64 KB feature reload (~2 100 cycles).  The work that has no place on
         // a tile's critical path goes there: the next super-tile's rays, bounds, jitter and depths (two dependent global
         // loads) into the first, the compositing of the previous super-tile's samples into the second.
-        if (kRender && L == kSpillLayer + 1 && st + gridDim.x < n_super) nxt = render_fetch(p, (st + gridDim.x) * 2 + t, row, lane);
+        if (kRender && L == kSpillLayer + 1 && st + gridDim.x < n_super) {
+          if constexpr (kList) nxt = render_fetch_list(p, (list_shard(p, 0) + st + gridDim.x) * 2 + t, row, lane);
+          else nxt = render_fetch(p, (st + gridDim.x) * 2 + t, row, lane);
+        }
         if (kRender && L == (kNL > kStaticLayers ? kReloadIssueLayer + 1 : kSpillLayer + 1) && have_done) {
           float* sc = reinterpret_cast<float*>(smem + kOffComp) + t * kCompFloats;      // (the park barrier separates two uses)
           render_composite(p, sc, t, q, lane, done_ray, done_k, done_d, done_dist, done_live, done_v[0], done_v[1], done_v[2], done_v[3],
@@ -1009,5 +1040,50 @@ TP_API int tp_render_fused_forward(const float* kinv, const float* pose_inv, int
   void (*kern)(const tc::Params) =
       stat ? (n128 ? tc::nerf_stl_forward_kernel<tc::kStaticLayers, 3, true> : tc::nerf_stl_forward_kernel<tc::kStaticLayers, 3>)
            : (n128 ? tc::nerf_stl_forward_kernel<tc::kNumLayers, 3, true> : tc::nerf_stl_forward_kernel<tc::kNumLayers, 3>);
+  return tc_launch(kern, p, grid, (cudaStream_t)stream);
+}
+
+// The same launch over an object-pixel list (kMode 4): one CTA per SM, since the host does not know the list's length; rank
+// shard_rank of shard_world renders its share of the list's super-tiles.
+TP_API int tp_render_fused_forward_list(const float* kinv, const float* pose_inv, int B, int H, int W, float pix_offset,
+                                        const int64_t* list, const int64_t* n_slots, int shard_rank, int shard_world,
+                                        const float* z_near, const float* z_far, int N, int depth_mode, const float* rand,
+                                        uint64_t seed, const void* packed, const float* biasbuf, const float* wview, int L_view,
+                                        const float* imgbias_rgb, const float* imgbias_trans, float min_uncert, float* rgb,
+                                        float* rgb_static, float* rgb_transient, float* depth, float* opacity,
+                                        float* opacity_static, float* opacity_transient, float* uncert, float* alpha_static,
+                                        float* alpha_transient, float* density, void* scratch, int64_t scratch_bytes, int flags,
+                                        void* stream) {
+  if (!kinv || !pose_inv || !list || !n_slots || !z_near || !z_far || !packed || !biasbuf || !wview || !imgbias_rgb ||
+      !imgbias_trans || !scratch)
+    return TP_ERR_BAD_ARG;
+  if (B < 1 || H < 1 || W < 1 || L_view < 0 || L_view > 4) return TP_ERR_BAD_SHAPE;
+  if (N != 32 && N != 64 && N != 128) return TP_ERR_BAD_SHAPE;
+  if (depth_mode < 0 || depth_mode > 2 || (depth_mode == 0 && !rand)) return TP_ERR_BAD_ARG;      // rand: [B*H*W*N], frame-sized
+  if (shard_world < 1 || shard_rank < 0 || shard_rank >= shard_world) return TP_ERR_BAD_ARG;
+  if (flags & ~(1 << 17)) return TP_ERR_BAD_ARG;
+  if (((uintptr_t)packed & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)wview & 15) || ((uintptr_t)imgbias_rgb & 15) ||
+      ((uintptr_t)imgbias_trans & 15) || ((uintptr_t)density & 7))
+    return TP_ERR_ALIGN;
+  if (!tp_device_is_sm100()) return TP_ERR_ARCH;
+  const int grid = tp_num_sms();
+  if (scratch_bytes < (int64_t)grid * (2 * tc::kABytes + 2 * 4 * 1024)) return TP_ERR_WORKSPACE;
+  tc::Params p = {};
+  p.S = 0; p.N = N; p.per_image = (int64_t)H * W * N;      // (list mode takes its rays and its length from the list)
+  p.list = reinterpret_cast<const long long*>(list); p.n_slots = reinterpret_cast<const long long*>(n_slots);
+  p.shard_rank = shard_rank; p.shard_world = shard_world;
+  p.packed = reinterpret_cast<const uint8_t*>(packed); p.biasbuf = biasbuf; p.imgbias = imgbias_trans;
+  p.density = density; p.scratch = reinterpret_cast<uint8_t*>(scratch);
+  p.prof_offset = tp_tc_prof_offset();
+  p.n_layers = (flags & (1 << 17)) ? tc::kStaticLayers : tc::kNumLayers;
+  p.kinv = kinv; p.pinv = pose_inv; p.H = H; p.W = W; p.pix_offset = pix_offset;
+  p.z_near = z_near; p.z_far = z_far; p.rand = rand; p.depth_mode = depth_mode; p.seed = seed;
+  p.wview = wview; p.L_view = L_view; p.imgbias_rgb = imgbias_rgb; p.min_uncert = min_uncert;
+  p.o_rgb = rgb; p.o_rgb_s = rgb_static; p.o_rgb_t = rgb_transient; p.o_depth = depth; p.o_op = opacity;
+  p.o_op_s = opacity_static; p.o_op_t = opacity_transient; p.o_unc = uncert; p.o_as = alpha_static; p.o_at = alpha_transient;
+  const bool stat = p.n_layers == tc::kStaticLayers, n128 = N == 128;
+  void (*kern)(const tc::Params) =
+      stat ? (n128 ? tc::nerf_stl_forward_kernel<tc::kStaticLayers, 4, true> : tc::nerf_stl_forward_kernel<tc::kStaticLayers, 4>)
+           : (n128 ? tc::nerf_stl_forward_kernel<tc::kNumLayers, 4, true> : tc::nerf_stl_forward_kernel<tc::kNumLayers, 4>);
   return tc_launch(kern, p, grid, (cudaStream_t)stream);
 }

@@ -57,9 +57,20 @@ constexpr uint32_t kMaskBitBytes = 4096;
 constexpr int kSmallBiasOffset = 0;            // biasbuf: [density b, rgb3 b(3), trans3 b(5)] (fp32, 16 floats)
 
 struct Params {
-  const float* center;       // [rays,3]                              (per-sample launches; the render launch generates rays)
-  const float* ray;          // [rays,3]
-  const float* depth;        // [S]
+  // list mode of the render launch (kMode 4, tp_render_fused_forward_list) keeps its inputs in the slots of per-sample inputs it
+  // does not read: the layout, and with it the code of every other launch, is that of the plain struct
+  union {
+    const float* center;     // [rays,3]                              (per-sample launches; the render launch generates rays)
+    const long long* list;   // list mode: object-pixel list (tp_mask_ray_list), entry q = view * HW + pixel, pad ~(view * HW)
+  };
+  union {
+    const float* ray;        // [rays,3]
+    const long long* n_slots;      // list mode: DEVICE count of list entries (a multiple of 256 / N)
+  };
+  union {
+    const float* depth;      // [S]
+    struct { int shard_rank, shard_world; };      // list mode: this rank renders super-tiles [r T / w, (r + 1) T / w)
+  };
   long long S;
   int N;                     // samples per ray
   long long per_image;       // samples per image

@@ -116,6 +116,14 @@ struct RenderParams : Params {
   float *o_rgb, *o_rgb_s, *o_rgb_t, *o_depth, *o_op, *o_op_s, *o_op_t, *o_unc, *o_as, *o_at, *o_density;
   long long vrow_off;        // byte offset in scratch of the view-bias rows: [CTA][8 drain warps][128] floats
 };
+// The render launch over an object-pixel list (tp_tc32_render_forward_list): ray j of the launch is slot j of the list
+// (tp_mask_ray_list), entry q = view * HW + pixel, a pad entry ~(view * HW) is pixel 0 of its view and stores nothing.  Its rays,
+// jitter keys and output addresses are those of pixel q of a full-frame launch (ray_idx NULL, ray0 = 0, R = HW).
+struct ListRenderParams : RenderParams {
+  const long long* list;
+  const long long* n_slots;  // device: list entries, a multiple of 256 / N (whole super-tiles = two 128-row tiles, one view each)
+  int shard_rank, shard_world;      // this rank renders super-tiles [floor(r T / w), floor((r + 1) T / w)), T = n_slots N / 256
+};
 
 // hi / lo fp16 words of two fp32 values (x0 in the low half): hi = fp16(x), lo = fp16(x - hi) -> x to ~22 mantissa bits
 __device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
@@ -163,6 +171,36 @@ __device__ __forceinline__ void render_unproject(const RenderParams& p, long lon
   unproject(p.kinv + b * 9, p.pinv + b * 12, __fadd_rn((float)(pix % p.W), p.pix_offset), __fadd_rn((float)(pix / p.W), p.pix_offset),
             c, dir);
 }
+// first (end = 0) / one past the last (end = 1) 128-row tile of this rank's share of the list
+__device__ __forceinline__ long long list_tiles(const ListRenderParams& p, int end) {
+  return 2 * (*p.n_slots / (256 / p.N) * (p.shard_rank + end) / p.shard_world);
+}
+// tiles of the launch; list mode: of this rank's share of the list (render_ray adds the first one's index)
+template <class P>
+__device__ __forceinline__ long long launch_tiles(const P& p) { return (p.S + 127) / 128; }
+__device__ __forceinline__ long long launch_tiles(const ListRenderParams& p) { return list_tiles(p, 1) - list_tiles(p, 0); }
+// view of a row (the per-image bias row it reads): its sample's; list mode: its list entry's
+template <class P>
+__device__ __forceinline__ long long image_of(const P& p, long long tile, int row, long long s) { return s / p.per_image; }
+__device__ __forceinline__ long long image_of(const ListRenderParams& p, long long tile, int row, long long s);
+// list mode: the "ray" of a row is its frame position q (a pad: pixel 0 of its view, not live)
+__device__ __forceinline__ long long render_ray(const ListRenderParams& p, long long tile, int row, bool& live) {
+  const long long q = p.list[(list_tiles(p, 0) + tile) * (128 / p.N) + row / p.N];
+  live = q >= 0;
+  return live ? q : ~q;
+}
+__device__ __forceinline__ long long image_of(const ListRenderParams& p, long long tile, int row, long long s) {
+  bool live;
+  return render_ray(p, tile, row, live) / ((long long)p.H * p.W);
+}
+__device__ __forceinline__ void render_unproject(const ListRenderParams& p, long long ray, long long& b, long long& pix, float c[3],
+                                                 float dir[3]) {
+  const long long HW = (long long)p.H * p.W;
+  b = ray / HW;
+  pix = ray - b * HW;
+  unproject(p.kinv + b * 9, p.pinv + b * 12, __fadd_rn((float)(pix % p.W), p.pix_offset), __fadd_rn((float)(pix / p.W), p.pix_offset),
+            c, dir);
+}
 
 // jitter of this lane's sample and of the next sample of its ray.  A warp holds 32 consecutive samples of one ray = 8 Philox
 // quads (counter = sample / 4): lanes 0..8 evaluate quads 0..8 once (quad 8: the next warp's first sample), shuffles hand out.
@@ -188,7 +226,8 @@ __device__ __forceinline__ void render_jitter_pair(const RenderParams& p, long l
   if (lane == 31) u1 = nq;
 }
 
-__device__ __noinline__ RenderSample render_sample(const RenderParams& p, long long tile, int row, int lane) {
+template <class P>
+__device__ __noinline__ RenderSample render_sample(const P& p, long long tile, int row, int lane) {
   RenderSample o;
   const int N = p.N;                                       // 32, 64 or 128: divides 128
   o.k = row & (N - 1);
@@ -212,8 +251,8 @@ __device__ __noinline__ RenderSample render_sample(const RenderParams& p, long l
 }
 
 // The E tile row of the sample: the same fp32 encoding as the per-sample launch's encode_tile (no save slot).
-template <bool kSingle>
-__device__ __noinline__ void render_encode(const RenderParams& p, long long tile, int row, int lane, uint32_t sbase) {
+template <bool kSingle, class P>
+__device__ __noinline__ void render_encode(const P& p, long long tile, int row, int lane, uint32_t sbase) {
   const RenderSample rs = render_sample(p, tile, row, lane);
   float v[64];
 #pragma unroll
@@ -246,7 +285,8 @@ __device__ __noinline__ void render_encode(const RenderParams& p, long long tile
 // + W_view [u, enc(u)], u = ray / |ray| (layers/nerf_static_transient_light.py:104-117), with tp_tc_ray_bias's operation order --
 // one fma chain per column, inputs ascending -- so the row has the table's bits.  Lane j holds input j, lane l computes columns
 // 4l .. 4l + 3 of the half; the row goes to the warp's slot `dst`, which the drain of this stage reads back.
-__device__ __noinline__ void render_view_row(const RenderParams& p, long long tile, int row, int lane, int half, float* dst) {
+template <class P>
+__device__ __noinline__ void render_view_row(const P& p, long long tile, int row, int lane, int half, float* dst) {
   bool live;
   const long long ray = render_ray(p, tile, row, live);
   long long b, pix;
@@ -402,11 +442,12 @@ __device__ __noinline__ void render_composite(const RenderParams& p, float* sc, 
 // drain can also keep every hidden activation as a bf16 tile image for the tensor-core backward (training of layers/nerf.py).
 // kSplitSave (with kSingle = false): the parity-mode arithmetic unchanged, and the drain also keeps every save-slot activation and
 // the encoding tile as bf16 hi + lo tile images (slots 2k, 2k + 1) plus the ReLU bitmasks: the operands of the split backward.
-// P = RenderParams: the render launch (samples made in-kernel, per-ray outputs; no save).
+// P = RenderParams: the render launch (samples made in-kernel, per-ray outputs; no save); P = ListRenderParams: the same over an
+// object-pixel list, this rank's share of its tiles.
 template <bool kSingle, bool kSplitSave, class P = Params>
 __device__ __forceinline__ void nerf_forward_split_body(const P& p) {
   static_assert(!(kSingle && kSplitSave), "the split save belongs to the three-pass arithmetic");
-  constexpr bool kRender = std::is_same<P, RenderParams>::value;
+  constexpr bool kRender = std::is_base_of<RenderParams, P>::value;
   static_assert(!(kRender && kSplitSave), "the render launch keeps no activations");
   constexpr bool kSave = (kSingle || kSplitSave) && !kRender;      // the launch can write tile images
   constexpr int kImgPerSlot = kSplitSave ? 2 : 1;     // tile images per save slot (hi, lo)
@@ -447,7 +488,7 @@ __device__ __forceinline__ void nerf_forward_split_body(const P& p) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const long long n_tiles = (p.S + 127) / 128;
+  const long long n_tiles = launch_tiles(p);
   const int n_stages = p.n_stages;
 
   if (warp == kProducerWarp) {
@@ -656,7 +697,7 @@ __device__ __forceinline__ void nerf_forward_split_body(const P& p) {
           const float* brow = kRender && sg.bias_kind == BIAS_RAY ? vrow
                             : (sg.bias_kind == BIAS_STATIC ? p.bias + sg.bias_off
                                : sg.bias_kind == BIAS_RAY  ? p.raybias + (s / p.N) * 256
-                                                           : p.imgbias + (s / p.per_image) * 256) + half * 128;
+                                                           : p.imgbias + image_of(p, tile, row, s) * 256) + half * 128;
           const uint32_t tmem_d = tmem_row + (uint32_t)(L & 1) * 256 + half * 128;
           const bool do_park = (sg.flags & F_PARK) != 0;
           uint8_t* const g_save = (kSave && p.save && sg.save_slot >= 0)
@@ -802,6 +843,10 @@ __global__ void __launch_bounds__(kThreads, 1) nerf_forward_split_save_kernel(co
 template <bool kSingle>
 __global__ void __launch_bounds__(kThreads, 1) nerf_render_split_kernel(const __grid_constant__ RenderParams p) {
   nerf_forward_split_body<kSingle, false, RenderParams>(p);
+}
+template <bool kSingle>
+__global__ void __launch_bounds__(kThreads, 1) nerf_render_list_split_kernel(const __grid_constant__ ListRenderParams p) {
+  nerf_forward_split_body<kSingle, false, ListRenderParams>(p);
 }
 
 // slot_desc row: [W ptr, ld, row0, rows_valid, col0, cols_valid, kind (256 | 16), unused]
@@ -1015,6 +1060,54 @@ TP_API int tp_tc32_render_forward(const float* kinv, const float* pose_inv, int 
   p.o_density = density;
   p.vrow_off = tp_tc32_status_offset() + 256;
   void (*kern)(const tcs::RenderParams) = precision ? tcs::nerf_render_split_kernel<true> : tcs::nerf_render_split_kernel<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcs::kSmemRender);
+  if (e != cudaSuccess) return (int)e;
+  kern<<<grid, tcs::kThreads, tcs::kSmemRender, (cudaStream_t)stream>>>(p);
+  return tp_launch_status();
+}
+
+/* The same launch over an object-pixel list: one CTA per SM (the host does not know the list's length); rank shard_rank of
+ * shard_world renders its share of the list's super-tiles. */
+TP_API int tp_tc32_render_forward_list(const float* kinv, const float* pose_inv, int B, int H, int W, float pix_offset,
+                                       const int64_t* list, const int64_t* n_slots, int shard_rank, int shard_world,
+                                       const float* z_near, const float* z_far, int N, int depth_mode, const float* rand, uint64_t seed,
+                                       const void* image, int n_weight_slots, const int32_t* stages, int n_stages, const float* bias,
+                                       const float* wview, int L_view, const float* imgbias_rgb, const float* imgbias, int chains,
+                                       float min_uncert, float* rgb, float* rgb_static, float* rgb_transient, float* depth,
+                                       float* opacity, float* opacity_static, float* opacity_transient, float* uncert,
+                                       float* alpha_static, float* alpha_transient, float* density, void* scratch,
+                                       int64_t scratch_bytes, int precision, void* stream) {
+  if (!kinv || !pose_inv || !list || !n_slots || !z_near || !z_far || !image || !stages || !bias || !wview || !imgbias_rgb || !scratch)
+    return TP_ERR_BAD_ARG;
+  if (B < 1 || H < 1 || W < 1 || L_view < 0 || L_view > 4 || n_stages < 1 || n_stages > tcs::kMaxStages) return TP_ERR_BAD_SHAPE;
+  if (N != 32 && N != 64 && N != 128) return TP_ERR_BAD_SHAPE;
+  if (depth_mode < 0 || depth_mode > 2 || (depth_mode == 0 && !rand)) return TP_ERR_BAD_ARG;      // rand: [B*H*W*N], frame-sized
+  if (shard_world < 1 || shard_rank < 0 || shard_rank >= shard_world) return TP_ERR_BAD_ARG;
+  if ((precision != 0 && precision != 1) || chains != 3) return TP_ERR_BAD_ARG;      // the static / transient / light model
+  if (((uintptr_t)image & 15) || ((uintptr_t)scratch & 15) || ((uintptr_t)bias & 15) || ((uintptr_t)wview & 15) ||
+      ((uintptr_t)imgbias_rgb & 15) || ((uintptr_t)imgbias & 15) || ((uintptr_t)density & 7))
+    return TP_ERR_ALIGN;
+  if (!tp_device_is_sm100()) return TP_ERR_ARCH;
+  tcs::ListRenderParams p = {};
+  const int err = tc32_parse_stages(p, stages, n_stages, n_weight_slots, true, imgbias != nullptr, nullptr, 0, -1);
+  if (err != TP_OK) return err;
+  if (scratch_bytes < tp_tc32_render_scratch_bytes()) return TP_ERR_WORKSPACE;
+  const int grid = tp_num_sms();
+  p.S = 0; p.N = N; p.per_image = (int64_t)H * W * N;      // (list mode takes its rays and its length from the list)
+  p.image = reinterpret_cast<const uint8_t*>(image); p.bias = bias; p.imgbias = imgbias;
+  p.scratch = reinterpret_cast<uint8_t*>(scratch);
+  p.status = reinterpret_cast<unsigned int*>(p.scratch + tp_tc32_status_offset());
+  p.enc_slot = -1;
+  p.kinv = kinv; p.pinv = pose_inv; p.H = H; p.W = W; p.pix_offset = pix_offset;
+  p.z_near = z_near; p.z_far = z_far; p.depth_mode = depth_mode; p.rand = rand; p.seed = seed;
+  p.wview = wview; p.L_view = L_view; p.imgbias_rgb = imgbias_rgb; p.chains = chains; p.min_uncert = min_uncert;
+  p.o_rgb = rgb; p.o_rgb_s = rgb_static; p.o_rgb_t = rgb_transient; p.o_depth = depth; p.o_op = opacity;
+  p.o_op_s = opacity_static; p.o_op_t = opacity_transient; p.o_unc = uncert; p.o_as = alpha_static; p.o_at = alpha_transient;
+  p.o_density = density;
+  p.vrow_off = tp_tc32_status_offset() + 256;
+  p.list = reinterpret_cast<const long long*>(list); p.n_slots = reinterpret_cast<const long long*>(n_slots);
+  p.shard_rank = shard_rank; p.shard_world = shard_world;
+  void (*kern)(const tcs::ListRenderParams) = precision ? tcs::nerf_render_list_split_kernel<true> : tcs::nerf_render_list_split_kernel<false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcs::kSmemRender);
   if (e != cudaSuccess) return (int)e;
   kern<<<grid, tcs::kThreads, tcs::kSmemRender, (cudaStream_t)stream>>>(p);

@@ -125,11 +125,12 @@ class NeRF(torch.nn.Module):
         return self.uses_tensor_cores(opt, mode)
 
     def render_rays(self, opt, kinv, pinv, ray_idx, ray0, R, z_near, z_far, latent_variable_trans, latent_variable_light,
-                    mode=None, rand=None, seed=0, want=None, out_ptrs=None):
+                    mode=None, rand=None, seed=0, want=None, out_ptrs=None, ray_list=None, shard=(0, 1)):
         """get_center_and_ray + ray_batch_sample + sample_depth + forward_samples + composite (model/nerf_adapt_st_gan.py:565-631)
         in one launch; returns the dict of the eleven outputs of Graph.render.  The lock-step bf16 render launch
         (tp_render_fused_forward) where it implements the precision and architecture; otherwise the staged kernel's render launch
-        (tp_tc32_render_forward, render_precision)."""
+        (tp_tc32_render_forward, render_precision).  List form: ray_list = (list, n_slots) of ops.mask_ray_list with ray_idx None,
+        ray0 0, R = H*W -- the object pixels of a mask prior, frame-sized outputs (mlp_tc.render_fused)."""
         from .. import mlp_tc
         cfg = self._config(opt, mode)
         pairs = lambda ml: [(l.weight.detach(), l.bias.detach()) for l in ml]
@@ -141,11 +142,12 @@ class NeRF(torch.nn.Module):
             return mlp_tc32.render(cfg, kinv, pinv, opt.H, opt.W, ray_idx, ray0, R, ops._f32(z_near), ops._f32(z_far),
                                    opt.nerf.sample_intvs, lt, ll, pairs(self.mlp_feat), pairs(self.mlp_rgb), pairs(self.mlp_trans),
                                    float(opt.nerf.min_uncert), rand=rand, stratified=bool(opt.nerf.sample_stratified), seed=seed,
-                                   precision=precision, want=want, out_ptrs=out_ptrs)
+                                   precision=precision, want=want, out_ptrs=out_ptrs, ray_list=ray_list, shard=shard)
         return mlp_tc.render_fused(cfg, kinv, pinv, opt.H, opt.W, ray_idx, ray0, R, ops._f32(z_near), ops._f32(z_far),
                                    opt.nerf.sample_intvs, lt, ll, pairs(self.mlp_feat), pairs(self.mlp_rgb), pairs(self.mlp_trans),
                                    float(opt.nerf.min_uncert), rand=rand, stratified=bool(opt.nerf.sample_stratified), seed=seed,
-                                   static_only=cfg.static_only, want=want or mlp_tc.RENDER_KEYS, out_ptrs=out_ptrs)
+                                   static_only=cfg.static_only, want=want or mlp_tc.RENDER_KEYS, out_ptrs=out_ptrs,
+                                   ray_list=ray_list, shard=shard)
 
     def _lockstep_render_applies(self, opt, cfg) -> bool:
         """render_rays takes tp_render_fused_forward: bf16 / auto precision and the architecture the lock-step kernel implements."""

@@ -196,13 +196,17 @@ RENDER_KEYS = ("rgb", "rgb_static", "rgb_transient", "depth", "opacity", "opacit
 
 
 def render_fused(cfg, kinv, pinv, H, W, ray_idx, ray0, R, z_near, z_far, N, lat_trans, lat_light, feat_p, rgb_p, trans_p,
-                 min_uncert, rand=None, stratified=True, seed=0, static_only=False, want=RENDER_KEYS, out_ptrs=None):
+                 min_uncert, rand=None, stratified=True, seed=0, static_only=False, want=RENDER_KEYS, out_ptrs=None, ray_list=None,
+                 shard=(0, 1)):
     """Graph.render after ray selection (model/nerf_adapt_st_gan.py:565-631) as ONE launch: tp_render_fused_forward.
 
     ray_idx: [B,R] int64 pixel indices, or None for the row block [ray0, ray0+R) of every view.  z_near / z_far: [B,H*W].
     want: which of the reference's eleven outputs are materialised.  out_ptrs: {key: raw device address} overriding the
     destination of an output (e.g. a row block of a frame buffer in a peer GPU's window: the stores then travel over NVLink);
-    such outputs are not returned.  Returns the dict of allocated outputs in the reference's shapes."""
+    such outputs are not returned.  Returns the dict of allocated outputs in the reference's shapes.
+    ray_list = (list, n_slots) from ops.mask_ray_list: the list form (tp_render_fused_forward_list) -- the rays are the list's
+    object pixels (R must be H*W), rank shard[0] of shard[1] renders its share of them, outputs and `rand` are frame-sized
+    ([B,H*W,...]) and only the object pixels' rows are written."""
     if N not in FUSED_N:
         raise NotImplementedError(f"the fused render launch takes {FUSED_N} samples per ray")
     if not supported(cfg, feat_p, rgb_p, trans_p):
@@ -233,10 +237,17 @@ def render_fused(cfg, kinv, pinv, H, W, ray_idx, ray0, R, z_near, z_far, N, lat_
         mode, rand_t = 1, None
     else:
         mode, rand_t = 2, None
+    scratch = _scratch_for(dev)
+    if ray_list is not None:
+        assert R == H * W
+        _C.call("tp_render_fused_forward_list", ops._p(kinv), ops._p(pinv), B, H, W, 0.5, ops._p(ray_list[0]), ops._p(ray_list[1]),
+                int(shard[0]), int(shard[1]), ops._p(z_near), ops._p(z_far), N, mode, ops._p(rand_t), int(seed), ops._p(pk.weights),
+                ops._p(pk.biasbuf), ops._p(pk.wview), cfg.L_view, ops._p(img_r), ops._p(img_t), float(min_uncert),
+                *[dst(k) for k in RENDER_KEYS], ops._p(scratch), scratch.numel(), STATIC_ONLY if static_only else 0, ops._stream())
+        return ret
     if ray_idx is not None:
         ray_idx = ray_idx.to(torch.int64).contiguous()
         assert ray_idx.shape == (B, R)
-    scratch = _scratch_for(dev)
     _C.call("tp_render_fused_forward", ops._p(kinv), ops._p(pinv), B, H, W, 0.5, ops._p(ray_idx), R, int(ray0), ops._p(z_near),
             ops._p(z_far), N, mode, ops._p(rand_t), int(seed), ops._p(pk.weights), ops._p(pk.biasbuf), ops._p(pk.wview),
             cfg.L_view, ops._p(img_r), ops._p(img_t), float(min_uncert), *[dst(k) for k in RENDER_KEYS], ops._p(scratch),

@@ -222,12 +222,13 @@ PLAIN_RENDER_KEYS = ("rgb", "depth", "opacity", "density")      # the plain mode
 
 
 def render(cfg, kinv, pinv, H, W, ray_idx, ray0, R, z_near, z_far, N, lat_trans, lat_light, feat_p, rgb_p, trans_p, min_uncert,
-           rand=None, stratified=True, seed=0, static_only=False, precision=0, want=None, out_ptrs=None):
+           rand=None, stratified=True, seed=0, static_only=False, precision=0, want=None, out_ptrs=None, ray_list=None, shard=(0, 1)):
     """Graph.render after ray selection as ONE launch of the staged kernel (tp_tc32_render_forward): rays, depths, the per-ray
     bias row and the compositing happen in-kernel.  static_only=True: the plain layers/nerf.py model (its layer list as
     NeRF._tc32_parameters builds it, one compositing chain, outputs PLAIN_RENDER_KEYS, density [B,R,N]); otherwise the static /
     transient / light model (the eleven RENDER_KEYS).  precision 0: split hi + lo (<= 1e-4); 1: single-pass bf16 (<= 1e-2).
-    ray_idx / ray0 / R, z_near / z_far, rand / stratified / seed, want and out_ptrs as mlp_tc.render_fused."""
+    ray_idx / ray0 / R, z_near / z_far, rand / stratified / seed, want, out_ptrs and the list form (ray_list, shard: the static /
+    transient / light model only; tp_tc32_render_forward_list) as mlp_tc.render_fused."""
     import ctypes
     if N not in mlp_tc.FUSED_N:
         raise NotImplementedError(f"the staged render launch takes {mlp_tc.FUSED_N} samples per ray")
@@ -268,10 +269,20 @@ def render(cfg, kinv, pinv, H, W, ray_idx, ray0, R, z_near, z_far, N, lat_trans,
         mode, rand_t = 1, None
     else:
         mode, rand_t = 2, None
+    scratch = _scratch_for(dev)
+    if ray_list is not None:
+        if static_only:
+            raise NotImplementedError("the list form of the staged render launch renders the static / transient / light model")
+        assert R == H * W
+        _C.call("tp_tc32_render_forward_list", ops._p(ops._f32(kinv)), ops._p(ops._f32(pinv)), B, H, W, 0.5, ops._p(ray_list[0]),
+                ops._p(ray_list[1]), int(shard[0]), int(shard[1]), ops._p(z_near), ops._p(z_far), N, mode, ops._p(rand_t), int(seed),
+                ops._p(pk.image), pk.n_slots, ops._p(pk.stages), pk.stages.shape[0], ops._p(pk.bias), ops._p(pk.wview), cfg.L_view,
+                ops._p(img_r), ops._p(img_t), 3, float(min_uncert), *[dst(k) for k in RENDER_KEYS], ops._p(scratch), scratch.numel(),
+                int(precision), ops._stream())
+        return ret
     if ray_idx is not None:
         ray_idx = ray_idx.to(torch.int64).contiguous()
         assert ray_idx.shape == (B, R)
-    scratch = _scratch_for(dev)
     _C.call("tp_tc32_render_forward", ops._p(ops._f32(kinv)), ops._p(ops._f32(pinv)), B, H, W, 0.5, ops._p(ray_idx), R, int(ray0),
             ops._p(z_near), ops._p(z_far), N, mode, ops._p(rand_t), int(seed), ops._p(pk.image), pk.n_slots, ops._p(pk.stages),
             pk.stages.shape[0], ops._p(pk.bias), ops._p(pk.wview), cfg.L_view, ops._p(img_r), ops._p(img_t),

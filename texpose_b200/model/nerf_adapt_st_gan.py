@@ -273,6 +273,52 @@ class Graph(torch.nn.Module):
                     ret_all[k][b, ray_idx[0]] = ret[k][0]
         return ret_all
 
+    def render_masked(self, opt, pose, intr, depth_range, object_mask, sample_idx=None, mode="eval", want=None, out_ptrs=None,
+                      shard=None):
+        """The mask-prior branch of render_by_slices (model/nerf_adapt_st_gan.py:647-680) for B views as one render launch (the
+        lock-step bf16 launch where it applies, otherwise the staged kernel's, as NeRF.render_rays chooses): the
+        object pixels (object_mask > 0) of every view are rendered from a ray list built on the device (ops.mask_ray_list), every
+        other pixel holds the defaults of :657-667.  No host synchronisation: the call can be captured in a CUDA graph.
+        Returns render_by_slices' eleven keys ([B,HW,C]; `want` restricts them).  Sample keys are those of a full-frame launch, so
+        with rng 'torch' the jitter is a frame-sized torch.rand(B, HW, N, 1): a seeded call equals the seeded full-frame
+        `_render_fused(range(0, HW))` call at the object pixels (the seeded stream of render_by_slices' per-view draws differs).
+        out_ptrs: {key: device address of a [B*HW,C] frame buffer}, as for _render_fused.  shard = (rank, world): render this
+        rank's share of the list and the defaults of the row block parallel.shard_rays(HW, rank, world, align=W) only.
+
+        Where it runs: wherever a render launch renders the model -- the lock-step launch where `fused_render_applies` (bf16 / auto and
+        the yaml's architecture), otherwise the staged launch (opt.b200.mlp = 'fp32', and bf16 for other 256-wide architectures), as
+        FrameGather's 'val' frames do.  There render_by_slices takes the multi-kernel path instead, whose compositing sums in another
+        order: the two agree to <= 1e-4 in the fp32 mode, not bit for bit.  Raises NotImplementedError in training, with a gradient
+        recorded, with opt.b200.fused_render = False, and (from NeRF.render_rays) for what neither render launch takes."""
+        if opt.camera.ndc:
+            raise NotImplementedError("camera.ndc is false in every reference yaml; not implemented")
+        if mode == "train" or torch.is_grad_enabled() or not self._b200(opt, "fused_render", True):
+            raise NotImplementedError("render_masked runs on a render launch: inference only (torch.no_grad(), not mode 'train')")
+        # (NeRF.render_rays raises NotImplementedError for whatever else neither render launch takes: N, precision, architecture)
+        from ..parallel import shard_rays
+        B, HW, N = len(pose), opt.H * opt.W, opt.nerf.sample_intvs
+        dev = pose.device
+        kinv, pinv = camera.view_matrices(pose, intr, one_launch=camera.one_launch_matrices(opt))
+        zn, zf = depth_range[0].reshape(B, HW), depth_range[1].reshape(B, HW)
+        lat_trans, lat_light = self._latents(opt, B, sample_idx, mode, dev)
+        mask = ops._f32(object_mask.reshape(B, HW))
+        ray_list, n_slots, _ = ops.mask_ray_list(mask, N)
+        rand, seed = None, 0
+        if opt.nerf.sample_stratified:
+            if self._b200(opt, "rng", "torch") == "philox":
+                seed = int(torch.randint(0, 2 ** 62, (1,)).item())      # (a host generator: no device read-back)
+            else:
+                rand = torch.rand(B, HW, N, 1, device=dev)
+        rank, world = shard if shard is not None else (0, 1)
+        keys = tuple(want) if want is not None else self.RENDER_KEYS
+        ret = self.nerf.render_rays(opt, kinv, pinv, None, 0, HW, zn, zf, lat_trans, lat_light, mode=mode, rand=rand, seed=seed,
+                                    want=keys, out_ptrs=out_ptrs, ray_list=(ray_list, n_slots), shard=(rank, world))
+        dst = dict(ret)
+        dst.update({k: int(v) for k, v in (out_ptrs or {}).items()})
+        pix0, pix1 = shard_rays(HW, rank, world, align=opt.W)
+        ops.mask_defaults(mask, N, float(opt.nerf.min_uncert), {k: dst[k] for k in keys}, pix0, pix1)
+        return AttrDict(ret)
+
     def evaluate_frame(self, opt, var):
         """Per-frame numbers of Model.evaluate_full (model/nerf_adapt_st_gan.py:341-362) for every view of the batch, without a
         host sync: rgb_map [B,3,H,W] (from rgb_static), depth_map [B,1,H,W] in metres, image * mask, per-view MSE / PSNR on

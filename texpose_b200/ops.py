@@ -76,6 +76,46 @@ def device_table(rows, dtype, device) -> Tensor:
 # ------------------------------------------------------------------------------------------------- rays
 
 
+def mask_ray_list(mask: Tensor, N: int) -> Tuple[Tensor, Tensor, Tensor]:
+    """Object-pixel ray list of a mask prior (render_by_slices, model/nerf_adapt_st_gan.py:655) for B views, built on the device
+    (tp_mask_ray_list): mask [B,...] (object pixel = mask > 0) -> (list int64 [capacity], n_slots int64 [1], counts int64 [B]).
+    Entries q = b*HW + pixel, views in order, pixels ascending, each view's run padded to a multiple of 256 / N with ~(b*HW);
+    n_slots and counts stay on the device (no read-back)."""
+    _need_cuda(mask)
+    B = mask.shape[0]
+    m = _f32(mask.reshape(B, -1))
+    HW = m.shape[1]
+    lib = _C.load()
+    cap = int(lib.tp_mask_ray_list_capacity(B, HW, N))
+    if cap == 0:
+        raise ValueError(f"mask_ray_list: B >= 1, H*W >= 1 and N in (32, 64, 128) (got {B}, {HW}, {N})")
+    lst = torch.empty(cap, dtype=torch.int64, device=m.device)
+    n_slots = torch.empty(1, dtype=torch.int64, device=m.device)
+    counts = torch.empty(B, dtype=torch.int64, device=m.device)
+    ws = torch.empty(int(lib.tp_mask_ray_list_workspace(B, HW)), dtype=torch.uint8, device=m.device)
+    _C.call("tp_mask_ray_list", _p(m), B, HW, N, _p(lst), cap, _p(n_slots), _p(counts), _p(ws), ws.numel(), _stream())
+    return lst, n_slots, counts
+
+
+MASK_DEFAULT_KEYS = ("rgb", "rgb_static", "rgb_transient", "depth", "opacity", "opacity_static", "opacity_transient", "uncert",
+                     "alpha_static", "alpha_transient", "density")
+
+
+def mask_defaults(mask: Tensor, N: int, min_uncert: float, dst: dict, pix0: int = 0, pix1: Optional[int] = None):
+    """The defaults of model/nerf_adapt_st_gan.py:657-667 at the background pixels (mask <= 0) of pixels [pix0, pix1) of every
+    view (tp_mask_defaults).  dst: {key: frame-layout tensor [B,HW,...] or raw device address}; absent keys are skipped."""
+    B = mask.shape[0]
+    m = _f32(mask.reshape(B, -1))
+    HW = m.shape[1]
+
+    def ptr(k):
+        v = dst.get(k)
+        return None if v is None else (ctypes.c_void_p(int(v)) if isinstance(v, int) else _p(v))
+
+    _C.call("tp_mask_defaults", _p(m), B, HW, int(pix0), HW if pix1 is None else int(pix1), N, float(min_uncert),
+            *[ptr(k) for k in MASK_DEFAULT_KEYS], _stream())
+
+
 def raygen(kinv: Tensor, pose_inv: Tensor, H: int, W: int, pix_offset: float = 0.5,
            ray_idx: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
     _need_cuda(kinv, pose_inv, ray_idx)

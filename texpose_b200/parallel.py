@@ -310,11 +310,22 @@ class FrameGather:
         buf = self.window.buffers[parity]
         return {k: buf[o:o + self.HW * c].view(1, self.HW, c) for k, (o, c) in self.layout.items()}
 
-    def render(self, graph, opt, pose, intr, depth_range, sample_idx=None, mode="val", local_keys: Sequence[str] = ()):
+    def render(self, graph, opt, pose, intr, depth_range, sample_idx=None, mode="val", local_keys: Sequence[str] = (),
+               object_mask=None):
         """Renders this rank's row block of the frame of view `pose` ([1,3,4]) and gathers it.  Returns (frame, local): `frame` =
-        {key: [1,HW,C]} on the root (None elsewhere), `local` = the `local_keys` outputs of this rank's rows."""
+        {key: [1,HW,C]} on the root (None elsewhere), `local` = the `local_keys` outputs of this rank's rows.
+
+        With `object_mask` (the eval frame of a mask prior, graph.render_masked): every rank builds the same object-pixel list,
+        renders its share of the list's super-tiles -- balanced by object pixels, not by rows -- straight into the root's frame
+        buffers at the pixels' frame positions, and writes the background defaults of its own row block `self.rows`: every
+        position is written once, by one rank.  Per-sample outputs are not gathered, so local_keys must be empty."""
         if len(pose) != 1:
             raise ValueError("FrameGather renders one view per call")
+        if object_mask is not None:
+            if local_keys:
+                raise ValueError("FrameGather gathers no per-sample outputs of a mask-prior frame: local_keys must be empty")
+            if not hasattr(graph, "render_masked"):
+                raise ValueError(f"{type(graph).__module__}.{type(graph).__name__} renders no mask-prior frame (no render_masked)")
         missing = [k for k in tuple(self.keys) + tuple(local_keys) if k not in getattr(graph, "RENDER_KEYS", ())]
         if missing:
             raise ValueError(f"{type(graph).__module__}.{type(graph).__name__} does not render {missing} "
@@ -323,6 +334,12 @@ class FrameGather:
         par = self.epoch & 1
         b, e = self.rows
         base = self.ptrs[self.root] + self._data_off[par]
+        if object_mask is not None:
+            out_ptrs = {k: base + 4 * o for k, (o, c) in self.layout.items()}
+            graph.render_masked(opt, pose, intr, depth_range, object_mask, sample_idx, mode, want=self.keys, out_ptrs=out_ptrs,
+                                shard=(self.rank, self.world))
+            peer_barrier(self.ptrs, self.rank, self.epoch, self.device, timeout_ms=self.timeout_ms)
+            return (self.frame_views(par) if self.rank == self.root else None), {}
         out_ptrs = {k: base + 4 * (o + b * c) for k, (o, c) in self.layout.items()}
         local = graph._render_fused(opt, pose, intr, range(b, e), depth_range, sample_idx, mode,
                                     want=tuple(self.keys) + tuple(local_keys), out_ptrs=out_ptrs)
