@@ -63,11 +63,25 @@ def cuda_step(opt, g, inp, images, dev, seed):
     var.update(ret)
     loss = base.summarize_loss(opt, var, g.compute_loss(opt, var, mode="train"))
     loss["all"].backward()
-    return {k: p.grad.detach().clone() for k, p in named_trainables(g)}, rand, {k: float(v) for k, v in loss.items()}, (zn.cpu(), zf.cpu())
+    return {k: p.grad.detach().clone() for k, p in named_trainables(g)}, rand, {k: float(v.detach()) for k, v in loss.items()}, (zn.cpu(), zf.cpu())
 
 
-def oracle_step(g, inp, images, rand):
-    """The same step through the CPU oracle (fp32): rays, bounds, depths, MLP, composite, losses, autograd."""
+def oracle_step(g, inp, images, rand, keep=None):
+    """The same step through the CPU oracle (fp32): rays, bounds, depths, MLP, composite, losses, autograd.  `keep` [n, P*P, N]
+    (0 / 1): the per-sample seeds of the masked samples are zeroed (the gradient without their contribution)."""
+    if keep is not None:
+        from tests.gradcheck import cotangent_mask
+        real = O.nerf_stl_forward
+
+        def masked(*a, **kw):
+            rgb, dens, unc = real(*a, **kw)
+            return (cotangent_mask(rgb, keep[..., None, None]), cotangent_mask(dens, keep[..., None]),
+                    cotangent_mask(unc, keep[..., None]))
+        O.nerf_stl_forward = masked
+        try:
+            return oracle_step(g, inp, images, rand)
+        finally:
+            O.nerf_stl_forward = real
     sl = images
     cpu = {k: p.detach().cpu().clone().requires_grad_(True) for k, p in named_trainables(g)}
     feat = [(l.weight.detach().cpu(), l.bias.detach().cpu()) for l in g.nerf.mlp_feat]
@@ -88,4 +102,4 @@ def oracle_step(g, inp, images, rand):
     losses = O.patch_losses(inp.image[sl], inp.mask[sl], coords, out["rgb"], out["uncert"], out["density"], 0.0, 0.0, -2.0)
     losses["all"].backward()
     grads = {k: (p.grad if p.grad is not None else torch.zeros_like(p)) for k, p in cpu.items()}
-    return grads, {k: float(losses[k]) for k in ("render", "uncert", "trans_reg", "all")}, (zn, zf)
+    return grads, {k: float(losses[k].detach()) for k in ("render", "uncert", "trans_reg", "all")}, (zn, zf)

@@ -10,11 +10,19 @@ from oracle import texpose_oracle as O
 from texpose_b200 import _C, synth
 from texpose_b200.config import AttrDict, adapt_gan_opt, env_opt
 from texpose_b200.layers import nerf, nerf_static_transient_light
-from tests.test_gpu_tc import _c1_inputs
+from tests.test_gpu_tc import _c1_inputs, _check_grads
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 TOL = 1e-4
+# relative bounds beside TOL (max-abs / max|grad|, error norm / norm, latent row), 2x the worst measured on one B200
+# (profiles/r06_pytest_grads.log): the plain step vs the oracle 4.52e-5, 3.40e-5; vs the SIMT step 2.40e-4, 2.81e-4; the
+# static/transient/light step vs the oracle 1.30e-4, 3.58e-5, 2.66e-5; the pre-training Graph vs the reference fixture 7.13e-5,
+# 3.61e-5
+REL_PLAIN = (9e-5, 6.7e-5, 0.0)
+REL_SIMT = (4.7e-4, 5.6e-4, 0.0)
+REL_STL = (2.6e-4, 7.1e-5, 5.3e-5)
+REL_GRAPH = (1.4e-4, 7.2e-5, 0.0)
 TC = AttrDict(mlp="fp32", fp32_engine="tc")
 
 
@@ -43,8 +51,9 @@ def _plain_loss(rgb, depth, opacity, sigma, image, mask):
     return (mask * (image - rgb) ** 2).sum() / (mask.sum() + 1e-5) + 0.1 * depth.mean() + 0.05 * opacity.mean() + 0.01 * sigma.mean()
 
 
-def _plain_vs_oracle(opt, m, cpu, R, N, use_forward_samples=True):
-    """One training step of the plain model on the GPU and on the oracle -> (rgb error, composite error, worst gradient error)."""
+def _plain_vs_oracle(opt, m, cpu, R, N, use_forward_samples=True, rel=REL_PLAIN):
+    """One training step of the plain model on the GPU and on the oracle -> (rgb error, composite error, worst gradient error);
+    every gradient within TOL and `rel` of the oracle's."""
     center, ray, depth = _c1_inputs(R=R, N=N, seed_pose=1)
     g = torch.Generator().manual_seed(9)
     image, mask = torch.rand(1, R, 3, generator=g), (torch.rand(1, R, 1, generator=g) > 0.3).float()
@@ -61,13 +70,12 @@ def _plain_vs_oracle(opt, m, cpu, R, N, use_forward_samples=True):
         rgb_g, sig_g = m.forward(opt, pts.to(DEV), unit.to(DEV), mode="train")
     comp_g = m.composite(opt, ray.to(DEV), rgb_g, sig_g, depth.to(DEV))
     _plain_loss(comp_g[0], comp_g[1], comp_g[2], sig_g, image.to(DEV), mask.to(DEV)).backward()
-    worst = 0.0
+    pairs = []
     for (n, a), b in zip(list(m.mlp_feat.named_parameters(prefix="mlp_feat")) + list(m.mlp_rgb.named_parameters(prefix="mlp_rgb")),
                          list(cpu.mlp_feat.parameters()) + list(cpu.mlp_rgb.parameters())):
         assert a.grad is not None and a.grad.shape == b.grad.shape, n
-        err = (a.grad.cpu() - b.grad).abs().max().item()
-        print(f"  {n:22s} |grad|max {b.grad.abs().max().item():9.3e}  max-abs err {err:9.3e}")
-        worst = max(worst, err)
+        pairs.append((n, a.grad, b.grad))
+    worst = _check_grads(f"plain {R}x{N} vs oracle", pairs, rel, tol=TOL)[0]
     out = max((rgb_g.cpu() - rgb_s).abs().max().item(), (sig_g.cpu() - sig).abs().max().item())
     return out, (comp_g[0].cpu() - comp[0]).abs().max().item(), worst
 
@@ -111,12 +119,10 @@ def test_plain_fp32_step_at_the_c3_shape_matches_simt_and_repeats_bit_for_bit():
     opt, m, _ = _plain_models()
     simt = _opt(env_opt, dict(mlp="fp32", fp32_engine="simt"), device=DEV)
     a, a2, ref = _plain_grads(m, opt, inputs), _plain_grads(m, opt, inputs), _plain_grads(m, simt, inputs)
-    worst = 0.0
-    for (n, _), x, x2, y in zip(m.named_parameters(), a, a2, ref):
+    for (n, _), x, x2 in zip(m.named_parameters(), a, a2):
         assert torch.equal(x, x2), n
-        err = (x - y).abs().max().item()
-        worst = max(worst, err)
-        assert err <= TOL, (n, err, y.abs().max().item())
+    worst = _check_grads("plain 16x256x128 tc vs SIMT", [(n, x, y) for (n, _), x, y in zip(m.named_parameters(), a, ref)], REL_SIMT,
+                         tol=TOL)[0]
     print(f"plain 16x256x128: tensor-core fp32 step vs SIMT fp32 step, worst gradient max-abs {worst:.2e}")
 
 
@@ -185,13 +191,7 @@ def test_static_transient_light_fp32_step_on_tensor_cores_vs_oracle(arch):
     for n, a, b in zip(names, list(m.mlp_rgb.parameters()) + list(m.mlp_trans.parameters()),
                        list(cpu.mlp_rgb.parameters()) + list(cpu.mlp_trans.parameters())):
         pairs.append((n, a.grad.cpu(), b.grad))
-    worst = 0.0
-    for n, a, b in pairs:
-        err = (a - b).abs().max().item()
-        print(f"  {n:22s} |grad|max {b.abs().max().item():9.3e}  max-abs err {err:9.3e}")
-        assert a.shape == b.shape
-        worst = max(worst, err)
-    print(f"static/transient/light {arch or 'yaml'}: worst gradient max-abs error {worst:.2e}")
+    worst = _check_grads(f"static/transient/light {arch or 'yaml'} vs oracle", pairs, REL_STL, tol=TOL)[0]
     assert worst <= TOL
 
 
@@ -227,11 +227,13 @@ def test_pretrain_graph_fp32_tc_step_matches_the_real_reference(golden, monkeypa
         assert _C.launch_counts.get("tp_tc32_forward_split_save") == 1 and _C.launch_counts.get("tp_tc_chain_backward_split") == 1
         errs = {k: (var[k].cpu() - g["o_" + k]).abs().max().item() for k in ("rgb", "depth", "opacity")}
         errs.update({"l_" + k: abs(loss[k].item() - float(g["l_" + k])) for k in ("render", "mask", "depth")})
-        worst, mag = 0.0, 0.0
+        worst, mag, pairs = 0.0, 0.0, []
         for n, p in gr.nerf.named_parameters():
             got = p.grad if p.grad.numel() <= 2048 else p.grad[:, ::8][::8]
             worst = max(worst, (got.cpu() - g["g/" + n]).abs().max().item())
             mag = max(mag, g["g/" + n].abs().max().item())
+            pairs.append((n, got, g["g/" + n]))
+        _check_grads("pretrain Graph vs reference", pairs, REL_GRAPH, tol=TOL)
         errs["grad"] = worst
         print("pretrain Graph, fp32 step on the tensor cores, vs the real reference:", {k: f"{v:.2e}" for k, v in errs.items()},
               f"gradient error relative to max |grad| {mag:.3e}: {worst / mag:.2e}")

@@ -9,11 +9,23 @@ from oracle import texpose_oracle as O
 from texpose_b200 import _C
 from texpose_b200.config import AttrDict, env_opt
 from texpose_b200.layers.nerf import NeRF
-from tests.test_gpu_tc import _c1_inputs
+from tests import bf16_reference as BR
+from tests import gradcheck as G
+from tests.test_gpu_tc import _c1_inputs, _check_grads
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 TOL = 1e-2
+# relative bounds beside TOL (max-abs / max|grad|, error norm / norm), 2x the worst measured on one B200
+# (profiles/r06_pytest_grads.log).  Oracle step: against the exact oracle the largest-entry error is 5.2e-2 (bound
+# REL_EXACT_MAX), but the trunk's early layers sit up to 7.7 % off in norm -- as far as the float64 reference that rounds to bf16
+# where the step rounds (tests/bf16_reference.py) sits from the exact oracle: bf16 rounding through eight trunk layers, not the
+# kernels.  Against that reference the step measures 7.7e-3 and 1.0e-2, held in both measures (REL_ORACLE).  vs SIMT 128 x 32 9.99e-3, 9.97e-3; C3 shape vs
+# SIMT 1.22e-2, 2.23e-2
+REL_EXACT_MAX = 0.10
+REL_ORACLE = (0.015, 0.020, 0.0)
+REL_SIMT = (0.019, 0.019, 0.0)
+REL_C3 = (0.024, 0.044, 0.0)
 
 
 def _models(seed=0):
@@ -58,15 +70,24 @@ def test_plain_training_step_gradients_vs_oracle(R, N):
     assert _C.launch_counts.get("tp_tc_dw_gemm") == 1 and "tp_linear_forward" not in _C.launch_counts
     assert "tp_linear_backward_input" not in _C.launch_counts
     assert (rgb_g.cpu() - rgb_s).abs().max() <= 2e-2 and (comp_g[0].cpu() - comp[0]).abs().max() <= TOL
-    worst = 0.0
-    for (n, a), b in zip(list(m.mlp_feat.named_parameters(prefix="mlp_feat")) + list(m.mlp_rgb.named_parameters(prefix="mlp_rgb")),
-                         list(cpu.mlp_feat.parameters()) + list(cpu.mlp_rgb.parameters())):
+    # ---- the bf16-rounding reference (float64, rounded where the step rounds: tests/bf16_reference.py), same loss
+    P = [(l.weight.detach().double().requires_grad_(True), l.bias.detach().double().requires_grad_(True))
+         for l in list(cpu.mlp_feat) + list(cpu.mlp_rgb)]
+    rgb_r, sig_r = BR.plain_forward(pts.double(), unit.double(), P[:len(cpu.mlp_feat)], P[len(cpu.mlp_feat):])
+    comp_r = O.composite_plain(ray.double(), rgb_r, sig_r, depth.double())
+    _loss(comp_r[0], comp_r[1], comp_r[2], sig_r, image.double(), mask.double()).backward()
+    ref = [t.grad for pair in P for t in pair]
+    pairs, gap = [], 0.0
+    for (n, a), b, r in zip(list(m.mlp_feat.named_parameters(prefix="mlp_feat")) + list(m.mlp_rgb.named_parameters(prefix="mlp_rgb")),
+                            list(cpu.mlp_feat.parameters()) + list(cpu.mlp_rgb.parameters()), ref):
         assert a.grad is not None and a.grad.shape == b.grad.shape, n
-        err, mag = (a.grad.cpu() - b.grad).abs().max().item(), b.grad.abs().max().item()
-        print(f"  {n:22s} |grad|max {mag:9.3e}  max-abs err {err:9.3e}")
-        worst = max(worst, err)
-        assert err <= TOL, (n, err, mag)
-    print(f"plain model, tensor-core training step: worst gradient max-abs error {worst:.2e}")
+        # the exact oracle: the north-star absolute bound and the largest-entry bound
+        err, (e_max, _) = float((a.grad.cpu() - b.grad).abs().max()), G.rel_errors(a.grad, b.grad)
+        assert err <= TOL and e_max <= REL_EXACT_MAX, (n, err, e_max)
+        gap = max(gap, G.rel_errors(r, b.grad.double())[1])
+        pairs.append((n, a.grad, r))
+    print(f"plain {R}x{N}: bf16-rounding reference vs exact oracle, worst error norm / norm {gap:.3e}")
+    _check_grads(f"plain {R}x{N} tensor-core step vs bf16-rounding reference", pairs, REL_ORACLE)
 
 
 def test_plain_training_is_deterministic_and_fp32_mode_keeps_simt():
@@ -87,8 +108,7 @@ def test_plain_training_is_deterministic_and_fp32_mode_keeps_simt():
     _C.launch_counts.clear()
     c = grads(o32)
     assert "tp_tc_chain_backward" not in _C.launch_counts and _C.launch_counts.get("tp_linear_forward", 0) > 0
-    for x, y in zip(a, c):
-        assert (x - y).abs().max() <= TOL
+    _check_grads("plain 128x32 tensor-core vs SIMT", [(n, x, y) for (n, _), x, y in zip(m.named_parameters(), a, c)], REL_SIMT)
 
 
 def test_chain_stage_list_is_validated():
@@ -131,6 +151,6 @@ def test_plain_training_step_at_the_c3_shape_matches_the_simt_step():
         return [p.grad.clone() for p in m.parameters()]
 
     a, a2, ref = grads(opt), grads(opt), grads(o32)
-    for (n, _), x, x2, y in zip(m.named_parameters(), a, a2, ref):
+    for (n, _), x, x2 in zip(m.named_parameters(), a, a2):
         assert torch.equal(x, x2), n
-        assert (x - y).abs().max() <= TOL, (n, float((x - y).abs().max()), float(y.abs().max()))
+    _check_grads("plain C3 shape tensor-core vs SIMT", [(n, x, y) for (n, _), x, y in zip(m.named_parameters(), a, ref)], REL_C3)

@@ -10,11 +10,14 @@ from oracle import texpose_oracle as O
 from texpose_b200 import _C, synth
 from texpose_b200.config import AttrDict, adapt_gan_opt
 from texpose_b200.layers.nerf_static_transient_light import NeRF
-from tests.test_gpu_tc import _c1_inputs
+from tests.test_gpu_tc import _c1_inputs, _check_grads
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 TOL = 1e-2
+# relative bounds beside TOL (max-abs / max|grad|, error norm / norm, latent row): 2x the worst measured on one B200 over both
+# architectures, 1.90e-2, 1.34e-2, 1.34e-2 (profiles/r06_pytest_grads.log)
+REL = (0.037, 0.026, 0.026)
 
 
 @pytest.mark.parametrize("arch", [
@@ -73,7 +76,4 @@ def test_other_architectures_train_on_the_staged_kernels(arch):
     for n, a, b in zip(names, list(m.mlp_rgb.parameters()) + list(m.mlp_trans.parameters()),
                        list(cpu.mlp_rgb.parameters()) + list(cpu.mlp_trans.parameters())):
         pairs.append((n, a.grad.cpu(), b.grad))
-    for n, a, b in pairs:
-        err = (a - b).abs().max().item()
-        print(f"  {n:22s} |grad|max {b.abs().max().item():9.3e}  max-abs err {err:9.3e}")
-        assert a.shape == b.shape and err <= TOL, (n, err)
+    _check_grads(f"staged {len(arch['layers_feat']) - 1}-layer trunk", pairs, REL)

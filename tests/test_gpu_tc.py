@@ -8,11 +8,36 @@ from oracle import texpose_oracle as O
 from texpose_b200 import _C, synth
 from texpose_b200.config import AttrDict, adapt_gan_opt
 from texpose_b200.layers.nerf_static_transient_light import NeRF
+from tests import gradcheck as G
 from tests.conftest import layer_list
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 TOL = 1e-2
+# gradient bounds relative to each tensor, beside the absolute TOL: (max-abs error / max|grad|, error norm / norm, latent row).
+# Worst measured on one B200 (profiles/r06_pytest_grads.log): C3 shape 4.07e-2, 3.92e-2, 3.92e-2; fused vs fp32 kernels (all three
+# shapes) 1.98e-2, 1.49e-2, 2.46e-2; tiny images 3.25e-2, 2.90e-2, 4.85e-2.  Bounds: 2x those, at most 10 % / 5 % / 5 %, and the
+# fused test keeps its 2 % of max|grad|.  Three sit close to what they bound -- fused max-abs 1.98e-2 under 0.02, tiny-images latent
+# row 4.85e-2 and C3-shape norm 3.92e-2 under 0.05: the kernels are deterministic, so these do not flake, but a change of a
+# reduction order can move them across; read such a failure against these figures first.
+REL_C3_SHAPE = (0.08, 0.05, 0.05)
+REL_FUSED = (0.02, 0.029, 0.049)
+REL_TINY = (0.065, 0.05, 0.05)
+
+
+def _check_grads(tag, pairs, rel, tol=TOL):
+    """pairs [(name, got, want)]: the absolute bound `tol` and the relative ones `rel`; per-image latent rows one by one (every image of
+    these batches has its own row).  -> (worst max-abs, worst rel max-abs, worst rel norm, worst latent row)."""
+    worst = [0.0, 0.0, 0.0, 0.0]
+    for n, a, b in pairs:
+        a, b = a.detach().cpu(), b.detach().cpu()
+        err = float((a - b).abs().max())
+        assert err <= tol, (n, err)
+        e = G.assert_grad_close(n, a, b, rel_max=rel[0], rel_norm=rel[1], tag=tag)
+        r = G.assert_latent_rows(a, b, range(b.shape[0]), rel[2], name=n, tag=tag) if n.startswith("latent") else 0.0
+        worst = [max(x, y) for x, y in zip(worst, (err, e[0], e[1], r))]
+    print(f"{tag}: worst max-abs {worst[0]:.2e}; relative: max-abs {worst[1]:.3e}, norm {worst[2]:.3e}, latent row {worst[3]:.3e}")
+    return worst
 
 
 def _c1_inputs(R=1024, N=64, seed_pose=0):
@@ -126,18 +151,11 @@ def test_c3_shape_gradients_bf16():
     for n, a, b in zip(names, list(m.mlp_rgb.parameters()) + list(m.mlp_trans.parameters()),
                        list(cpu.mlp_rgb.parameters()) + list(cpu.mlp_trans.parameters())):
         pairs.append((n, a.grad.cpu(), b.grad))
-    worst, gmax = 0.0, 0.0
-    for n, a, b in pairs:
-        err, mag = (a - b).abs().max().item(), b.abs().max().item()
-        print(f"  {n:22s} |grad|max {mag:9.3e}  max-abs err {err:9.3e}  ({100 * err / max(mag, 1e-12):5.2f} % of max)")
-        worst, gmax = max(worst, err), max(gmax, mag)
-    print(f"bf16 fwd gradient max-abs error {worst:.2e} (largest gradient entry {gmax:.2e})")
     # north_star: 1e-2 max-abs with the bf16 MLP path, for gradients of the reference's mean-normalised losses -- every tensor,
     # no relative carve-out (the output layers carry their weights as bf16 hi + lo rows: the systematic rounding of those few
-    # rows was the dominant term for mlp_trans.3.weight, whose entries reach 1.86; DESIGN.md section 2)
-    for n, a, b in pairs:
-        err = (a - b).abs().max().item()
-        assert err <= TOL, (n, err)
+    # rows was the dominant term for mlp_trans.3.weight, whose entries reach 1.86; DESIGN.md section 2) -- and the bounds
+    # relative to each tensor
+    _check_grads("C3-shape", pairs, REL_C3_SHAPE)
 
 
 @pytest.mark.parametrize("B,R,N", [(3, 50, 48), (2, 1200, 32), (16, 256, 128)])
@@ -171,14 +189,7 @@ def test_fused_backward_matches_fp32_kernels(B, R, N):
     assert _C.launch_counts.get("tp_tc_heads_backward", 0) == 1 and "tp_tc_chain_backward" not in _C.launch_counts
     opt32, m32 = _module("fp32")
     b = grads(m32, opt32)
-    worst = 0.0
-    for (n, x), (_, y) in zip(a, b):
-        err, mag = (x - y).abs().max().item(), y.abs().max().item()
-        print(f"  {n:22s} |grad|max {mag:9.3e}  fused-vs-fp32 {err:9.3e}")
-        assert x.shape == y.shape and torch.isfinite(x).all()
-        assert err <= max(1e-3, 0.02 * mag) and err <= TOL, (n, err, mag)
-        worst = max(worst, err)
-    print(f"B,R,N = {B},{R},{N}: worst fused-vs-fp32 gradient max-abs error {worst:.2e}")
+    _check_grads(f"fused-vs-fp32 {B},{R},{N}", [(n, x, y) for (n, x), (_, y) in zip(a, b)], REL_FUSED)
     # deterministic: fixed-order reductions everywhere
     c = grads(m16, opt16)
     for (n, x), (_, y) in zip(a, c):
@@ -207,9 +218,12 @@ def test_backward_falls_back_when_images_are_tiny():
         if prec == "bf16":
             assert _C.launch_counts.get("tp_tc32_forward") == 1 and _C.launch_counts.get("tp_tc_chain_backward") == 2
             assert "tp_tc_nerf_stl_forward" not in _C.launch_counts and "tp_tc_heads_backward" not in _C.launch_counts
-        res[prec] = [lt.grad, ll.grad] + [p.grad for p in list(m.mlp_rgb.parameters()) + list(m.mlp_trans.parameters())]
-    for a, b in zip(res["bf16"], res["fp32"]):
-        assert (a - b).abs().max() <= max(1e-3, 0.02 * b.abs().max().item())
+        named = list(m.mlp_rgb.named_parameters(prefix="mlp_rgb")) + list(m.mlp_trans.named_parameters(prefix="mlp_trans"))
+        res[prec] = [("latent_trans", lt.grad), ("latent_light", ll.grad)] + [(n, p.grad) for n, p in named]
+    pairs = [(n, x, y) for (n, x), (_, y) in zip(res["bf16"], res["fp32"])]
+    _check_grads("tiny-images staged-vs-fp32", pairs, REL_TINY)
+    for n, a, b in pairs:
+        assert (a - b).abs().max() <= max(1e-3, 0.02 * b.abs().max().item()), n
 
 
 @pytest.mark.parametrize("layers_rgb", [[None, 128, 3], [None, 256, 256, 256, 3], [None, 192, 96, 3]])
