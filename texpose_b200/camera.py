@@ -87,6 +87,9 @@ def view_matrices(pose_, intr, one_launch=False):
         ops._C.call("tp_view_matrices", ops._p(intr_c), ops._p(pose_c), B, ops._p(kinv), ops._p(pinv), ops._stream())
         return kinv, pinv
     if HOST_MATRICES and pose_.is_cuda:
+        from .train_graph import refuse_capture
+        refuse_capture("camera.HOST_MATRICES", "the CPU inversion synchronises; compute the matrices eagerly with "
+                       "view_matrices() and pass them to Graph.render as a static `view=(kinv, pinv)`")
         dev = pose_.device
         return (intr.detach().cpu().float().inverse().contiguous().to(dev),
                 Pose().invert(pose_.detach().cpu().float()).contiguous().to(dev))
@@ -107,13 +110,26 @@ def one_launch_matrices(opt) -> bool:
     return v == "kernel"
 
 
-def get_center_and_ray(opt, pose_, intr=None, H=None, W=None, ray_idx=None):
+def view_or_matrices(opt, pose_, intr, view=None):
+    """`view` = (K^-1 [B,3,3], pose^-1 [B,3,4]) computed by the caller (view_matrices, e.g. eagerly outside a captured CUDA graph)
+    or None: view_matrices(pose_, intr) as opt selects."""
+    if view is not None:
+        kinv, pinv = view
+        B = pose_.shape[0]
+        if tuple(kinv.shape) != (B, 3, 3) or tuple(pinv.shape) != (B, 3, 4):
+            raise ValueError(f"view matrices must be [{B},3,3] and [{B},3,4]; got {tuple(kinv.shape)} and {tuple(pinv.shape)}")
+        return kinv, pinv
+    return view_matrices(pose_, intr, one_launch=one_launch_matrices(opt))
+
+
+def get_center_and_ray(opt, pose_, intr=None, H=None, W=None, ray_idx=None, view=None):
     """camera.get_center_and_ray (camera.py:292-314).  Extra `ray_idx` [B,R] fuses Graph.ray_batch_sample
-    (model/nerf_adapt_st_gan.py:702-710) so only the requested pixels are ever generated."""
+    (model/nerf_adapt_st_gan.py:702-710) so only the requested pixels are ever generated; extra `view` = precomputed
+    (K^-1, pose^-1), see view_or_matrices."""
     assert opt.camera.model == "perspective"
     if H is None and W is None:
         H, W = opt.H, opt.W
-    kinv, pinv = view_matrices(pose_, intr, one_launch=one_launch_matrices(opt))
+    kinv, pinv = view_or_matrices(opt, pose_, intr, view)
     return ops.raygen(kinv, pinv, H, W, 0.5, ray_idx)
 
 

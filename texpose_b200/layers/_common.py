@@ -47,6 +47,11 @@ def b200_option(opt, name, default=None):
     return default if v is None else v
 
 
+def given_keywords(**kw):
+    """The optional keywords a caller was given (None = absent), so that a call passes them on only when they were given."""
+    return {k: v for k, v in kw.items() if v is not None}
+
+
 def flat_params(*module_lists):
     out = []
     for ml in module_lists:

@@ -166,6 +166,8 @@ def check_range(device=None):
     k = (dev.type, dev.index)
     if k not in _scratch:
         return
+    from .train_graph import refuse_capture
+    refuse_capture("mlp_tc32.check_range", "it reads the status word back to the host; call it between replays")
     off = _C.load().tp_tc32_status_offset()
     word = _scratch[k][off:off + 4]
     bad = int(word.view(torch.int32).item())

@@ -19,6 +19,11 @@ from ..config import AttrDict
 from ..layers.nerf_static_transient_light import NeRF
 from ..tools.ray_sampler import RaySampler
 from ..tools.patch_sampler import FlexPatchSampler
+from ..layers._common import given_keywords as _given
+from ..train_graph import refuse_capture
+
+
+_PHILOX = ("opt.b200.rng = 'philox'", "its seed is drawn on the host; use rng = 'torch'")
 
 
 def rotation_distance(R1, R2, eps=1e-7):
@@ -157,12 +162,12 @@ class Graph(torch.nn.Module):
             lat_light = lat_light.expand(B, -1).contiguous()
         return lat_trans, lat_light
 
-    def _render_fused(self, opt, pose, intr, ray_idx, depth_range, sample_idx, mode, want=None, out_ptrs=None):
+    def _render_fused(self, opt, pose, intr, ray_idx, depth_range, sample_idx, mode, want=None, out_ptrs=None, view=None):
         """model/nerf_adapt_st_gan.py:565-631 as one launch (csrc/mlp_tc.cu, render mode): rays, depths, view-direction bias
         and compositing happen inside the fused kernel.  ray_idx: [B,R] tensor, or a `range` = contiguous row block."""
         B = len(pose)
         HW = opt.H * opt.W
-        kinv, pinv = camera.view_matrices(pose, intr, one_launch=camera.one_launch_matrices(opt))
+        kinv, pinv = camera.view_or_matrices(opt, pose, intr, view)
         zn, zf = depth_range[0].reshape(B, HW), depth_range[1].reshape(B, HW)
         if isinstance(ray_idx, range):
             assert ray_idx.step == 1
@@ -173,6 +178,7 @@ class Graph(torch.nn.Module):
         rand, seed = None, 0
         if opt.nerf.sample_stratified:
             if self._b200(opt, "rng", "torch") == "philox":
+                refuse_capture(*_PHILOX)
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())
             else:
                 rand = torch.rand(B, R, opt.nerf.sample_intvs, 1, device=pose.device)      # the reference's draw (:690)
@@ -180,28 +186,31 @@ class Graph(torch.nn.Module):
                                     seed=seed, want=want, out_ptrs=out_ptrs)
         return AttrDict(ret)
 
-    def render(self, opt, pose, intr=None, ray_idx=None, depth_range=None, sample_idx=None, mode=None):
-        """model/nerf_adapt_st_gan.py:547-631 -> dict of 11 tensors."""
+    def render(self, opt, pose, intr=None, ray_idx=None, depth_range=None, sample_idx=None, mode=None, view=None):
+        """model/nerf_adapt_st_gan.py:547-631 -> dict of 11 tensors.  view: (K^-1, pose^-1) computed by the caller
+        (camera.view_matrices), e.g. eagerly outside a captured training step; None computes them here."""
         depth_min, depth_max = depth_range
         if opt.camera.ndc:
             raise NotImplementedError("camera.ndc is false in every reference yaml; not implemented")
         if mode != "train" and not self._b200(opt, "nan_guard", False) and self.nerf.fused_render_applies(opt, mode):
-            return self._render_fused(opt, pose, intr, ray_idx, depth_range, sample_idx, mode)
+            return self._render_fused(opt, pose, intr, ray_idx, depth_range, sample_idx, mode, view=view)
         if isinstance(ray_idx, range):
             ray_idx = torch.arange(ray_idx.start, ray_idx.stop, device=pose.device)[None].expand(len(pose), -1)
         if mode == "train":
             B, h, w, _ = ray_idx.shape
-            center, ray = self.ray_sampler.get_rays(opt, intrinsics=intr, coords=ray_idx, pose=pose)
+            center, ray = self.ray_sampler.get_rays(opt, intrinsics=intr, coords=ray_idx, pose=pose, **_given(view=view))
             zn, zf = self.ray_sampler.get_bounds(opt, coords=ray_idx, z_near=depth_min, z_far=depth_max)
             center, ray = center.view(B, h * w, 3), ray.view(B, h * w, 3)
             zn, zf = zn.reshape(B, h * w), zf.reshape(B, h * w)
         else:
             B = len(pose)
-            center, ray = camera.get_center_and_ray(opt, pose, intr=intr, ray_idx=ray_idx)
+            center, ray = camera.get_center_and_ray(opt, pose, intr=intr, ray_idx=ray_idx, **_given(view=view))
             zn = self.ray_batch_sample(depth_min, ray_idx).squeeze(-1)
             zf = self.ray_batch_sample(depth_max, ray_idx).squeeze(-1)
-        if self._b200(opt, "nan_guard", False) and bool(ray.isnan().any()):
-            raise FloatingPointError("NaN in generated rays")
+        if self._b200(opt, "nan_guard", False):
+            refuse_capture("opt.b200.nan_guard", "the NaN check reads the rays back to the host")
+            if bool(ray.isnan().any()):
+                raise FloatingPointError("NaN in generated rays")
         depth_samples = self.sample_depth(opt, B, (zn, zf), num_rays=ray.shape[1])       # [B,R,N,1]
 
         lat_trans, lat_light = self._latents(opt, B, sample_idx, mode, ray.device)
@@ -306,6 +315,7 @@ class Graph(torch.nn.Module):
         rand, seed = None, 0
         if opt.nerf.sample_stratified:
             if self._b200(opt, "rng", "torch") == "philox":
+                refuse_capture(*_PHILOX)
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())      # (a host generator: no device read-back)
             else:
                 rand = torch.rand(B, HW, N, 1, device=dev)
@@ -349,6 +359,7 @@ class Graph(torch.nn.Module):
         if not opt.nerf.sample_stratified:
             return ops.sample_depth(zn, zf, N, stratified=False)
         if self._b200(opt, "rng", "torch") == "philox":
+            refuse_capture(*_PHILOX)
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
             return ops.sample_depth(zn, zf, N, seed=seed)
         rand = torch.rand(batch_size, num_rays, N, 1, device=zn.device)

@@ -21,6 +21,8 @@ import torch
 from .. import camera, ops
 from ..config import AttrDict
 from ..layers.nerf import NeRF
+from ..layers._common import given_keywords as _given
+from ..train_graph import refuse_capture
 
 
 class Graph(torch.nn.Module):
@@ -70,8 +72,9 @@ class Graph(torch.nn.Module):
         return var
 
     # ---------------------------------------------------------------- the hot path
-    def render(self, opt, pose, intr=None, ray_idx=None, depth_range=None, mode=None):
-        """model/nerf_pretrain.py:588-627 -> rgb [B,R,3], depth [B,R,1], opacity [B,R,1]."""
+    def render(self, opt, pose, intr=None, ray_idx=None, depth_range=None, mode=None, view=None):
+        """model/nerf_pretrain.py:588-627 -> rgb [B,R,3], depth [B,R,1], opacity [B,R,1].  view: (K^-1, pose^-1) computed by the
+        caller (camera.view_matrices), e.g. eagerly outside a captured training step; None computes them here."""
         if opt.camera.ndc:
             raise NotImplementedError("camera.ndc is false in every reference yaml; not implemented")
         B = len(pose)
@@ -79,9 +82,11 @@ class Graph(torch.nn.Module):
             ray_idx = range(0, opt.H * opt.W)
         if isinstance(ray_idx, range):
             ray_idx = torch.arange(ray_idx.start, ray_idx.stop, device=pose.device)[None].expand(B, -1)
-        center, ray = camera.get_center_and_ray(opt, pose, intr=intr, ray_idx=ray_idx)
-        if self._b200(opt, "nan_guard", False) and bool(ray.isnan().any()):
-            raise FloatingPointError("NaN in generated rays")
+        center, ray = camera.get_center_and_ray(opt, pose, intr=intr, ray_idx=ray_idx, **_given(view=view))
+        if self._b200(opt, "nan_guard", False):
+            refuse_capture("opt.b200.nan_guard", "the NaN check reads the rays back to the host")
+            if bool(ray.isnan().any()):
+                raise FloatingPointError("NaN in generated rays")
         depth_min, depth_max = depth_range
         zn = self.ray_batch_sample(depth_min, ray_idx).squeeze(-1)
         zf = self.ray_batch_sample(depth_max, ray_idx).squeeze(-1)
@@ -107,6 +112,7 @@ class Graph(torch.nn.Module):
         rand, seed = None, 0
         if opt.nerf.sample_stratified:
             if self._b200(opt, "rng", "torch") == "philox":
+                refuse_capture("opt.b200.rng = 'philox'", "its seed is drawn on the host; use rng = 'torch'")
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())
             else:
                 rand = torch.rand(B, R, opt.nerf.sample_intvs, 1, device=pose.device)      # sample_depth's draw (:707-728)

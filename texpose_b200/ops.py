@@ -65,6 +65,9 @@ def device_table(rows, dtype, device) -> Tensor:
     key = (str(device), dtype, flat)
     t = _TABLES.get(key)
     if t is None:
+        if torch.cuda.is_available() and torch.cuda.is_current_stream_capturing():
+            raise RuntimeError("ops.device_table cannot upload a new table while a CUDA graph is being captured: run the same "
+                               "call once before the capture (train_graph.GraphedStep's warm-up does)")
         t = _TABLES[key] = torch.tensor(rows, dtype=dtype, device=device)
         if len(_TABLES) > 256:
             _TABLES.popitem(last=False)

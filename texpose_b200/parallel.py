@@ -195,9 +195,13 @@ class PeerGradExchange(GradBucket):
     buffer of the next device epoch and advance it), `tp_peer_allreduce_mean_dev` into `flat`, and the views of `unpack()`.
     Eager calls and replays advance the same device counter, so every rank must make the same sequence of exchanges --
     counting GraphedStep's eager warm-up steps -- as it must make the same sequence of calls without a graph.  Without
-    capturable, a call made while the current stream is capturing raises: the host epoch would be frozen into the graph."""
+    capturable, a call made while the current stream is capturing raises: the host epoch would be frozen into the graph.
 
-    def __init__(self, params: Iterable[torch.nn.Parameter], group=None, timeout_ms: int = 10000, capturable: bool = False):
+    grid_ctas: CTAs of the exchange kernel (0: the library's default, two per SM up to the bucket size).  A waiting rank's CTAs
+    hold their SMs until every peer has published; ranks that share one device need a small grid so the others' steps still run."""
+
+    def __init__(self, params: Iterable[torch.nn.Parameter], group=None, timeout_ms: int = 10000, capturable: bool = False,
+                 grid_ctas: int = 0):
         super().__init__(params)
         if not (dist.is_available() and dist.is_initialized()):
             raise RuntimeError("PeerGradExchange needs an initialised process group (use GradBucket for a single process)")
@@ -211,6 +215,7 @@ class PeerGradExchange(GradBucket):
         self.ptrs = [self.window.ptr if r == self.rank else self.window.open_peer(h) for r, h in enumerate(handles)]
         self.flat = torch.zeros((self.n + 3) // 4 * 4, dtype=torch.float32, device=dev)    # the reduced gradients land here
         self.epoch = 0
+        self.grid_ctas = int(grid_ctas)
         self.capturable = bool(capturable)
         self.staging = torch.zeros_like(self.flat) if self.capturable else None
         torch.cuda.synchronize(dev)
@@ -220,7 +225,7 @@ class PeerGradExchange(GradBucket):
         if self.capturable:
             self.pack(into=self.staging[:self.n])
             peer_stage(self.window.ptr, self.n, self.staging)
-            peer_allreduce_mean_dev(self.ptrs, self.rank, self.n, self.flat, timeout_ms=self.timeout_ms)
+            peer_allreduce_mean_dev(self.ptrs, self.rank, self.n, self.flat, grid_ctas=self.grid_ctas, timeout_ms=self.timeout_ms)
             self.unpack()
             return
         if torch.cuda.is_current_stream_capturing():
@@ -228,7 +233,8 @@ class PeerGradExchange(GradBucket):
                                "host-chosen epoch: construct the exchange with capturable=True")
         self.epoch += 1
         self.pack(into=self.window.buffers[self.epoch & 1])
-        peer_allreduce_mean(self.ptrs, self.rank, self.n, self.epoch, self.flat, timeout_ms=self.timeout_ms)
+        peer_allreduce_mean(self.ptrs, self.rank, self.n, self.epoch, self.flat, grid_ctas=self.grid_ctas,
+                            timeout_ms=self.timeout_ms)
         self.unpack()
 
     def check(self):

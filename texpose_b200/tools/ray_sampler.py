@@ -32,9 +32,9 @@ class RaySampler(object):
         return zn[:, 0], zf[:, 0]
 
     @staticmethod
-    def get_rays(opt, intrinsics, coords, pose, H=None, W=None):
-        """tools/ray_sampler.py:39-69 -> center, ray [B,h,w,3]."""
+    def get_rays(opt, intrinsics, coords, pose, H=None, W=None, view=None):
+        """tools/ray_sampler.py:39-69 -> center, ray [B,h,w,3].  view: precomputed (K^-1, pose^-1), camera.view_or_matrices."""
         H, W = RaySampler._hw(opt, H, W)
         with torch.no_grad():
-            kinv, pinv = camera.view_matrices(pose, intrinsics, one_launch=camera.one_launch_matrices(opt))
+            kinv, pinv = camera.view_or_matrices(opt, pose, intrinsics, view)
             return ops.patch_rays(kinv, pinv, coords, H, W)

@@ -12,10 +12,31 @@ of the bf16 weight images that the updated weights require -- can be captured on
     for batch in loader:
         out = step(coords=batch.coords, image=batch.image, ...)      # copies into the static buffers, replays
 
+Capturable steps (each tested replay == eager, bit for bit: tests/test_gpu_train_graph.py, test_gpu_graph_pretrain.py,
+test_gpu_graph_fp32.py):
+  * adaptation `model.nerf_adapt_st_gan.Graph`, opt.b200.mlp 'bf16' / 'auto' (lock-step forward + fused heads backward, or the
+    staged kernels) and 'fp32' with fp32_engine = 'tc' (split save + split staged heads backward);
+  * pre-training `model.nerf_pretrain.Graph` (and nerf_pretrain_env), opt.b200.mlp 'bf16' / 'auto' and 'fp32' with
+    fp32_engine = 'tc' (mlp_tc_plain: the trunk trains).
+Static inputs -- everything the step reads that changes between steps, allocated once and passed in `static`: the adaptation
+step's patch coordinates, image and mask; the pre-training step's ray subset (`Graph.get_ray_idx` draws it with torch.randperm:
+call it eagerly, outside the graph, so the random stream is the reference's, and pass `var.ray_idx`), image, obj_mask,
+erode_mask, depth_gt; and for either engine pose, intr, z_near / z_far whenever they change per batch.  View matrices: the bf16
+modes build them on the device in one launch (tp_view_matrices), the fp32 mode with torch.linalg.inv_ex, which is captured as
+it stands.  With camera.HOST_MATRICES (K^-1 / pose^-1 inverted on the CPU, a synchronisation) compute them eagerly with
+`camera.view_matrices` and pass them as a static `view=(kinv, pinv)` to `Graph.render`; capturing the host inversion raises.
+
 Requirements (checked where they can be): the optimizer is capturable (`torch.optim.Adam(..., capturable=True)`); `fn` reads its
-inputs from the static tensors, takes no data-dependent Python branch and makes no host read-back -- in `opt.b200` terms:
-`rng = 'torch'` (the in-kernel Philox mode draws its seed on the host) and no `nan_guard`; shapes are fixed.  The warm-up
-iterations are real training steps on the inputs present in the static buffers.
+inputs from the static tensors, takes no data-dependent Python branch and makes no host read-back; shapes are fixed.  What
+would freeze a host decision into the graph raises while capturing, naming the option: opt.b200.rng = 'philox' (its seed is drawn
+on the host: use 'torch', whose generator advances on every replay), opt.b200.nan_guard (reads back), mlp_tc32.check_range
+(reads back), camera.HOST_MATRICES without `view`, and an ops.device_table miss (a host upload).  The warm-up iterations are real
+training steps on the inputs present in the static buffers.
+
+Weight caches: the packed weight images are keyed by the parameters' addresses and `_version`.  A replay changes the weights
+without Python seeing it, so the step bumps the version counter of every parameter the optimizer updates before the capture
+(every pack launch is then recorded in the graph, never skipped on a stale key) and after every replay (an eager render between
+replays re-packs from the weights the replays wrote).
 
 Data-parallel: call the gradient exchange inside `fn` after `backward()`.  `parallel.PeerGradExchange(params, capturable=True)`
 keeps its epoch on the device, so every replay runs a new exchange and nothing NCCL-side is captured; its warm-up calls here are
@@ -28,6 +49,14 @@ from __future__ import annotations
 from typing import Callable, Dict, Optional
 
 import torch
+from torch.autograd.graph import increment_version
+
+
+def refuse_capture(option: str, reason: str):
+    """Raises when the current stream is capturing a CUDA graph: the caller is about to decide something on the host (`reason`)
+    that a replay would repeat with the captured value instead of deciding it again."""
+    if torch.cuda.is_available() and torch.cuda.is_current_stream_capturing():
+        raise RuntimeError(f"{option} cannot be captured in a CUDA graph: {reason}")
 
 
 class GraphedStep:
@@ -46,6 +75,7 @@ class GraphedStep:
                 raise ValueError(f"static input {k!r} must be a CUDA tensor")
         self.optimizer = optimizer
         self.warmup_steps = int(warmup)
+        self._trained = [p for group in optimizer.param_groups for p in group["params"]] if optimizer is not None else []
 
         def one():
             out = fn()
@@ -67,6 +97,7 @@ class GraphedStep:
         # gradients are created inside the capture, from the graph's private pool; a replay overwrites them in place
         if optimizer is not None:
             optimizer.zero_grad(set_to_none=True)
+        increment_version(self._trained)        # no weight cache may hit during the capture: every pack launch is recorded
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             self.out = one()
@@ -83,5 +114,6 @@ class GraphedStep:
                 raise ValueError(f"static input {k!r} has shape {tuple(dst.shape)}; got {tuple(v.shape)} (a graph has fixed shapes)")
             dst.copy_(v, non_blocking=True)
         self.graph.replay()
+        increment_version(self._trained)        # the replay rewrote the weights: version-keyed caches must re-pack
         self.replays += 1
         return self.out
